@@ -5,7 +5,7 @@ Workload (BASELINE.json configs[1]): batched negacyclic polynomial multiplicatio
 q = 12289, 2^20 independent operand pairs per GPU, synthetic uniform coefficients.  One "step" is
 one pass of the fused polymul kernel over the whole batch.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 N > 1 is launched by the driver under torch.distributed.run (one rank per GPU).  The batch shards by
 polynomial index with no data-path collective (weak scaling: 2^20 pairs per GPU); NCCL is used only for
@@ -13,9 +13,12 @@ the barrier and the max-over-ranks of the device time.
 
 Prints ONE JSON line.  `value` = polymuls/s with operands resident in HBM (CUDA events on the launching
 stream); `e2e` = the same metric through scgpu_polymul_batch_host() with pinned HOST buffers, H2D and
-D2H inside the timed region; `roofline` = algorithmic bytes (12 n per product) / kernel time against
+D2H inside the timed region (that leg runs max(3, min(K, 10)) steps, recorded as e2e.steps; `--steps K`
+sets the device-resident leg's count); `roofline` = algorithmic bytes (12 n per product) / kernel time against
 the measured HBM copy bandwidth; `cpu_baseline` = the reference's own C code (oracle/_ref) on the
-host cores of this box.  `--impl reference` times that CPU path alone.
+host cores of this box.  `--impl reference` times that CPU path alone.  `--dump-outputs DIR` writes a fixed,
+seeded sample of 2^14 rows of the last timed step's product (rank 0) to DIR/polymul_out.npy as float32; the
+operands are seeded, so two builds given the same arguments can be compared output for output.
 """
 import argparse
 import json
@@ -182,6 +185,19 @@ def bind_to_gpu_numa_node(index):
         return 0
 
 
+DUMP_ROWS = 1 << 14             # 2^14 of the 2^20 products x 512 coefficients in float32 = 32 MiB
+
+
+def dump_outputs(path, out):
+    """What the timed path returned in its last step, for comparing two builds output for output: the same seeded
+    sample of rows of `out` (rank 0's batch) on every run.  Residues are below 2^24, so float32 holds them exactly."""
+    import torch
+    rows = np.sort(np.random.default_rng(20261020).choice(out.shape[0], size=min(DUMP_ROWS, out.shape[0]), replace=False))
+    sample = out[torch.from_numpy(rows).to(out.device)].cpu().numpy().astype(np.float32)
+    os.makedirs(path, exist_ok=True)
+    np.save(os.path.join(path, "polymul_out.npy"), sample)
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -189,7 +205,14 @@ def main():
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write a fixed sample of the last timed step's polymul output to DIR/polymul_out.npy (float32)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        # the reference arm sizes its sample from a timing calibration, so its inputs differ from run to run
+        ap.error("--dump-outputs applies to --impl ours only")
     if args.warmup < 3 and args.impl == "ours":
         args.warmup = 3
 
@@ -261,6 +284,8 @@ def main():
     ev1.record()
     barrier()
     launches = sc.launch_count() - launches0
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, out)
     elapsed_ms = ev0.elapsed_time(ev1)
     kernel_ms = [s.elapsed_time(e) for s, e in evs]
     if world > 1:

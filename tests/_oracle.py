@@ -292,6 +292,32 @@ def ref():
     return _cache["ref"]
 
 
+def golden(name):
+    """Arrays of tests/golden/<name>.npz as a dict.  A fixture stores each distinct array once: its optional
+    `_aliases` member lists (name, stored name) pairs for the arrays equal to one already stored."""
+    with np.load(os.path.join(ROOT, "tests", "golden", name + ".npz")) as z:
+        out = {k: z[k] for k in z.files}
+    for alias, stored in out.pop("_aliases", np.zeros((0, 2), dtype=str)):
+        out[str(alias)] = out[str(stored)]
+    return out
+
+
+def dedup_arrays(arrays):
+    """The inverse of golden(): keep the first of each group of equal arrays, list the others in `_aliases`."""
+    import hashlib
+    out, seen, aliases = {}, {}, []
+    for k, a in arrays.items():
+        h = hashlib.sha256(a.dtype.str.encode() + str(a.shape).encode() + np.ascontiguousarray(a).tobytes()).digest()
+        if h in seen:
+            aliases.append((k, seen[h]))
+        else:
+            seen[h] = k
+            out[k] = a
+    if aliases:
+        out["_aliases"] = np.array(aliases, dtype=str)
+    return out
+
+
 def tables(q, n, tw_bits):
     """(w, r) for a parameter set -- from the port's generator (validated against the reference's
     generated ntt_tables.c in tests/test_oracle_vs_ref.py and tests/golden/tables.json)."""

@@ -1,9 +1,9 @@
 """Generate tests/golden/*.npz from the COMPILED REFERENCE (oracle/_ref/libscref.so).
 
-Run in the dev container only (needs /root/reference for `make -C oracle ref` and for the
-fixed vectors of src/unit/unit_ntt.c::test_ibe):
+Needs the reference's source tree, named by REF as for oracle/Makefile (`make -C oracle ref` builds
+the library from it; src/unit/unit_ntt.c::test_ibe holds the fixed vectors read below):
 
-    python tests/golden/make_golden.py
+    REF=<reference sources> python tests/golden/make_golden.py
 
 The fixtures are what pins the oracle port (and, through it, the CUDA path) on machines where
 the reference library is absent.  Inputs are stored next to outputs, so the tests need no RNG
@@ -20,7 +20,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, os.path.dirname(HERE))
 import _oracle as O  # noqa: E402
 
-REF_SRC = "/root/reference"
+REF_SRC = os.environ.get("REF", "")
 
 
 def variants_for(q):
@@ -33,6 +33,8 @@ def variants_for(q):
 
 
 def main():
+    if not os.path.isdir(os.path.join(REF_SRC, "src")):
+        sys.exit("make_golden.py: set REF to the reference's source tree")
     ref = O.ref()
     rng = np.random.default_rng(20261017)
     out = {}
@@ -113,8 +115,10 @@ def main():
         out["gauss_ber64_%s" % pname] = ref.gauss_streams(O.SAMPLER_BERNOULLI, 64, 0, pt, 13.42, 215.0, seeds, 128)
         out["gauss_ber64s_%s" % pname] = ref.gauss_streams(O.SAMPLER_BERNOULLI, 64, 0, pt, 13.0, 4.5, seeds, 512)
 
+    # many variants return identical arrays: each is stored once (O.golden() restores the aliases), which keeps the
+    # file under 1 MB
     path = os.path.join(HERE, "golden_v1.npz")
-    np.savez_compressed(path, **out)
+    np.savez_compressed(path, **O.dedup_arrays(out))
     print("wrote", path, os.path.getsize(path), "bytes,", len(out), "arrays")
 
     # ---- golden_v2: 128 / 192-bit CDF sampling (gaussian_cdf.c:112-509) over an injected table ------------

@@ -15,7 +15,7 @@ if not torch.cuda.is_available():
 
 import libsafecrypto_b200 as sc  # noqa: E402
 
-G = np.load(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "golden_v1.npz"))
+G = O.golden("golden_v1")
 DEV = "cuda:0"
 
 

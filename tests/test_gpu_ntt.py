@@ -19,7 +19,7 @@ if not torch.cuda.is_available():
 
 import libsafecrypto_b200 as sc  # noqa: E402
 
-G = np.load(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "golden_v1.npz"))
+G = O.golden("golden_v1")
 PARAMS = [(12289, 512, 16), (12289, 1024, 16), (7681, 256, 16), (8380417, 256, 32), (8399873, 512, 32)]
 DEV = "cuda:0"
 

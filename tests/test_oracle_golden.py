@@ -11,7 +11,7 @@ import pytest
 
 import _oracle as O
 
-G = np.load(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "golden_v1.npz"))
+G = O.golden("golden_v1")
 P = O.port()
 
 
