@@ -55,6 +55,9 @@ def lib():
         L.scgpu_matvec_batch.argtypes = [vp, vp, vp, vp, ctypes.c_int, ctypes.c_int, sz, vp]
         L.scgpu_rand_product_csprng_batch.argtypes = [vp, vp, vp, vp, sz, ctypes.c_int, u32, ctypes.c_int, ctypes.c_int, ctypes.c_int, sz, vp]
         L.scgpu_rand_product_csprng_batch_host.argtypes = [vp, vp, vp, vp, sz, ctypes.c_int, u32, ctypes.c_int, ctypes.c_int, ctypes.c_int, sz]
+        L.scgpu_matvec_shared_batch.argtypes = [vp, vp, vp, vp, ctypes.c_int, ctypes.c_int, sz, vp]
+        L.scgpu_rand_product_csprng_shared_batch.argtypes = [vp, vp, vp, vp, sz, ctypes.c_int, u32, ctypes.c_int, ctypes.c_int, ctypes.c_int, sz, vp]
+        L.scgpu_rand_product_csprng_shared_batch_host.argtypes = [vp, vp, vp, vp, sz, ctypes.c_int, u32, ctypes.c_int, ctypes.c_int, ctypes.c_int, sz]
         L.scgpu_rand_matrix_csprng_batch.argtypes = [vp, vp, sz, ctypes.c_int, i32, u32, ctypes.c_int, ctypes.c_int, ctypes.c_int, ctypes.c_int, sz, vp]
         L.scgpu_ntt_plans_create_all.argtypes = [ctypes.POINTER(vp), ctypes.c_int, vp, ctypes.c_int, vp, vp, ctypes.c_int]
         L.scgpu_polymul_batch_host_multi.argtypes = [ctypes.POINTER(vp), ctypes.c_int, vp, vp, vp, sz, sz]
@@ -196,6 +199,13 @@ class NttPlan:
         return _check(lib().scgpu_matvec_batch(self.handle, _ptr(out), _ptr(A), _ptr(s), k, l, count,
                                                _stream_handle(stream)), "scgpu_matvec_batch")
 
+    def matvec_shared(self, out, A, s, k, l, count=None, stream=None):
+        """matvec with ONE matrix A [k, l, n] for every instance of s [count, l, n]."""
+        if count is None:
+            count = s.shape[0]
+        return _check(lib().scgpu_matvec_shared_batch(self.handle, _ptr(out), _ptr(A), _ptr(s), k, l, count,
+                                                      _stream_handle(stream)), "scgpu_matvec_shared_batch")
+
     def rand_product(self, out, y, seeds, prng_type, q_bits, k, l, transpose=False, count=None, stream=None):
         """create_rand_product_{16,32}_csprng with the matrix sampled on the device from seeds [count, seed_len]."""
         if count is None:
@@ -210,6 +220,21 @@ class NttPlan:
         return _check(lib().scgpu_rand_product_csprng_batch_host(self.handle, _ptr(out), _ptr(y), _ptr(seeds), seeds.shape[-1],
                                                                  prng_type, q_bits, k, l, 1 if transpose else 0, count),
                       "scgpu_rand_product_csprng_batch_host")
+
+    def rand_product_shared(self, out, y, seed, prng_type, q_bits, k, l, transpose=False, count=None, stream=None):
+        """rand_product with ONE seed [seed_len] (the key's rho) for every instance: the matrix is drawn once."""
+        if count is None:
+            count = y.shape[0]
+        return _check(lib().scgpu_rand_product_csprng_shared_batch(self.handle, _ptr(out), _ptr(y), _ptr(seed), seed.shape[-1],
+                                                                   prng_type, q_bits, k, l, 1 if transpose else 0, count,
+                                                                   _stream_handle(stream)), "scgpu_rand_product_csprng_shared_batch")
+
+    def rand_product_shared_host(self, out, y, seed, prng_type, q_bits, k, l, transpose=False, count=None):
+        if count is None:
+            count = y.shape[0]
+        return _check(lib().scgpu_rand_product_csprng_shared_batch_host(self.handle, _ptr(out), _ptr(y), _ptr(seed), seed.shape[-1],
+                                                                        prng_type, q_bits, k, l, 1 if transpose else 0, count),
+                      "scgpu_rand_product_csprng_shared_batch_host")
 
     # ---- host buffers (numpy arrays or pinned torch CPU tensors) -----------------------------------
     def batch_host(self, op, out, a, b=None, b_stride=None, count=None, scalar=0, rc=None):

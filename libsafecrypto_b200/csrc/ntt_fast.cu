@@ -249,7 +249,8 @@ k_polymul(int32_t *__restrict__ out, const int32_t *__restrict__ a, const void *
 // One instance per thread group: forward the l secret polynomials once (kept in a shared-memory
 // stash in NTT domain), then for each of the k rows accumulate A_ij o s_j in registers, one
 // inverse transform per row.  A is read exactly once, s once, t written once: 4n(k l + l + k) bytes.
-template <int LOGN, int MAXL>
+// SHARED_A: one matrix for every instance (instance stride 0)
+template <int LOGN, int MAXL, bool SHARED_A = false>
 __global__ void __launch_bounds__(kCtaThreads)
 k_matvec(int32_t *__restrict__ out, const int32_t *__restrict__ A, const int32_t *__restrict__ s,
          int k, int l, size_t count, FastConst c)
@@ -283,7 +284,7 @@ k_matvec(int32_t *__restrict__ out, const int32_t *__restrict__ A, const int32_t
 #pragma unroll
             for (int m = 0; m < 8; m++) acc[m] = 0;
             for (int j = 0; j < l; j++) {
-                const int32_t *arow = A + ((irow * k + i) * l + j) * N;
+                const int32_t *arow = A + (((SHARED_A ? (size_t)0 : irow * k) + i) * l + j) * N;
 #pragma unroll
                 for (int m = 0; m < 8; m++) {
                     const int idx = (int)(__brev((unsigned)(elem_index<PassCfg<LOGN, LAST>::D>(tau, m))) >> (32 - LOGN));
@@ -492,7 +493,7 @@ int launch_mul_key(const NttPlanDev &p, int32_t *out, const int32_t *t, const vo
 }
 
 int launch_matvec(const NttPlanDev &p, int32_t *out, const int32_t *A, const int32_t *s,
-                  int k, int l, size_t count, cudaStream_t st)
+                  int k, int l, size_t count, cudaStream_t st, bool shared)
 {
     if (count == 0) return SCGPU_OK;
     SCGPU_REQUIRE_FAST(p);
@@ -501,20 +502,21 @@ int launch_matvec(const NttPlanDev &p, int32_t *out, const int32_t *A, const int
     if (l > 4) {
         // only the Shoup-policy kernels take l at run time (Dilithium k = 6, l = 5)
         if (use_sh32(p) && p.sh32_mv_ok && l <= p.sh32_mv_lmax && !(use_fq32(p) && p.fq32_mv_ok))
-            return launch_matvec_sh32(p, out, A, s, k, l, count, st);
+            return launch_matvec_sh32(p, out, A, s, k, l, count, st, shared);
         set_error("matvec l > 4 not instantiated for this modulus");
         return SCGPU_ERR_UNSUPPORTED;
     }
-    if (force_sh32(p) && p.sh32_mv_ok) return launch_matvec_sh32(p, out, A, s, k, l, count, st);
-    if (use_fq32(p) && p.fq32_mv_ok) return launch_matvec_fq32(p, out, A, s, k, l, count, st);
-    if (use_fq(p)) return launch_matvec_fq(p, out, A, s, k, l, count, st);
-    if (use_sq(p)) return launch_matvec_sq(p, out, A, s, k, l, count, st);
-    if (use_sh32(p) && p.sh32_mv_ok) return launch_matvec_sh32(p, out, A, s, k, l, count, st);
+    if (force_sh32(p) && p.sh32_mv_ok) return launch_matvec_sh32(p, out, A, s, k, l, count, st, shared);
+    if (use_fq32(p) && p.fq32_mv_ok) return launch_matvec_fq32(p, out, A, s, k, l, count, st, shared);
+    if (use_fq(p)) return launch_matvec_fq(p, out, A, s, k, l, count, st, shared);
+    if (use_sq(p)) return launch_matvec_sq(p, out, A, s, k, l, count, st, shared);
+    if (use_sh32(p) && p.sh32_mv_ok) return launch_matvec_sh32(p, out, A, s, k, l, count, st, shared);
     FastConst c = make_const(p);
     const size_t G = kCtaThreads / (p.n / 8);
     // shared-memory stash limits residency to 1-2 CTAs per SM
     const unsigned grid = grid_for(p, (count + G - 1) / G);
-    if (l <= 4) k_matvec<8, 4><<<grid, kCtaThreads, 0, st>>>(out, A, s, k, l, count, c);
+    if (l <= 4 && shared) k_matvec<8, 4, true><<<grid, kCtaThreads, 0, st>>>(out, A, s, k, l, count, c);
+    else if (l <= 4) k_matvec<8, 4><<<grid, kCtaThreads, 0, st>>>(out, A, s, k, l, count, c);
     else {
         set_error("matvec l > 4 not instantiated");
         return SCGPU_ERR_UNSUPPORTED;

@@ -304,7 +304,8 @@ k_polymul_fq(int32_t *__restrict__ out, const int32_t *__restrict__ a, const voi
 }
 
 // module-LWE matrix-vector product t_i = INTT(sum_j A_ij o NTT(s_j)), same structure as k_matvec (ntt_fast.cu)
-template <int LOGN, int MAXL>
+// SHARED_A: one matrix for every instance (instance stride 0)
+template <int LOGN, int MAXL, bool SHARED_A = false>
 __global__ void __launch_bounds__(kCtaThreads)
 k_matvec_fq(int32_t *__restrict__ out, const int32_t *__restrict__ A, const int32_t *__restrict__ s,
             int k, int l, size_t count, const __grid_constant__ FqConst c)
@@ -337,7 +338,7 @@ k_matvec_fq(int32_t *__restrict__ out, const int32_t *__restrict__ A, const int3
 #pragma unroll
             for (int m = 0; m < 8; m++) acc[m] = (u32)kBias;
             for (int j = 0; j < l; j++) {
-                const int32_t *arow = A + ((irow * k + i) * l + j) * N;
+                const int32_t *arow = A + (((SHARED_A ? (size_t)0 : irow * k) + i) * l + j) * N;
                 int32_t av[8];
                 bool wide = false;
 #pragma unroll
@@ -467,12 +468,13 @@ int launch_polymul_fq(const NttPlanDev &p, int mode, int32_t *out, const int32_t
 }
 
 int launch_matvec_fq(const NttPlanDev &p, int32_t *out, const int32_t *A, const int32_t *s, int k, int l,
-                     size_t count, cudaStream_t st)
+                     size_t count, cudaStream_t st, bool shared)
 {
     const FqConst c = fq_const(p, true);
     const size_t G = kCtaThreads / (p.n / 8);
     const unsigned grid = fq_grid(p, (count + G - 1) / G, 2);
-    k_matvec_fq<8, 4><<<grid, kCtaThreads, 0, st>>>(out, A, s, k, l, count, c);
+    if (shared) k_matvec_fq<8, 4, true><<<grid, kCtaThreads, 0, st>>>(out, A, s, k, l, count, c);
+    else        k_matvec_fq<8, 4><<<grid, kCtaThreads, 0, st>>>(out, A, s, k, l, count, c);
     count_launch();
     SCGPU_CUDA_CHECK(cudaGetLastError());
     return SCGPU_OK;

@@ -300,10 +300,10 @@ void free_fq32_tables(NttPlanDev &p)
 
 // n = 256 (Kyber); returns SCGPU_ERR_UNSUPPORTED when this schedule does not apply (the caller falls back)
 int launch_matvec_fq32(const NttPlanDev &p, int32_t *out, const int32_t *A, const int32_t *s, int k, int l,
-                       size_t count, cudaStream_t st)
+                       size_t count, cudaStream_t st, bool shared)
 {
     if (!p.fq32_ok || !p.fq32_mv_ok || p.logn != 8 || l > 4) return SCGPU_ERR_UNSUPPORTED;
-    return w32::launch_matvec_w32<ArFq>(fq32_const(p, p.fq32_r0_mv), p.sm_count, out, A, s, k, l, count, st, !p.inputs_in_range);
+    return w32::launch_matvec_w32<ArFq>(fq32_const(p, p.fq32_r0_mv), p.sm_count, out, A, s, k, l, count, st, !p.inputs_in_range, shared);
 }
 
 int launch_polymul_fq32(const NttPlanDev &p, int mode, int32_t *out, const int32_t *a, const void *b,

@@ -241,10 +241,10 @@ void free_sh32_tables(NttPlanDev &p)
 }
 
 int launch_matvec_sh32(const NttPlanDev &p, int32_t *out, const int32_t *A, const int32_t *s, int k, int l,
-                       size_t count, cudaStream_t st)
+                       size_t count, cudaStream_t st, bool shared)
 {
     if (!p.sh32_ok || !p.sh32_mv_ok || p.logn != 8 || l > p.sh32_mv_lmax) return SCGPU_ERR_UNSUPPORTED;
-    return w32::launch_matvec_w32<ArSh>(sh32_const(p, p.sh32_r0_mv), p.sm_count, out, A, s, k, l, count, st, !p.inputs_in_range);
+    return w32::launch_matvec_w32<ArSh>(sh32_const(p, p.sh32_r0_mv), p.sm_count, out, A, s, k, l, count, st, !p.inputs_in_range, shared);
 }
 
 int launch_polymul_sh32(const NttPlanDev &p, int mode, int32_t *out, const int32_t *a, const void *b,

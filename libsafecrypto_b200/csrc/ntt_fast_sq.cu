@@ -233,7 +233,8 @@ k_polymul_sq(int32_t *__restrict__ out, const int32_t *__restrict__ a, const voi
 }
 
 // module-LWE matrix-vector product, same structure as k_matvec in ntt_fast.cu
-template <int LOGN, int MAXL>
+// SHARED_A: one matrix for every instance (instance stride 0)
+template <int LOGN, int MAXL, bool SHARED_A = false>
 __global__ void __launch_bounds__(kCtaThreads)
 k_matvec_sq(int32_t *__restrict__ out, const int32_t *__restrict__ A, const int32_t *__restrict__ s,
             int k, int l, size_t count, SqConst c)
@@ -266,7 +267,7 @@ k_matvec_sq(int32_t *__restrict__ out, const int32_t *__restrict__ A, const int3
 #pragma unroll
             for (int m = 0; m < 8; m++) acc[m] = 0;
             for (int j = 0; j < l; j++) {
-                const int32_t *arow = A + ((irow * k + i) * l + j) * N;
+                const int32_t *arow = A + (((SHARED_A ? (size_t)0 : irow * k) + i) * l + j) * N;
 #pragma unroll
                 for (int m = 0; m < 8; m++) {
                     const int idx = (int)(__brev((unsigned)(elem_index<PassCfg<LOGN, LAST>::D>(tau, m))) >> (32 - LOGN));
@@ -439,13 +440,14 @@ int launch_polymul_sq(const NttPlanDev &p, int mode, int32_t *out, const int32_t
 }
 
 int launch_matvec_sq(const NttPlanDev &p, int32_t *out, const int32_t *A, const int32_t *s, int k, int l,
-                     size_t count, cudaStream_t st)
+                     size_t count, cudaStream_t st, bool shared)
 {
     SqConst c = sq_const(p);
     for (int i = 0; i < 4; i++) c.r_inv[i] = p.sq_r_inv_mv[i];
     const size_t G = kCtaThreads / (p.n / 8);
     const unsigned grid = sq_grid(p, (count + G - 1) / G, 2);
-    k_matvec_sq<8, 4><<<grid, kCtaThreads, 0, st>>>(out, A, s, k, l, count, c);
+    if (shared) k_matvec_sq<8, 4, true><<<grid, kCtaThreads, 0, st>>>(out, A, s, k, l, count, c);
+    else        k_matvec_sq<8, 4><<<grid, kCtaThreads, 0, st>>>(out, A, s, k, l, count, c);
     count_launch();
     SCGPU_CUDA_CHECK(cudaGetLastError());
     return SCGPU_OK;

@@ -101,8 +101,9 @@ int launch_polymul(const NttPlanDev &plan, int32_t *out, const int32_t *a, const
                    size_t b_stride, size_t count, cudaStream_t stream);
 int launch_mul_key(const NttPlanDev &plan, int32_t *out, const int32_t *t, const void *key,
                    int key_bits, size_t key_stride, size_t count, cudaStream_t stream);
+// shared: A is ONE matrix [k][l][n] for all `count` instances (scgpu_matvec_shared_batch)
 int launch_matvec(const NttPlanDev &plan, int32_t *out, const int32_t *A, const int32_t *s,
-                  int k, int l, size_t count, cudaStream_t stream);
+                  int k, int l, size_t count, cudaStream_t stream, bool shared = false);
 int build_fast_tables(NttPlanDev &plan, const int32_t *w_host);
 void free_fast_tables(NttPlanDev &plan);
 int set_force_montgomery(int on);
@@ -120,19 +121,19 @@ void free_sh32_tables(NttPlanDev &plan);
 int launch_polymul_sh32(const NttPlanDev &plan, int mode, int32_t *out, const int32_t *a, const void *b,
                         size_t b_stride, size_t count, cudaStream_t stream);
 int launch_matvec_sh32(const NttPlanDev &plan, int32_t *out, const int32_t *A, const int32_t *s, int k, int l,
-                       size_t count, cudaStream_t stream);
+                       size_t count, cudaStream_t stream, bool shared = false);
 int launch_ntt_fq32(const NttPlanDev &plan, int inverse, int32_t *out, const int32_t *a, size_t count, cudaStream_t stream);
 int launch_ntt_sh32(const NttPlanDev &plan, int inverse, int32_t *out, const int32_t *a, size_t count, cudaStream_t stream);
 int launch_ntt_canonical(const NttPlanDev &plan, int inverse, int32_t *out, const int32_t *a, size_t count, cudaStream_t stream);
 int launch_matvec_fq32(const NttPlanDev &plan, int32_t *out, const int32_t *A, const int32_t *s, int k, int l,
-                       size_t count, cudaStream_t stream);
+                       size_t count, cudaStream_t stream, bool shared = false);
 int launch_matvec_fq(const NttPlanDev &plan, int32_t *out, const int32_t *A, const int32_t *s, int k, int l,
-                     size_t count, cudaStream_t stream);
+                     size_t count, cudaStream_t stream, bool shared = false);
 int build_sq_tables(NttPlanDev &plan, const int32_t *w_host);
 void free_sq_tables(NttPlanDev &plan);
 int launch_polymul_sq(const NttPlanDev &plan, int mode, int32_t *out, const int32_t *a, const void *b,
                       size_t b_stride, size_t count, cudaStream_t stream);
 int launch_matvec_sq(const NttPlanDev &plan, int32_t *out, const int32_t *A, const int32_t *s, int k, int l,
-                     size_t count, cudaStream_t stream);
+                     size_t count, cudaStream_t stream, bool shared = false);
 
 }  // namespace scgpu

@@ -334,6 +334,14 @@ extern "C" int scgpu_matvec_batch(const scgpu_ntt_plan_t *plan, int32_t *out, co
     return launch_matvec(plan->dev, out, A, s, k, l, count, static_cast<cudaStream_t>(stream));
 }
 
+extern "C" int scgpu_matvec_shared_batch(const scgpu_ntt_plan_t *plan, int32_t *out, const int32_t *A,
+                                         const int32_t *s, int k, int l, size_t count, void *stream)
+{
+    if (!plan || !out || !A || !s) { set_error("matvec_shared_batch: null argument"); return SCGPU_ERR_ARG; }
+    SCGPU_CUDA_CHECK(cudaSetDevice(plan->dev.device));
+    return launch_matvec(plan->dev, out, A, s, k, l, count, static_cast<cudaStream_t>(stream), true);
+}
+
 // ---- module product with the matrix sampled on the device (rand_product.cu) ----------------------------------------
 
 static int check_rand_args(const char *what, int prng_type, size_t seed_len, int n, int k, int l)
@@ -396,11 +404,37 @@ extern "C" int scgpu_rand_product_csprng_batch(const scgpu_ntt_plan_t *plan, int
     return e;
 }
 
-extern "C" int scgpu_rand_product_csprng_batch_host(const scgpu_ntt_plan_t *plan, int32_t *t, const int32_t *y, const uint8_t *seeds,
-                                                    size_t seed_len, int prng_type, uint32_t q_bits, int k, int l, int transpose,
-                                                    size_t count)
+extern "C" int scgpu_rand_product_csprng_shared_batch(const scgpu_ntt_plan_t *plan, int32_t *t, const int32_t *y, const uint8_t *seed,
+                                                      size_t seed_len, int prng_type, uint32_t q_bits, int k, int l, int transpose,
+                                                      size_t count, void *stream)
 {
-    if (!plan || !t || !y || !seeds) { set_error("rand_product_host: null argument"); return SCGPU_ERR_ARG; }
+    if (!plan || !t || !y || !seed) { set_error("rand_product_shared: null argument"); return SCGPU_ERR_ARG; }
+    if (!plan->dev.w || !plan->dev.r) { set_error("rand_product_shared: the plan has no twiddle tables"); return SCGPU_ERR_ARG; }
+    const int n = plan->dev.n;
+    int e = check_rand_args("rand_product_shared", prng_type, seed_len, n, k, l);
+    if (e != SCGPU_OK) return e;
+    if (transpose && plan->dev.tw_bits == 32 && l > 1) {
+        set_error("rand_product_shared: create_rand_product_32_csprng's transposed branch adds the matrix ring instead of the running "
+                  "sum (module_lwe.c:623-628); no scheme calls it and it is not reproduced");
+        return SCGPU_ERR_UNSUPPORTED;
+    }
+    if (count == 0) return SCGPU_OK;
+    SCGPU_CUDA_CHECK(cudaSetDevice(plan->dev.device));
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    // one seed: the matrix is drawn once, then the whole batch runs the shared-matrix product (no chunking)
+    int32_t *scratch = nullptr;
+    SCGPU_CUDA_CHECK(cudaMallocAsync(&scratch, (size_t)k * l * n * sizeof(int32_t), st));
+    e = launch_gen_rings(prng_type, seed, seed_len, 1, scratch, n, k, l, transpose, plan->dev.rc.q, q_bits, st);
+    if (e == SCGPU_OK) e = launch_matvec(plan->dev, t, scratch, y, k, l, count, st, true);
+    SCGPU_CUDA_CHECK(cudaFreeAsync(scratch, st));
+    return e;
+}
+
+// three-stream pipeline over chunks of instances: y (and the seeds) in, t out; the matrix never crosses the bus.
+// shared: ONE seed for every instance, copied once
+static int rand_product_host(const scgpu_ntt_plan_t *plan, int32_t *t, const int32_t *y, const uint8_t *seeds, size_t seed_len,
+                             int prng_type, uint32_t q_bits, int k, int l, int transpose, size_t count, bool shared)
+{
     if (count == 0) return SCGPU_OK;
     scgpu_ntt_plan *p = const_cast<scgpu_ntt_plan *>(plan);
     std::lock_guard<std::mutex> lock(p->mu);
@@ -415,23 +449,33 @@ extern "C" int scgpu_rand_product_csprng_batch_host(const scgpu_ntt_plan_t *plan
     if (rows > count) rows = count;
     int status = SCGPU_OK;
     void *dy[scgpu_ntt_plan::kStreams] = {}, *dt[scgpu_ntt_plan::kStreams] = {}, *ds[scgpu_ntt_plan::kStreams] = {};
+    void *dseed = nullptr;                                   // shared: the one seed, read by every stream
     auto cuda_ok = [&](cudaError_t e, const char *what) {
         if (e != cudaSuccess && status == SCGPU_OK) { set_error("%s failed: %s", what, cudaGetErrorString(e)); status = SCGPU_ERR_CUDA; }
         return e == cudaSuccess;
     };
+    if (shared && cuda_ok(cudaMallocAsync(&dseed, seed_len, p->streams[0]), "cudaMallocAsync")
+        && cuda_ok(cudaMemcpyAsync(dseed, seeds, seed_len, cudaMemcpyHostToDevice, p->streams[0]), "H2D copy"))
+        cuda_ok(cudaStreamSynchronize(p->streams[0]), "cudaStreamSynchronize");
     for (int i = 0; i < scgpu_ntt_plan::kStreams && status == SCGPU_OK; i++) {
         cuda_ok(cudaMallocAsync(&dy[i], rows * yb, p->streams[i]), "cudaMallocAsync");
         cuda_ok(cudaMallocAsync(&dt[i], rows * tb, p->streams[i]), "cudaMallocAsync");
-        cuda_ok(cudaMallocAsync(&ds[i], rows * seed_len, p->streams[i]), "cudaMallocAsync");
+        if (!shared) cuda_ok(cudaMallocAsync(&ds[i], rows * seed_len, p->streams[i]), "cudaMallocAsync");
     }
     for (size_t off = 0, ci = 0; off < count && status == SCGPU_OK; off += rows, ci++) {
         const int s = (int)(ci % scgpu_ntt_plan::kStreams);
         cudaStream_t st = p->streams[s];
         const size_t cnt = count - off < rows ? count - off : rows;
         if (!cuda_ok(cudaMemcpyAsync(dy[s], reinterpret_cast<const char *>(y) + off * yb, cnt * yb, cudaMemcpyHostToDevice, st), "H2D copy")) break;
-        if (!cuda_ok(cudaMemcpyAsync(ds[s], seeds + off * seed_len, cnt * seed_len, cudaMemcpyHostToDevice, st), "H2D copy")) break;
-        const int e = scgpu_rand_product_csprng_batch(plan, static_cast<int32_t *>(dt[s]), static_cast<const int32_t *>(dy[s]),
-                                                      static_cast<const uint8_t *>(ds[s]), seed_len, prng_type, q_bits, k, l, transpose, cnt, st);
+        int e;
+        if (shared) {
+            e = scgpu_rand_product_csprng_shared_batch(plan, static_cast<int32_t *>(dt[s]), static_cast<const int32_t *>(dy[s]),
+                                                       static_cast<const uint8_t *>(dseed), seed_len, prng_type, q_bits, k, l, transpose, cnt, st);
+        } else {
+            if (!cuda_ok(cudaMemcpyAsync(ds[s], seeds + off * seed_len, cnt * seed_len, cudaMemcpyHostToDevice, st), "H2D copy")) break;
+            e = scgpu_rand_product_csprng_batch(plan, static_cast<int32_t *>(dt[s]), static_cast<const int32_t *>(dy[s]),
+                                                static_cast<const uint8_t *>(ds[s]), seed_len, prng_type, q_bits, k, l, transpose, cnt, st);
+        }
         if (e != SCGPU_OK) { status = e; break; }
         cuda_ok(cudaMemcpyAsync(reinterpret_cast<char *>(t) + off * tb, dt[s], cnt * tb, cudaMemcpyDeviceToHost, st), "D2H copy");
     }
@@ -442,7 +486,27 @@ extern "C" int scgpu_rand_product_csprng_batch_host(const scgpu_ntt_plan_t *plan
         if (ds[i]) cudaFreeAsync(ds[i], p->streams[i]);
         cuda_ok(cudaStreamSynchronize(p->streams[i]), "cudaStreamSynchronize");
     }
+    if (dseed) {                                             // every stream has drained: nobody reads the seed any more
+        cudaFreeAsync(dseed, p->streams[0]);
+        cuda_ok(cudaStreamSynchronize(p->streams[0]), "cudaStreamSynchronize");
+    }
     return status;
+}
+
+extern "C" int scgpu_rand_product_csprng_batch_host(const scgpu_ntt_plan_t *plan, int32_t *t, const int32_t *y, const uint8_t *seeds,
+                                                    size_t seed_len, int prng_type, uint32_t q_bits, int k, int l, int transpose,
+                                                    size_t count)
+{
+    if (!plan || !t || !y || !seeds) { set_error("rand_product_host: null argument"); return SCGPU_ERR_ARG; }
+    return rand_product_host(plan, t, y, seeds, seed_len, prng_type, q_bits, k, l, transpose, count, false);
+}
+
+extern "C" int scgpu_rand_product_csprng_shared_batch_host(const scgpu_ntt_plan_t *plan, int32_t *t, const int32_t *y,
+                                                           const uint8_t *seed, size_t seed_len, int prng_type, uint32_t q_bits,
+                                                           int k, int l, int transpose, size_t count)
+{
+    if (!plan || !t || !y || !seed) { set_error("rand_product_shared_host: null argument"); return SCGPU_ERR_ARG; }
+    return rand_product_host(plan, t, y, seed, seed_len, prng_type, q_bits, k, l, transpose, count, true);
 }
 
 // ---- host-buffer entry points: chunked three-stream pipeline -----------------------------------------

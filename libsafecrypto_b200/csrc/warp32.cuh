@@ -787,7 +787,8 @@ k_ntt_w32(int32_t *__restrict__ out, const int32_t *__restrict__ a, size_t count
 // brev5(e) * (n/32) + brev(tau) of the row (ntt_index), so for a fixed e the lanes of an instance read n/32
 // consecutive words: conflict-free from the staging row (instances 8 banks apart), one full sector from HBM
 // in the LDG variant.
-template <class AR, int LOGN, bool TMA, bool CHK = true>
+// SHARED_A: one matrix [k][l][n] for every instance (scgpu_matvec_shared_batch), addressed with an instance stride of 0
+template <class AR, int LOGN, bool TMA, bool CHK = true, bool SHARED_A = false>
 __global__ void __launch_bounds__(kThreads32)
 k_matvec_w32(int32_t *__restrict__ out, const int32_t *__restrict__ A, const int32_t *__restrict__ s,
               int k, int l, size_t count, unsigned long long *ctr, const __grid_constant__ W32Const<AR> c)
@@ -830,7 +831,7 @@ k_matvec_w32(int32_t *__restrict__ out, const int32_t *__restrict__ A, const int
         for (int p = 0; p < C::PW; p++) {
             size_t row = nbase + (size_t)warp * C::PW + p;
             if (row >= count) row = 0;
-            bulk_g2s(dst + (warp * C::PW + p) * AROW, A + (row * k * l + step) * N, ROW_BYTES, &bars[warp][1 + which]);
+            bulk_g2s(dst + (warp * C::PW + p) * AROW, A + ((SHARED_A ? (size_t)0 : row * k * l) + step) * N, ROW_BYTES, &bars[warp][1 + which]);
         }
     };
     const size_t first = (size_t)blockIdx.x * C::POLYS;
@@ -913,7 +914,7 @@ k_matvec_w32(int32_t *__restrict__ out, const int32_t *__restrict__ A, const int
                         }
                     }
                 } else {
-                    const int32_t *arow = A + ((irow * k + i) * l + j) * N + taurev;
+                    const int32_t *arow = A + (((SHARED_A ? (size_t)0 : irow * k) + i) * l + j) * N + taurev;
 #pragma unroll
                     for (int e = 0; e < 32; e++) {
                         av[e] = __ldg(arow + (int)((__brev((unsigned)e) >> 27) << (LOGN - 5)));
@@ -981,6 +982,57 @@ k_matvec_w32(int32_t *__restrict__ out, const int32_t *__restrict__ A, const int
 }
 
 
+// ---- one matrix for the whole launch (scgpu_matvec_shared_batch) --------------------------------------------------
+// With SHARED_A, k_matvec_rows_w32 and k_matvec16_w32 take the matrix from a table that k_matrix_table writes once per
+// launch: every coefficient reduced to its centred residue (|a| <= q/2, inside every range window, so the kernels drop
+// the range vote on it), each of the k l rows in thread-major order.  128-bit word v of thread tau of row r sits at
+// (r V + v) T + tau and holds the thread's elements e = EW v .. EW v + EW - 1 (EW = 16 / sizeof(TE), V = 32 / EW), so
+// for a fixed v the lanes of an instance read T consecutive 16-byte words -- the layout of the pass-1 twiddle tables.
+// The table (8-16 KiB at Kyber's int16, up to 30 KiB at Dilithium's int32) stays in L1 / L2: only the s rows come from
+// HBM.  The AR parameter only keeps the instantiations of the two policies' translation units apart.
+template <class AR, class TE>
+__global__ void k_matrix_table(TE *__restrict__ tab, const int32_t *__restrict__ A, int rows, int32_t q)
+{
+    using C = Cfg32<8>;
+    constexpr int EW = 16 / (int)sizeof(TE), V = 32 / EW;
+    const int t = blockIdx.x * blockDim.x + threadIdx.x;
+    if (t >= rows * V * C::T) return;
+    const int tau = t % C::T, v = (t / C::T) % V, r = t / (C::T * V);
+    const int taurev = (int)(__brev((unsigned)tau) >> (32 - 3));
+    alignas(16) TE w[EW];
+#pragma unroll
+    for (int u = 0; u < EW; u++) {
+        const int e = v * EW + u;
+        int32_t x = A[(size_t)r * C::N + taurev + (int)((__brev((unsigned)e) >> 27) << 3)] % q;
+        if (x < 0) x += q;
+        if (x > q / 2) x -= q;
+        w[u] = (TE)x;
+    }
+    reinterpret_cast<int4 *>(tab)[t] = *reinterpret_cast<const int4 *>(w);
+}
+
+// the 32 elements of thread tau in row r of a k_matrix_table table (n = 256)
+template <class TE>
+__device__ __forceinline__ void load_table_row(int32_t (&av)[32], const int32_t *tab, int r, int tau)
+{
+    constexpr int T = Cfg32<8>::T, EW = 16 / (int)sizeof(TE), V = 32 / EW;
+    const int4 *p = reinterpret_cast<const int4 *>(tab) + r * V * T + tau;
+#pragma unroll
+    for (int v = 0; v < V; v++) {
+        const int4 w = __ldg(p + v * T);
+        const int32_t wd[4] = {w.x, w.y, w.z, w.w};
+#pragma unroll
+        for (int u = 0; u < 4; u++) {
+            if constexpr (sizeof(TE) == 2) {
+                av[8 * v + 2 * u] = (int32_t)(int16_t)(wd[u] & 0xFFFF);
+                av[8 * v + 2 * u + 1] = wd[u] >> 16;
+            } else {
+                av[4 * v + u] = wd[u];
+            }
+        }
+    }
+}
+
 // ---- mat-vec, one warp per OUTPUT ROW: the k warps of a CTA share the transformed vectors ------------------------
 // k_matvec_w32 keeps l full 32-bit tiles per instance for ONE warp: 8 one-warp CTAs per SM at l = 4, two warps per
 // scheduler, and the kernel is bound by fixed-latency dependencies (issue slots 41 % used, profiles/dil_matvec_r2g_ncu.json).
@@ -989,7 +1041,8 @@ k_matvec_w32(int32_t *__restrict__ out, const int32_t *__restrict__ A, const int
 // exchange tile and staging row (two matrix rows in flight per warp, as above).  Shared memory per warp falls from
 // l + 2 to l / k + 2 tiles: 15 warps per SM at k = 5, l = 4.  The s rows of the next group can only be requested after
 // every warp has left the stash (second barrier); the matrix rows of the next group are requested before it.
-template <class AR, int LOGN, bool CHK = true>
+// SHARED_A: the matrix is a k_matrix_table table (int32) read by 128-bit loads; no staging rows, no mbarrier per row.
+template <class AR, int LOGN, bool CHK = true, bool SHARED_A = false>
 __global__ void __launch_bounds__(256, 2)
 k_matvec_rows_w32(int32_t *__restrict__ out, const int32_t *__restrict__ A, const int32_t *__restrict__ s,
                   int k, int l, size_t count, unsigned long long *ctr, const __grid_constant__ W32Const<AR> c)
@@ -999,6 +1052,7 @@ k_matvec_rows_w32(int32_t *__restrict__ out, const int32_t *__restrict__ A, cons
     constexpr int N = C::N, T = C::T, SUB = C::SUB, NSUB = C::NSUB, PW = C::PW;
     constexpr int AROW = N + T;
     constexpr int TILE = PW * C::TS;                                 // one tile per instance of the group
+    constexpr int WARP_WORDS = SHARED_A ? TILE : TILE + PW * AROW;  // per warp: exchange tile (+ staging rows)
     constexpr uint32_t ROW_BYTES = (uint32_t)N * 4u;
     extern __shared__ __align__(16) int32_t dyn_tiles[];             // [l][PW][TS] stash | per warp: [PW][TS] | [PW][AROW]
     __shared__ __align__(8) uint64_t bar_s;                          // the s rows of a group (whole CTA)
@@ -1009,7 +1063,7 @@ k_matvec_rows_w32(int32_t *__restrict__ out, const int32_t *__restrict__ A, cons
     const int nw = blockDim.x / 32;                                  // = k
     const int tau = lane % T;
     const int slot = lane / T;
-    int32_t *mine = dyn_tiles + (size_t)l * TILE + (size_t)warp * (TILE + PW * AROW);
+    int32_t *mine = dyn_tiles + (size_t)l * TILE + (size_t)warp * WARP_WORDS;
     int32_t *xt = mine + slot * C::TS;
     const int32_t *astage = mine + TILE + slot * AROW;
     const int32_t *xstage = mine + slot * AROW;
@@ -1044,7 +1098,7 @@ k_matvec_rows_w32(int32_t *__restrict__ out, const int32_t *__restrict__ A, cons
     __syncthreads();
     if ((size_t)g * PW < count) {
         if (threadIdx.x == 0) fetch_s((size_t)g * PW);
-        if (lane == 0) { fetch_a((size_t)g * PW, warp * l, 0); if (l >= 2) fetch_a((size_t)g * PW, warp * l + 1, 1); }
+        if (!SHARED_A && lane == 0) { fetch_a((size_t)g * PW, warp * l, 0); if (l >= 2) fetch_a((size_t)g * PW, warp * l + 1, 1); }
     }
 
     while ((size_t)g * PW < count) {
@@ -1089,22 +1143,26 @@ k_matvec_rows_w32(int32_t *__restrict__ out, const int32_t *__restrict__ A, cons
             for (int j = 0; j < l; j++) {
                 int32_t av[32];
                 bool wide = false;
-                const int which = j & 1;
-                if (which) { mbar_wait(&bars[warp][1], par_a1); par_a1 ^= 1u; }
-                else       { mbar_wait(&bars[warp][0], par_a0); par_a0 ^= 1u; }
-                const int32_t *arow = which ? xstage : astage;
+                if constexpr (SHARED_A) {
+                    load_table_row<int32_t>(av, A, i * l + j, tau);
+                } else {
+                    const int which = j & 1;
+                    if (which) { mbar_wait(&bars[warp][1], par_a1); par_a1 ^= 1u; }
+                    else       { mbar_wait(&bars[warp][0], par_a0); par_a0 ^= 1u; }
+                    const int32_t *arow = which ? xstage : astage;
 #pragma unroll
-                for (int e = 0; e < 32; e++) {
-                    av[e] = arow[taurev + (int)((__brev((unsigned)e) >> 27) << (LOGN - 5))];
-                    if (CHK) wide |= W::out_of_range(av[e], c);
+                    for (int e = 0; e < 32; e++) {
+                        av[e] = arow[taurev + (int)((__brev((unsigned)e) >> 27) << (LOGN - 5))];
+                        if (CHK) wide |= W::out_of_range(av[e], c);
+                    }
+                    fence_proxy_async();
+                    __syncwarp();
+                    if (lane == 0) {
+                        if (j + 2 < l) fetch_a(base, i * l + j + 2, which);
+                        else if (!which && nbase < count) fetch_a(nbase, i * l, 0);  // this warp's row of the next group
+                    }
                 }
-                fence_proxy_async();
-                __syncwarp();
-                if (lane == 0) {
-                    if (j + 2 < l) fetch_a(base, i * l + j + 2, which);
-                    else if (!which && nbase < count) fetch_a(nbase, i * l, 0);      // this warp's row of the next group
-                }
-                if (CHK && __any_sync(0xFFFFFFFFu, wide)) {
+                if (!SHARED_A && CHK && __any_sync(0xFFFFFFFFu, wide)) {
 #pragma unroll
                     for (int e = 0; e < 32; e++) av[e] = W::bred(av[e], c);
                 }
@@ -1145,7 +1203,7 @@ k_matvec_rows_w32(int32_t *__restrict__ out, const int32_t *__restrict__ A, cons
                     for (int m = 0; m < 32; m++) orow[tau + m * T] = (int32_t)x[m];
                 }
             }
-            if (l >= 2) {
+            if (!SHARED_A && l >= 2) {
                 fence_proxy_async();
                 __syncwarp();
                 if (lane == 0 && nbase < count) fetch_a(nbase, i * l + 1, 1);
@@ -1169,7 +1227,9 @@ k_matvec_rows_w32(int32_t *__restrict__ out, const int32_t *__restrict__ A, cons
 // IACC: the l products of an output coefficient cannot leave 32 bits (l |a| |s| < 2^31 with |a| <= x0 and the stash
 // reduced to |s| <= 0.55 q), so they are summed by plain IMADs and the quotient comes from ONE conversion of the sum --
 // instead of an IMAD, an FFMA and two conversions per term (AR::Acc), and in 32 instead of 64 accumulator registers.
-template <class AR, int LOGN, bool TMA, bool CHK = true, bool IACC = false>
+// SHARED_A (with TMA): the matrix is a k_matrix_table table (int16) read by 128-bit loads; only the s rows travel
+// through the staging row, and s_0 of the warp's next instances is put in flight as soon as s_{l-1} is in registers.
+template <class AR, int LOGN, bool TMA, bool CHK = true, bool IACC = false, bool SHARED_A = false>
 __global__ void __launch_bounds__(kThreads32, 16)        // 128 registers: 4 warps per scheduler fit (140 allowed 3)
 k_matvec16_w32(int32_t *__restrict__ out, const int32_t *__restrict__ A, const int32_t *__restrict__ s,
                int k, int l, size_t count, unsigned long long *ctr, const __grid_constant__ W32Const<AR> c)
@@ -1209,7 +1269,7 @@ k_matvec16_w32(int32_t *__restrict__ out, const int32_t *__restrict__ A, const i
         for (int p = 0; p < C::PW; p++) {
             size_t inst = nbase + (size_t)warp * C::PW + p;
             if (inst >= count) inst = 0;
-            const int32_t *src = r < l ? s + (inst * l + r) * N : A + (inst * k * l + (r - l)) * N;
+            const int32_t *src = (SHARED_A || r < l) ? s + (inst * l + r) * N : A + (inst * k * l + (r - l)) * N;
             bulk_g2s(dst + (warp * C::PW + p) * AROW, src, ROW_BYTES, &bars[warp][which]);
         }
     };
@@ -1253,7 +1313,7 @@ k_matvec16_w32(int32_t *__restrict__ out, const int32_t *__restrict__ A, const i
             if (TMA) {
                 mbar_wait(&bars[warp][0], par_s); par_s ^= 1u;
                 W::template load_operand_staged<LOGN, CHK>(x, stage, tau, c);
-                advance_s(j + 1);                                    // s row j + 1, or matrix row (0, 0) = number l
+                advance_s(SHARED_A && j + 1 == l ? -1 : j + 1);      // s row j + 1, or matrix row (0, 0) = number l
             } else {
                 W::template load_operand<LOGN, CHK>(x, s + (irow * l + j) * N, tau, c);
             }
@@ -1280,7 +1340,7 @@ k_matvec16_w32(int32_t *__restrict__ out, const int32_t *__restrict__ A, const i
             }
             __syncwarp();                                            // the exchange tile is reused by the next vector
         }
-        if (TMA && l >= 2) {
+        if (!SHARED_A && TMA && l >= 2) {
             // the exchange tile is free until the first inverse transform: matrix row (0, 1) into X
             fence_proxy_async();
             __syncwarp();
@@ -1296,7 +1356,9 @@ k_matvec16_w32(int32_t *__restrict__ out, const int32_t *__restrict__ A, const i
             for (int j = 0; j < l; j++) {
                 int32_t av[32];
                 bool wide = false;
-                if (TMA) {
+                if constexpr (SHARED_A) {
+                    load_table_row<int16_t>(av, A, i * l + j, tau);
+                } else if (TMA) {
                     const int which = j & 1;
                     if (which) { mbar_wait(&bars[warp][1], par_x); par_x ^= 1u; }
                     else       { mbar_wait(&bars[warp][0], par_s); par_s ^= 1u; }
@@ -1321,7 +1383,7 @@ k_matvec16_w32(int32_t *__restrict__ out, const int32_t *__restrict__ A, const i
                         if (CHK) wide |= W::out_of_range(av[e], c);
                     }
                 }
-                if (CHK && __any_sync(0xFFFFFFFFu, wide)) {
+                if (!SHARED_A && CHK && __any_sync(0xFFFFFFFFu, wide)) {
 #pragma unroll
                     for (int e = 0; e < 32; e++) av[e] = W::bred(av[e], c);
                 }
@@ -1369,7 +1431,7 @@ k_matvec16_w32(int32_t *__restrict__ out, const int32_t *__restrict__ A, const i
                     for (int m = 0; m < 32; m++) orow[tau + m * T] = (int32_t)x[m];
                 }
             }
-            if (TMA && l >= 2 && i + 1 < k) {
+            if (!SHARED_A && TMA && l >= 2 && i + 1 < k) {
                 // the exchange tile is free again: column 1 of the next output row into X
                 fence_proxy_async();
                 __syncwarp();
@@ -1524,13 +1586,43 @@ int launch_ntt_w32(const W32Const<AR> &c, int logn, int sm_count, int inverse, i
     return SCGPU_OK;
 }
 
-// n = 256 (Kyber, Dilithium)
+// One shared matrix: its k_matrix_table table in a stream-ordered scratch of the call (not of the plan: two streams may
+// run shared products with different matrices on one plan), written once before the batch kernel.
+template <class AR, class TE>
+int matrix_table(const W32Const<AR> &c, const int32_t *A, int rows, cudaStream_t st, int32_t **tab)
+{
+    const size_t words = (size_t)rows * Cfg32<8>::N * sizeof(TE) / 16;          // one thread per 128-bit word
+    SCGPU_CUDA_CHECK(cudaMallocAsync(reinterpret_cast<void **>(tab), words * 16, st));
+    k_matrix_table<AR, TE><<<(unsigned)((words + 127) / 128), 128, 0, st>>>(reinterpret_cast<TE *>(*tab), A, rows, c.q);
+    count_launch();
+    const cudaError_t e = cudaGetLastError();
+    if (e != cudaSuccess) {
+        cudaFreeAsync(*tab, st);
+        set_error("k_matrix_table launch failed: %s", cudaGetErrorString(e));
+        return SCGPU_ERR_CUDA;
+    }
+    return SCGPU_OK;
+}
+
+// the batch kernel has been launched (or refused): check it, release the table in stream order
+inline int launched_with_table(int32_t *tab, cudaStream_t st)
+{
+    const cudaError_t e = cudaGetLastError();
+    const cudaError_t fe = tab ? cudaFreeAsync(tab, st) : cudaSuccess;
+    if (e != cudaSuccess) { set_error("matvec launch failed: %s", cudaGetErrorString(e)); return SCGPU_ERR_CUDA; }
+    if (fe != cudaSuccess) { set_error("cudaFreeAsync failed: %s", cudaGetErrorString(fe)); return SCGPU_ERR_CUDA; }
+    return SCGPU_OK;
+}
+
+// n = 256 (Kyber, Dilithium).  shared: A is ONE matrix [k][l][n] for every instance (scgpu_matvec_shared_batch)
 template <class AR>
 int launch_matvec_w32(const W32Const<AR> &c, int sm_count, int32_t *out, const int32_t *A, const int32_t *s, int k, int l,
-                      size_t count, cudaStream_t st, bool chk = true)
+                      size_t count, cudaStream_t st, bool chk = true, bool shared = false)
 {
     using C = Cfg32<8>;
     const bool tma = ((uintptr_t)A % 16) == 0 && ((uintptr_t)s % 16) == 0 && tma_allowed();
+    // the kernels below that read a shared matrix from its table stage only the s rows
+    const bool tma_rows = shared ? ((uintptr_t)s % 16) == 0 && tma_allowed() : tma;
     const int sms = sm_count > 0 ? sm_count : 148;
     const size_t groups = (count + C::POLYS - 1) / C::POLYS;
     unsigned long long *ctr = nullptr;
@@ -1541,17 +1633,26 @@ int launch_matvec_w32(const W32Const<AR> &c, int sm_count, int32_t *out, const i
     // the rows are not prefetched at all and the 32-bit stash kernel is used.  SCGPU_MATVEC16_MINL raises the threshold.
     const char *minl_env = getenv("SCGPU_MATVEC16_MINL");
     const int minl = minl_env ? atoi(minl_env) : 1;
-    if (AR::STASH16 && c.q < 59000 && l >= minl && tma && !(no16 && atoi(no16) != 0)) {
+    if (AR::STASH16 && c.q < 59000 && l >= minl && tma_rows && !(no16 && atoi(no16) != 0)) {
         const size_t smem = ((size_t)C::POLYS * (C::TS + (C::N + C::T)) + (size_t)l * C::POLYS * (20 * C::T + C::T)) * sizeof(int32_t);
         // integer accumulators: l |a| |s| < 2^31 with |a| <= x0 (the range vote's window, also what the flag promises) and
         // |s| <= 0.55 q + 2 (the reduced stash)
         const char *facc = getenv("SCGPU_MATVEC_FLOAT_ACC");
         const bool iacc = (double)l * (double)c.x0 * (0.55 * (double)c.q + 2.0) < 2147483648.0 && !(facc && atoi(facc) != 0);
-        SCGPU_CUDA_CHECK(cudaFuncSetAttribute(k_matvec16_w32<AR, 8, true, true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
-        SCGPU_CUDA_CHECK(cudaFuncSetAttribute(k_matvec16_w32<AR, 8, true, false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
-        if constexpr (AR::STASH16) {
-            SCGPU_CUDA_CHECK(cudaFuncSetAttribute(k_matvec16_w32<AR, 8, true, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
-            SCGPU_CUDA_CHECK(cudaFuncSetAttribute(k_matvec16_w32<AR, 8, true, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
+        if (shared) {
+            if constexpr (AR::STASH16) {
+                SCGPU_CUDA_CHECK(cudaFuncSetAttribute(k_matvec16_w32<AR, 8, true, true, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
+                SCGPU_CUDA_CHECK(cudaFuncSetAttribute(k_matvec16_w32<AR, 8, true, false, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
+                SCGPU_CUDA_CHECK(cudaFuncSetAttribute(k_matvec16_w32<AR, 8, true, true, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
+                SCGPU_CUDA_CHECK(cudaFuncSetAttribute(k_matvec16_w32<AR, 8, true, false, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
+            }
+        } else {
+            SCGPU_CUDA_CHECK(cudaFuncSetAttribute(k_matvec16_w32<AR, 8, true, true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
+            SCGPU_CUDA_CHECK(cudaFuncSetAttribute(k_matvec16_w32<AR, 8, true, false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
+            if constexpr (AR::STASH16) {
+                SCGPU_CUDA_CHECK(cudaFuncSetAttribute(k_matvec16_w32<AR, 8, true, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
+                SCGPU_CUDA_CHECK(cudaFuncSetAttribute(k_matvec16_w32<AR, 8, true, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
+            }
         }
         int per_sm = (int)((227 * 1024) / (smem + 1024 + 64));
         if (per_sm > 16) per_sm = 16;
@@ -1560,6 +1661,19 @@ int launch_matvec_w32(const W32Const<AR> &c, int sm_count, int32_t *out, const i
         if (grid > groups) grid = groups;
         if (!groups_fit(groups, grid)) { set_error("batch of %zu rows is too large", count); return SCGPU_ERR_ARG; }
         if (groups > grid) { const int e = next_work_counter(st, &ctr, 2); if (e != SCGPU_OK) return e; }
+        if (shared) {
+            if constexpr (AR::STASH16) {
+                int32_t *tab = nullptr;
+                const int e = matrix_table<AR, int16_t>(c, A, k * l, st, &tab);
+                if (e != SCGPU_OK) return e;
+                if (iacc && chk) k_matvec16_w32<AR, 8, true, true, true, true><<<(unsigned)grid, kThreads32, smem, st>>>(out, tab, s, k, l, count, ctr, c);
+                else if (iacc)   k_matvec16_w32<AR, 8, true, false, true, true><<<(unsigned)grid, kThreads32, smem, st>>>(out, tab, s, k, l, count, ctr, c);
+                else if (chk)    k_matvec16_w32<AR, 8, true, true, false, true><<<(unsigned)grid, kThreads32, smem, st>>>(out, tab, s, k, l, count, ctr, c);
+                else             k_matvec16_w32<AR, 8, true, false, false, true><<<(unsigned)grid, kThreads32, smem, st>>>(out, tab, s, k, l, count, ctr, c);
+                count_launch();
+                return launched_with_table(tab, st);
+            }
+        }
         bool launched = false;
         if constexpr (AR::STASH16) {
             if (iacc) {
@@ -1577,12 +1691,19 @@ int launch_matvec_w32(const W32Const<AR> &c, int sm_count, int32_t *out, const i
         return SCGPU_OK;
     }
     {
-        // one warp per output row (k_matvec_rows_w32): aligned rows, 2 <= k <= 8; SCGPU_MATVEC_ONE_WARP=1 keeps k_matvec_w32
+        // one warp per output row (k_matvec_rows_w32): aligned rows, 2 <= k <= 8; SCGPU_MATVEC_ONE_WARP=1 keeps k_matvec_w32.
+        // A shared matrix needs no staging rows: each warp keeps only its exchange tile
         const char *ow = getenv("SCGPU_MATVEC_ONE_WARP");
-        const size_t smem_rows = ((size_t)l * C::PW * C::TS + (size_t)k * (C::PW * C::TS + C::PW * (C::N + C::T))) * sizeof(int32_t);
-        if (tma && k >= 2 && k <= 8 && smem_rows <= 110 * 1024 && !(ow && atoi(ow) != 0)) {
-            SCGPU_CUDA_CHECK(cudaFuncSetAttribute(k_matvec_rows_w32<AR, 8, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
-            SCGPU_CUDA_CHECK(cudaFuncSetAttribute(k_matvec_rows_w32<AR, 8, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
+        const size_t warp_words = shared ? (size_t)C::PW * C::TS : (size_t)C::PW * C::TS + C::PW * (C::N + C::T);
+        const size_t smem_rows = ((size_t)l * C::PW * C::TS + (size_t)k * warp_words) * sizeof(int32_t);
+        if (tma_rows && k >= 2 && k <= 8 && smem_rows <= 110 * 1024 && !(ow && atoi(ow) != 0)) {
+            if (shared) {
+                SCGPU_CUDA_CHECK(cudaFuncSetAttribute(k_matvec_rows_w32<AR, 8, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
+                SCGPU_CUDA_CHECK(cudaFuncSetAttribute(k_matvec_rows_w32<AR, 8, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
+            } else {
+                SCGPU_CUDA_CHECK(cudaFuncSetAttribute(k_matvec_rows_w32<AR, 8, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
+                SCGPU_CUDA_CHECK(cudaFuncSetAttribute(k_matvec_rows_w32<AR, 8, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
+            }
             const size_t rgroups = (count + C::PW - 1) / C::PW;
             int per_sm = (int)((227 * 1024) / (smem_rows + 1024 + 256));
             const int by_regs = 65536 / (k * 32 * 128);
@@ -1592,6 +1713,15 @@ int launch_matvec_w32(const W32Const<AR> &c, int sm_count, int32_t *out, const i
             if (grid > rgroups) grid = rgroups;
             if (!groups_fit(rgroups, grid)) { set_error("batch of %zu rows is too large", count); return SCGPU_ERR_ARG; }
             if (rgroups > grid) { const int e = next_work_counter(st, &ctr, 1); if (e != SCGPU_OK) return e; }
+            if (shared) {
+                int32_t *tab = nullptr;
+                const int e = matrix_table<AR, int32_t>(c, A, k * l, st, &tab);
+                if (e != SCGPU_OK) return e;
+                if (chk) k_matvec_rows_w32<AR, 8, true, true><<<(unsigned)grid, 32 * k, smem_rows, st>>>(out, tab, s, k, l, count, ctr, c);
+                else     k_matvec_rows_w32<AR, 8, false, true><<<(unsigned)grid, 32 * k, smem_rows, st>>>(out, tab, s, k, l, count, ctr, c);
+                count_launch();
+                return launched_with_table(tab, st);
+            }
             if (chk) k_matvec_rows_w32<AR, 8, true><<<(unsigned)grid, 32 * k, smem_rows, st>>>(out, A, s, k, l, count, ctr, c);
             else     k_matvec_rows_w32<AR, 8, false><<<(unsigned)grid, 32 * k, smem_rows, st>>>(out, A, s, k, l, count, ctr, c);
             count_launch();
@@ -1601,7 +1731,15 @@ int launch_matvec_w32(const W32Const<AR> &c, int sm_count, int32_t *out, const i
     }
     const size_t smem = ((size_t)(l + 1) * C::POLYS * C::TS + (tma ? (size_t)C::POLYS * (C::N + C::T) : 0)) * sizeof(int32_t);
     // per launch, not once: the attribute belongs to the current device's context and plans exist per device
-    if (tma) {
+    if (shared) {
+        if (tma) {
+            SCGPU_CUDA_CHECK(cudaFuncSetAttribute(k_matvec_w32<AR, 8, true, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
+            SCGPU_CUDA_CHECK(cudaFuncSetAttribute(k_matvec_w32<AR, 8, true, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
+        } else {
+            SCGPU_CUDA_CHECK(cudaFuncSetAttribute(k_matvec_w32<AR, 8, false, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
+            SCGPU_CUDA_CHECK(cudaFuncSetAttribute(k_matvec_w32<AR, 8, false, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
+        }
+    } else if (tma) {
         SCGPU_CUDA_CHECK(cudaFuncSetAttribute(k_matvec_w32<AR, 8, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
         SCGPU_CUDA_CHECK(cudaFuncSetAttribute(k_matvec_w32<AR, 8, true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
     } else {
@@ -1616,7 +1754,14 @@ int launch_matvec_w32(const W32Const<AR> &c, int sm_count, int32_t *out, const i
     if (grid > groups) grid = groups;
     if (!groups_fit(groups, grid)) { set_error("batch of %zu rows is too large", count); return SCGPU_ERR_ARG; }
     if (groups > grid) { const int e = next_work_counter(st, &ctr, 2); if (e != SCGPU_OK) return e; }
-    if (tma && chk)  k_matvec_w32<AR, 8, true, true><<<(unsigned)grid, kThreads32, smem, st>>>(out, A, s, k, l, count, ctr, c);
+    // k = 1, unaligned rows, SCGPU_MATVEC_ONE_WARP: a shared matrix is addressed with an instance stride of 0
+    if (shared) {
+        if (tma && chk)  k_matvec_w32<AR, 8, true, true, true><<<(unsigned)grid, kThreads32, smem, st>>>(out, A, s, k, l, count, ctr, c);
+        else if (tma)    k_matvec_w32<AR, 8, true, false, true><<<(unsigned)grid, kThreads32, smem, st>>>(out, A, s, k, l, count, ctr, c);
+        else if (chk)    k_matvec_w32<AR, 8, false, true, true><<<(unsigned)grid, kThreads32, smem, st>>>(out, A, s, k, l, count, ctr, c);
+        else             k_matvec_w32<AR, 8, false, false, true><<<(unsigned)grid, kThreads32, smem, st>>>(out, A, s, k, l, count, ctr, c);
+    }
+    else if (tma && chk)  k_matvec_w32<AR, 8, true, true><<<(unsigned)grid, kThreads32, smem, st>>>(out, A, s, k, l, count, ctr, c);
     else if (tma)    k_matvec_w32<AR, 8, true, false><<<(unsigned)grid, kThreads32, smem, st>>>(out, A, s, k, l, count, ctr, c);
     else if (chk)    k_matvec_w32<AR, 8, false, true><<<(unsigned)grid, kThreads32, smem, st>>>(out, A, s, k, l, count, ctr, c);
     else             k_matvec_w32<AR, 8, false, false><<<(unsigned)grid, kThreads32, smem, st>>>(out, A, s, k, l, count, ctr, c);
