@@ -500,8 +500,10 @@ int launch_matvec(const NttPlanDev &p, int32_t *out, const int32_t *A, const int
     if (k < 1 || l < 1 || l > 8) { set_error("matvec supports 1 <= l <= 8 (got k=%d l=%d)", k, l); return SCGPU_ERR_ARG; }
     if (p.logn != 8) { set_error("matvec is instantiated for n = 256 (Kyber / Dilithium); got n=%d", p.n); return SCGPU_ERR_UNSUPPORTED; }
     if (l > 4) {
-        // only the Shoup-policy kernels take l at run time (Dilithium k = 6, l = 5)
-        if (use_sh32(p) && p.sh32_mv_ok && l <= p.sh32_mv_lmax && !(use_fq32(p) && p.fq32_mv_ok))
+        // only the Shoup-policy kernels take l at run time (Dilithium k = 6, l = 5).  A modulus the float-quotient
+        // mat-vec serves (the small moduli) stays at l <= 4 under every arithmetic, as scgpu.h promises, not only
+        // under the automatic one
+        if (use_sh32(p) && p.sh32_mv_ok && l <= p.sh32_mv_lmax && !(p.fq32_ok && p.fq32_mv_ok))
             return launch_matvec_sh32(p, out, A, s, k, l, count, st, shared);
         set_error("matvec l > 4 not instantiated for this modulus");
         return SCGPU_ERR_UNSUPPORTED;
