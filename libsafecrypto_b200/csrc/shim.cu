@@ -366,6 +366,9 @@ extern "C" int scgpu_rand_matrix_csprng_batch(int32_t *A, const uint8_t *seeds, 
                                               uint32_t q_bits, int n, int k, int l, int transpose, size_t count, void *stream)
 {
     if (!A || !seeds) { set_error("rand_matrix: null argument"); return SCGPU_ERR_ARG; }
+    // the generation kernels store whole 8- and 16-byte groups of coefficients (a ring is 1 KiB, so every ring of an
+    // aligned A is aligned too)
+    if (reinterpret_cast<uintptr_t>(A) % 16 != 0) { set_error("rand_matrix: A is not 16-byte aligned"); return SCGPU_ERR_ARG; }
     const int e = check_rand_args("rand_matrix", prng_type, seed_len, n, k, l);
     if (e != SCGPU_OK) return e;
     return launch_gen_rings(prng_type, seeds, seed_len, count, A, n, k, l, transpose, q, q_bits, static_cast<cudaStream_t>(stream));
@@ -435,6 +438,9 @@ extern "C" int scgpu_rand_product_csprng_shared_batch(const scgpu_ntt_plan_t *pl
 static int rand_product_host(const scgpu_ntt_plan_t *plan, int32_t *t, const int32_t *y, const uint8_t *seeds, size_t seed_len,
                              int prng_type, uint32_t q_bits, int k, int l, int transpose, size_t count, bool shared)
 {
+    // before the pipeline is sized from k and l (k = l = 0 would divide by zero below)
+    const int e0 = check_rand_args(shared ? "rand_product_shared_host" : "rand_product_host", prng_type, seed_len, plan->dev.n, k, l);
+    if (e0 != SCGPU_OK) return e0;
     if (count == 0) return SCGPU_OK;
     scgpu_ntt_plan *p = const_cast<scgpu_ntt_plan *>(plan);
     std::lock_guard<std::mutex> lock(p->mu);
