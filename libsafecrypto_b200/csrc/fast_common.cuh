@@ -65,5 +65,14 @@ __device__ __forceinline__ void tile_load(const int32_t *tile, int32_t (&x)[8], 
     for (int m = 0; m < 8; m++) x[m] = tile[swz<LOGN>(elem_index<PassCfg<LOGN, PASS>::D>(tau, m))];
 }
 
+// grid-stride launch of `count` polynomials (n/8 threads each): per_sm resident CTAs per SM, no more CTAs than groups
+inline unsigned cta_grid(int sm_count, int n, size_t count, int per_sm)
+{
+    const size_t G = kCtaThreads / (n / 8), groups = (count + G - 1) / G;
+    size_t grid = (size_t)(sm_count > 0 ? sm_count : 148) * per_sm;
+    if (grid > groups) grid = groups;
+    return grid == 0 ? 1u : (unsigned)grid;
+}
+
 }  // namespace fast
 }  // namespace scgpu

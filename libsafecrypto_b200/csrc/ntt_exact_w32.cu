@@ -68,7 +68,7 @@ __host__ __device__ constexpr int by4(int T, int t, int j) { return ((j >> 2) * 
 // V_AVXF: the AVX2 variant with the single-precision lanes (16-bit tables, 512 < q <= 12289, ntt_template.c.in:1367-1402):
 // a kernel of its own, so that no butterfly carries both lane flavours behind a run-time test of q
 constexpr int V_AVXF = 6;
-// Integer forms of the double arithmetic (file header), selected per plan (xw32_fpint: 16-bit tables, 0 <= w < q < 2^15,
+// Integer forms of the double arithmetic (file header), selected per plan (Xw32State::fpint: 16-bit tables, 0 <= w < q < 2^15,
 // and no quotient m < 2^31 whose product m q rounds below m): fp, avx with double lanes, avx with float lanes
 constexpr int V_FPI = 7, V_AVXI = 8, V_AVXFI = 9;
 // 32-bit tables: the same integer forms hold while every multiplicand stays below 2^29 (and every lane product below
@@ -398,14 +398,14 @@ int32_t centre(int32_t w, int32_t q) { return w > q / 2 ? w - q : w; }
 
 // the two words of a twiddle entry for the plan's variant.  kind: 0 = stage with the AVX2 vector lanes (avx only),
 // 1 = scalar stage, 2 = pre / post twist
-void make_entry(const NttPlanDev &p, int32_t w, int kind, int32_t *ow, int32_t *oa)
+void make_entry(const NttPlanDev &p, bool fpint, int32_t w, int kind, int32_t *ow, int32_t *oa)
 {
     const int32_t q = p.rc.q;
     const bool tw16 = p.tw_bits == 16;
     bool centred = false;
     if (p.variant == V_REFERENCE) centred = true;
-    else if (p.variant == V_FP) centred = p.xw32_fpint != 0;
-    else if (p.variant == V_AVX && p.xw32_fpint) {
+    else if (p.variant == V_FP) centred = fpint;
+    else if (p.variant == V_AVX && fpint) {
         const bool avxf = tw16 && q <= 12289;                    // float lanes in the vector stages
         if (kind == 0) centred = !avxf;                          // double lanes: canonical Shoup product
         else if (kind == 1) centred = true;                      // fp code
@@ -427,17 +427,23 @@ void make_entry(const NttPlanDev &p, int32_t w, int kind, int32_t *ow, int32_t *
 
 }  // namespace
 
+struct Xw32State {
+    int32_t *tab;                        // [pass-1 w | aux | fwd twist w | aux | inv twist w | aux], n words each
+    bool inverse;                        // r given: inverse transforms too
+    bool fpint;                          // fp / avx: the double quotient is evaluated in integers (file header)
+    XConst fwd, inv;
+};
+
 // Eligibility and tables.  reference / barrett need canonical twiddles 0 <= w < q (the sign of the remainder follows
 // the dividend only then; every table the reference generates qualifies) and, for barrett, k in [0, 31] with
 // w * m inside 32 bits; anything else stays on the first kernel.
 int build_xw32_tables(NttPlanDev &p, const int32_t *w_host, const int32_t *r_host)
 {
-    p.xw32_ok = 0; p.xw32_tab = nullptr;
     if (p.logn < 8 || p.logn > 10 || !w_host) return SCGPU_OK;
     const int n = p.n, L = p.logn, T = n / 32;
     const int32_t q = p.rc.q;
     if (q < 3 || q >= (1 << 30)) return SCGPU_OK;
-    p.xw32_fpint = 0;
+    bool fpint = false;
     bool canonical = true;
     for (int i = 0; i < n; i++) {
         if (w_host[i] < 0 || w_host[i] >= q) canonical = false;
@@ -459,10 +465,8 @@ int build_xw32_tables(NttPlanDev &p, const int32_t *w_host, const int32_t *r_hos
         // only when m |delta| exceeds half the spacing below m, i.e. (m / 2^k) |delta| 2^53 > 1 with m / 2^k < 2.
         const long double delta = (long double)p.rc.inv_q_dbl * (long double)q - 1.0L;      // exact: 53 + 15 bits < 64
         const long double D = -delta * 9007199254740992.0L;                                  // |delta| 2^53 when delta < 0
-        if (delta >= 0.0L || D <= 0.5L) p.xw32_fpint = 1;
-        if (p.variant == V_AVX && q == 7681) p.xw32_fpint = 0;      // its twist runs the float lanes (mul_32_pointwise_16, :1081-1094)
-        const char *off = getenv("SCGPU_EXACT_FP_DOUBLES");
-        if (off && atoi(off) != 0) p.xw32_fpint = 0;
+        if (delta >= 0.0L || D <= 0.5L) fpint = true;
+        if (p.variant == V_AVX && q == 7681) fpint = false;      // its twist runs the float lanes (mul_32_pointwise_16, :1081-1094)
     }
     auto brev_bits = [](int v, int bits) { int r = 0; for (int b = 0; b < bits; b++) if (v & (1 << b)) r |= 1 << (bits - 1 - b); return r; };
     // natural table: entry 2^s + g = w[brev_s(g) * n / 2^s]
@@ -472,7 +476,7 @@ int build_xw32_tables(NttPlanDev &p, const int32_t *w_host, const int32_t *r_hos
         for (int g = 0; g < (1 << s); g++) {
             Ent e;
             const int vec = (p.variant == V_AVX && (1 << s) < (n >> 3)) ? 0 : 1;       // ntt_template.c.in:1164, :1361
-            make_entry(p, w_host[(size_t)brev_bits(g, s) << (L - s)], vec, &e.w, &e.a);
+            make_entry(p, fpint, w_host[(size_t)brev_bits(g, s) << (L - s)], vec, &e.w, &e.a);
             z[(1 << s) + g] = e;
         }
     // layout: [pass-1 w | pass-1 aux | fwd twist w | fwd twist aux | inv twist w | inv twist aux], n words each
@@ -483,26 +487,38 @@ int build_xw32_tables(NttPlanDev &p, const int32_t *w_host, const int32_t *r_hos
     for (int t = 0; t < T; t++)
         for (int j = 0; j < 32; j++) {
             int32_t ew, ea;
-            make_entry(p, w_host[t + T * j], 2, &ew, &ea);                            // pre-twist of element tau + T m
+            make_entry(p, fpint, w_host[t + T * j], 2, &ew, &ea);                            // pre-twist of element tau + T m
             pack[2 * n + by4(T, t, j)] = ew; pack[3 * n + by4(T, t, j)] = ea;
             if (r_host) {
                 const int k = (brev_bits(j, 5) << (L - 5)) | brev_bits(t, L - 5);      // coefficient of element j, thread t
-                make_entry(p, r_host[k], 2, &ew, &ea);
+                make_entry(p, fpint, r_host[k], 2, &ew, &ea);
                 pack[4 * n + by4(T, t, j)] = ew; pack[5 * n + by4(T, t, j)] = ea;
             }
         }
-    SCGPU_CUDA_CHECK(cudaMalloc(&p.xw32_tab, sizeof(int32_t) * pack.size()));
-    SCGPU_CUDA_CHECK(cudaMemcpy(p.xw32_tab, pack.data(), sizeof(int32_t) * pack.size(), cudaMemcpyHostToDevice));
-    for (int i = 0; i < 31; i++) { p.xw32_f0[i] = z[i + 1].w; p.xw32_f0[31 + i] = z[i + 1].a; }
-    p.xw32_ok = r_host ? 2 : 1;
+    Xw32State *xs = p.xw32 = new Xw32State();
+    xs->inverse = r_host != nullptr;
+    xs->fpint = fpint;
+    SCGPU_CUDA_CHECK(cudaMalloc(&xs->tab, sizeof(int32_t) * pack.size()));
+    SCGPU_CUDA_CHECK(cudaMemcpy(xs->tab, pack.data(), sizeof(int32_t) * pack.size(), cudaMemcpyHostToDevice));
+    XConst c;
+    c.p1 = xs->tab;
+    for (int i = 0; i < 31; i++) { c.f0w[i] = z[i + 1].w; c.f0a[i] = z[i + 1].a; }
+    c.rc = p.rc;
+    c.nq = -q;
+    c.qm1 = q - 1;
+    c.wp1 = (int32_t)(int64_t)nearbyint(4294967296.0 / (double)q);
+    xs->fwd = xs->inv = c;
+    xs->fwd.tw = xs->tab + 2 * (size_t)n;
+    xs->inv.tw = xs->tab + 4 * (size_t)n;
     return SCGPU_OK;
 }
 
 void free_xw32_tables(NttPlanDev &p)
 {
-    if (p.xw32_tab) cudaFree(p.xw32_tab);
-    p.xw32_tab = nullptr;
-    p.xw32_ok = 0;
+    if (!p.xw32) return;
+    cudaFree(p.xw32->tab);
+    delete p.xw32;
+    p.xw32 = nullptr;
 }
 
 namespace {
@@ -510,21 +526,14 @@ namespace {
 template <int V, int LOGN, bool TW16>
 int launch_x(const NttPlanDev &p, bool inverse, int32_t *out, const int32_t *a, size_t count, const XConst &c, cudaStream_t st)
 {
-    using C = Cfg32<LOGN>;
-    const int sms = p.sm_count > 0 ? p.sm_count : 148;
     // rows that are not 16-byte aligned cannot be bulk-copied: they stay on the first kernel
     if (((uintptr_t)a % 16) != 0 || !tma_allowed()) return SCGPU_ERR_UNSUPPORTED;
-    const size_t groups = (count + C::POLYS - 1) / C::POLYS;
-    size_t grid = (size_t)sms * 16;
-    if (grid > groups) grid = groups;
-    if (!groups_fit(groups, grid)) { set_error("batch of %zu rows is too large", count); return SCGPU_ERR_ARG; }
-    unsigned long long *ctr = nullptr;
-    if (groups > grid) { const int e = next_work_counter(st, &ctr, 4); if (e != SCGPU_OK) return e; }
-    if (inverse) k_exact_w32<V, LOGN, TW16, true, true><<<(unsigned)grid, kThreads32, 0, st>>>(out, a, count, ctr, c);
-    else         k_exact_w32<V, LOGN, TW16, false, true><<<(unsigned)grid, kThreads32, 0, st>>>(out, a, count, ctr, c);
-    count_launch();
-    SCGPU_CUDA_CHECK(cudaGetLastError());
-    return SCGPU_OK;
+    unsigned grid;
+    unsigned long long *ctr;
+    const int e = persistent_grid(p.sm_count, 16, count, Cfg32<LOGN>::POLYS, 4, st, &grid, &ctr);
+    if (e != SCGPU_OK) return e;
+    if (inverse) return launch_kernel(k_exact_w32<V, LOGN, TW16, true, true>, grid, kThreads32, 0, st, out, a, count, ctr, c);
+    return launch_kernel(k_exact_w32<V, LOGN, TW16, false, true>, grid, kThreads32, 0, st, out, a, count, ctr, c);
 }
 
 template <int V>
@@ -580,25 +589,14 @@ int launch_exact_w32(const NttPlanDev &p, int op, int32_t *out, const int32_t *a
 {
     if (op != SCGPU_OP_FWD && op != SCGPU_OP_INV) return SCGPU_ERR_UNSUPPORTED;
     const bool inverse = op == SCGPU_OP_INV;
-    if (!p.xw32_ok || (inverse && p.xw32_ok < 2)) return SCGPU_ERR_UNSUPPORTED;
-    static const bool off = [] { const char *e = getenv("SCGPU_EXACT_V1"); return e && atoi(e) != 0; }();
-    if (off) return SCGPU_ERR_UNSUPPORTED;
+    if (!p.xw32 || (inverse && !p.xw32->inverse)) return SCGPU_ERR_UNSUPPORTED;
     if (out == a && count > 0) {
         // in place is fine: a row is read completely (into registers / the staging row) before any of it is written,
         // and rows are independent -- except that the NEXT group's rows are prefetched while this one is written;
         // they are other rows.
     }
-    XConst c;
-    const int n = p.n;
-    const int32_t *tab = static_cast<const int32_t *>(p.xw32_tab);
-    c.p1 = tab;
-    c.tw = tab + (inverse ? 4 : 2) * (size_t)n;
-    memcpy(c.f0w, p.xw32_f0, sizeof(int32_t) * 31);
-    memcpy(c.f0a, p.xw32_f0 + 31, sizeof(int32_t) * 31);
-    c.rc = p.rc;
-    c.nq = -p.rc.q;
-    c.qm1 = p.rc.q - 1;
-    c.wp1 = (int32_t)(int64_t)nearbyint(4294967296.0 / (double)p.rc.q);
+    const XConst &c = inverse ? p.xw32->inv : p.xw32->fwd;
+    const bool fpint = p.xw32->fpint;
 #ifndef XW32_VARIANTS
 #define XW32_VARIANTS 0x3F
 #endif
@@ -611,7 +609,7 @@ int launch_exact_w32(const NttPlanDev &p, int op, int32_t *out, const int32_t *a
 #endif
 #if XW32_VARIANTS & 4
     case V_FP:
-        if (!p.xw32_fpint) return launch_xv<V_FP>(p, inverse, out, a, count, c, st);
+        if (!fpint) return launch_xv<V_FP>(p, inverse, out, a, count, c, st);
         return p.tw_bits == 16 ? launch_xv<V_FPI>(p, inverse, out, a, count, c, st) : launch_xv<V_FPG>(p, inverse, out, a, count, c, st);
 #endif
 #if XW32_VARIANTS & 8
@@ -619,9 +617,9 @@ int launch_exact_w32(const NttPlanDev &p, int op, int32_t *out, const int32_t *a
         // single-precision lanes for 16-bit tables with q <= 12289 (:1367-1402); the magic-number rounding needs q > 512
         if (p.tw_bits == 16 && p.rc.q <= 12289) {
             if (p.rc.q <= 512) return SCGPU_ERR_UNSUPPORTED;
-            return p.xw32_fpint ? launch_xv<V_AVXFI>(p, inverse, out, a, count, c, st) : launch_xv<V_AVXF>(p, inverse, out, a, count, c, st);
+            return fpint ? launch_xv<V_AVXFI>(p, inverse, out, a, count, c, st) : launch_xv<V_AVXF>(p, inverse, out, a, count, c, st);
         }
-        if (!p.xw32_fpint) return launch_xv<V_AVX>(p, inverse, out, a, count, c, st);
+        if (!fpint) return launch_xv<V_AVX>(p, inverse, out, a, count, c, st);
         return p.tw_bits == 16 ? launch_xv<V_AVXI>(p, inverse, out, a, count, c, st) : launch_xv<V_AVXG>(p, inverse, out, a, count, c, st);
 #endif
 #if XW32_VARIANTS & 16

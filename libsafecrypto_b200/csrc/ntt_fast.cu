@@ -320,43 +320,24 @@ MontTw make_tw(int64_t v, int64_t q, uint32_t qinv)
     return t;
 }
 
-FastConst make_const(const NttPlanDev &p)
-{
-    FastConst c;
-    c.zf = p.zeta_fwd; c.zi = p.zeta_inv;
-    c.ninv = p.ninv; c.rsq = p.rsq;
-    c.q = p.rc.q; c.qinv = p.qinv;
-    c.qbits = 0;
-    while ((1ll << c.qbits) < p.rc.q) c.qbits++;
-    c.bigq = ((int64_t)p.rc.q << p.logn) >= (1ll << 30);
-    // R mod q in Montgomery form is R^2 mod q ... "multiply by one": mont(x, R) = x
-    c.rone = make_tw(1, p.rc.q, (uint32_t)p.qinv);
-    return c;
-}
-
-unsigned grid_for(const NttPlanDev &p, size_t groups)
-{
-    const int sms = p.sm_count > 0 ? p.sm_count : 148;
-    size_t grid = (size_t)sms * 4;          // 4 resident 256-thread CTAs per SM
-    if (grid > groups) grid = groups;
-    if (grid == 0) grid = 1;
-    return (unsigned)grid;
-}
-
 }  // namespace
+
+struct MontState {
+    MontTw *zeta_fwd;    // [n]: index 2^s + b  -> psi^brv(.) * R
+    MontTw *zeta_inv;    // [n]: inverses, last-stage entries pre-multiplied by n^-1
+    FastConst c;
+};
 
 int build_fast_tables(NttPlanDev &p, const int32_t *w_host)
 {
     const int n = p.n;
     const int64_t q = p.rc.q;
-    p.zeta_fwd = nullptr; p.zeta_inv = nullptr;
     if ((q & 1) == 0 || q < 3 || q >= (1ll << 30)) return SCGPU_OK;      // fused kernels unavailable
     // the caller's table must be powers of a 2n-th root of unity: w[1]^n == -1
     const int64_t psi = ((int64_t)w_host[1] % q + q) % q;
     if (powmod(psi, n, q) != q - 1) return SCGPU_OK;
     uint32_t qinv = 1;
     for (int i = 0; i < 5; i++) qinv *= 2u - (uint32_t)q * qinv;         // Newton: q^-1 mod 2^32
-    p.qinv = (int32_t)qinv;
     const int64_t ninv = powmod(n, q - 2, q);
     std::vector<MontTw> zf(n), zi(n);
     zf[0] = make_tw(1, q, qinv); zi[0] = zf[0];
@@ -369,21 +350,31 @@ int build_fast_tables(NttPlanDev &p, const int32_t *w_host)
         zf[k] = make_tw(z, q, qinv);
         zi[k] = make_tw(zinv, q, qinv);
     }
-    p.ninv = make_tw(ninv, q, qinv);
-    const int64_t r1 = (int64_t)(((__int128)1 << 32) % q);
-    p.rsq = make_tw(r1, q, qinv);                                        // value R -> stored as R^2 mod q
-    SCGPU_CUDA_CHECK(cudaMalloc(&p.zeta_fwd, sizeof(MontTw) * n));
-    SCGPU_CUDA_CHECK(cudaMalloc(&p.zeta_inv, sizeof(MontTw) * n));
-    SCGPU_CUDA_CHECK(cudaMemcpy(p.zeta_fwd, zf.data(), sizeof(MontTw) * n, cudaMemcpyHostToDevice));
-    SCGPU_CUDA_CHECK(cudaMemcpy(p.zeta_inv, zi.data(), sizeof(MontTw) * n, cudaMemcpyHostToDevice));
+    MontState *s = p.mont = new MontState();
+    SCGPU_CUDA_CHECK(cudaMalloc(&s->zeta_fwd, sizeof(MontTw) * n));
+    SCGPU_CUDA_CHECK(cudaMalloc(&s->zeta_inv, sizeof(MontTw) * n));
+    SCGPU_CUDA_CHECK(cudaMemcpy(s->zeta_fwd, zf.data(), sizeof(MontTw) * n, cudaMemcpyHostToDevice));
+    SCGPU_CUDA_CHECK(cudaMemcpy(s->zeta_inv, zi.data(), sizeof(MontTw) * n, cudaMemcpyHostToDevice));
+    FastConst &c = s->c;
+    c.zf = s->zeta_fwd; c.zi = s->zeta_inv;
+    c.ninv = make_tw(ninv, q, qinv);
+    c.rsq = make_tw((int64_t)(((__int128)1 << 32) % q), q, qinv);      // value R -> stored as R^2 mod q
+    c.q = (int32_t)q; c.qinv = (int32_t)qinv;
+    c.qbits = 0;
+    while ((1ll << c.qbits) < q) c.qbits++;
+    c.bigq = (q << p.logn) >= (1ll << 30);
+    // R mod q in Montgomery form is R^2 mod q ... "multiply by one": mont(x, R) = x
+    c.rone = make_tw(1, q, qinv);
     return SCGPU_OK;
 }
 
 void free_fast_tables(NttPlanDev &p)
 {
-    if (p.zeta_fwd) cudaFree(p.zeta_fwd);
-    if (p.zeta_inv) cudaFree(p.zeta_inv);
-    p.zeta_fwd = p.zeta_inv = nullptr;
+    if (!p.mont) return;
+    cudaFree(p.mont->zeta_fwd);
+    cudaFree(p.mont->zeta_inv);
+    delete p.mont;
+    p.mont = nullptr;
 }
 
 // Arithmetic of the fused kernels: 0 = automatic (float-quotient where its bounds are proven -- the warp-local
@@ -404,11 +395,6 @@ static int arith_mode()
     }
     return m;
 }
-static bool use_fq(const NttPlanDev &p) { const int m = arith_mode(); return p.fq_ok && (m == 0 || m == 3); }
-static bool use_fq32(const NttPlanDev &p) { return p.fq32_ok && arith_mode() == 0; }
-static bool use_sh32(const NttPlanDev &p) { return p.sh32_ok && (arith_mode() == 0 || arith_mode() == 4); }
-static bool force_sh32(const NttPlanDev &p) { return p.sh32_ok && arith_mode() == 4; }
-static bool use_sq(const NttPlanDev &p) { return p.sq_ok && arith_mode() != 1; }
 int set_fast_arith(int mode)
 {
     const int old = arith_mode();
@@ -422,34 +408,72 @@ int set_force_montgomery(int on)
     return old;
 }
 
-#define SCGPU_REQUIRE_FAST(p)                                                                   \
-    if (!(p).zeta_fwd) {                                                                        \
-        set_error("fused kernels need an odd q < 2^30 and a table with w[1]^n == -1 (q=%d n=%d)", (p).rc.q, (p).n); \
-        return SCGPU_ERR_UNSUPPORTED;                                                           \
+namespace {
+
+enum Arith { AR_NONE, AR_MONT, AR_SQ, AR_FQ, AR_FQ32, AR_SH32 };
+enum FusedOp { OP_PRODUCT, OP_MATVEC, OP_CANONICAL };       // OP_PRODUCT: two-operand and key products
+
+// what the plan's arithmetics serve; *_lmax: largest l of their mat-vec (0: none)
+struct Caps {
+    bool mont, sq, fq, fq32, sh32;
+    int fq32_lmax, sh32_lmax;
+};
+
+// The arithmetic that runs an operation (l: the mat-vec's inner dimension) under arithmetic mode m.  AR_NONE: none
+// serves it.  The canonical transforms exist on the warp-local schedules only and follow mode 4 alone.
+Arith choose_arith(int m, const Caps &cp, FusedOp op, int l)
+{
+    if (op == OP_CANONICAL) {
+        if (cp.sh32 && (m == 4 || !cp.fq32)) return AR_SH32;
+        return cp.fq32 ? AR_FQ32 : AR_NONE;
     }
+    const bool mv = op == OP_MATVEC;
+    const bool sh32 = cp.sh32 && (!mv || l <= cp.sh32_lmax);
+    if (mv && l > 4) {
+        // only the Shoup-policy kernels take l at run time (Dilithium k = 6, l = 5).  A modulus the float-quotient
+        // mat-vec serves (the small moduli) stays at l <= 4 under every arithmetic, as scgpu.h promises, not only
+        // under the automatic one
+        return sh32 && (m == 0 || m == 4) && !(cp.fq32 && cp.fq32_lmax > 0) ? AR_SH32 : AR_NONE;
+    }
+    if (m == 4 && sh32) return AR_SH32;
+    if (m == 0 && cp.fq32 && (!mv || l <= cp.fq32_lmax)) return AR_FQ32;
+    if ((m == 0 || m == 3) && cp.fq) return AR_FQ;
+    if (m != 1 && cp.sq) return AR_SQ;
+    if (m == 0 && sh32) return AR_SH32;
+    return cp.mont ? AR_MONT : AR_NONE;
+}
+
+Arith choose_arith(const NttPlanDev &p, FusedOp op, int l = 1)
+{
+    const Caps cp{p.mont != nullptr, p.sq != nullptr, p.fq != nullptr, p.fq32 != nullptr, p.sh32 != nullptr,
+                  fq32_matvec_lmax(p), sh32_matvec_lmax(p)};
+    return choose_arith(arith_mode(), cp, op, l);
+}
+
+int fused_unavailable(const NttPlanDev &p)
+{
+    set_error("fused kernels need an odd q < 2^30 and a table with w[1]^n == -1 (q=%d n=%d)", p.rc.q, p.n);
+    return SCGPU_ERR_UNSUPPORTED;
+}
+
+}  // namespace
 
 int launch_polymul(const NttPlanDev &p, int32_t *out, const int32_t *a, const int32_t *b,
                    size_t b_stride, size_t count, cudaStream_t st)
 {
     if (count == 0) return SCGPU_OK;
-    if (force_sh32(p)) return launch_polymul_sh32(p, 0, out, a, b, b_stride, count, st);
-    if (use_fq32(p)) return launch_polymul_fq32(p, 0, out, a, b, b_stride, count, st);
-    if (use_fq(p)) return launch_polymul_fq(p, 0, out, a, b, b_stride, count, st);
-    if (use_sq(p)) return launch_polymul_sq(p, 0, out, a, b, b_stride, count, st);
-    if (use_sh32(p)) return launch_polymul_sh32(p, 0, out, a, b, b_stride, count, st);
-    SCGPU_REQUIRE_FAST(p);
-    FastConst c = make_const(p);
-    const size_t G = kCtaThreads / (p.n / 8);
-    const unsigned grid = grid_for(p, (count + G - 1) / G);
-    switch (p.logn) {
-    case 8:  k_polymul<8, MODE_POLYMUL><<<grid, kCtaThreads, 0, st>>>(out, a, b, b_stride, count, c); break;
-    case 9:  k_polymul<9, MODE_POLYMUL><<<grid, kCtaThreads, 0, st>>>(out, a, b, b_stride, count, c); break;
-    case 10: k_polymul<10, MODE_POLYMUL><<<grid, kCtaThreads, 0, st>>>(out, a, b, b_stride, count, c); break;
-    default: set_error("unsupported n=%d", p.n); return SCGPU_ERR_UNSUPPORTED;
+    switch (choose_arith(p, OP_PRODUCT)) {
+    case AR_SH32: return launch_polymul_sh32(p, 0, out, a, b, b_stride, count, st);
+    case AR_FQ32: return launch_polymul_fq32(p, 0, out, a, b, b_stride, count, st);
+    case AR_FQ:   return launch_polymul_fq(p, 0, out, a, b, b_stride, count, st);
+    case AR_SQ:   return launch_polymul_sq(p, 0, out, a, b, b_stride, count, st);
+    case AR_MONT: break;
+    default:      return fused_unavailable(p);
     }
-    count_launch();
-    SCGPU_CUDA_CHECK(cudaGetLastError());
-    return SCGPU_OK;
+    const unsigned grid = cta_grid(p.sm_count, p.n, count, 4);      // 4 resident 256-thread CTAs per SM
+    return with_int<8, 9, 10>(p.logn, [&](auto L) {
+        return launch_kernel(k_polymul<L, MODE_POLYMUL>, grid, kCtaThreads, 0, st, out, a, b, b_stride, count, p.mont->c);
+    });
 }
 
 // normalize_32(fwd_ntt(a)) / inv_ntt(a) through the warp-local kernels; SCGPU_ERR_UNSUPPORTED when neither
@@ -457,10 +481,11 @@ int launch_polymul(const NttPlanDev &p, int32_t *out, const int32_t *a, const in
 int launch_ntt_canonical(const NttPlanDev &p, int inverse, int32_t *out, const int32_t *a, size_t count, cudaStream_t st)
 {
     if (count == 0) return SCGPU_OK;
-    const int m = arith_mode();
-    if (p.sh32_ok && (m == 4 || !p.fq32_ok)) return launch_ntt_sh32(p, inverse, out, a, count, st);
-    if (p.fq32_ok) return launch_ntt_fq32(p, inverse, out, a, count, st);
-    return SCGPU_ERR_UNSUPPORTED;
+    switch (choose_arith(p, OP_CANONICAL)) {
+    case AR_SH32: return launch_ntt_sh32(p, inverse, out, a, count, st);
+    case AR_FQ32: return launch_ntt_fq32(p, inverse, out, a, count, st);
+    default:      return SCGPU_ERR_UNSUPPORTED;
+    }
 }
 
 int launch_mul_key(const NttPlanDev &p, int32_t *out, const int32_t *t, const void *key,
@@ -468,64 +493,41 @@ int launch_mul_key(const NttPlanDev &p, int32_t *out, const int32_t *t, const vo
 {
     if (count == 0) return SCGPU_OK;
     if (key_bits != 16 && key_bits != 32) { set_error("key_bits must be 16 or 32"); return SCGPU_ERR_ARG; }
-    if (force_sh32(p)) return launch_polymul_sh32(p, key_bits == 16 ? 1 : 2, out, t, key, key_stride, count, st);
-    if (use_fq32(p)) return launch_polymul_fq32(p, key_bits == 16 ? 1 : 2, out, t, key, key_stride, count, st);
-    if (use_fq(p)) return launch_polymul_fq(p, key_bits == 16 ? 1 : 2, out, t, key, key_stride, count, st);
-    if (use_sq(p)) return launch_polymul_sq(p, key_bits == 16 ? 1 : 2, out, t, key, key_stride, count, st);
-    if (use_sh32(p)) return launch_polymul_sh32(p, key_bits == 16 ? 1 : 2, out, t, key, key_stride, count, st);
-    SCGPU_REQUIRE_FAST(p);
-    FastConst c = make_const(p);
-    const size_t G = kCtaThreads / (p.n / 8);
-    const unsigned grid = grid_for(p, (count + G - 1) / G);
-#define SCGPU_KEY_LAUNCH(L)                                                                          \
-    if (key_bits == 16) k_polymul<L, MODE_KEY16><<<grid, kCtaThreads, 0, st>>>(out, t, key, key_stride, count, c); \
-    else                k_polymul<L, MODE_KEY32><<<grid, kCtaThreads, 0, st>>>(out, t, key, key_stride, count, c);
-    switch (p.logn) {
-    case 8:  SCGPU_KEY_LAUNCH(8); break;
-    case 9:  SCGPU_KEY_LAUNCH(9); break;
-    case 10: SCGPU_KEY_LAUNCH(10); break;
-    default: set_error("unsupported n=%d", p.n); return SCGPU_ERR_UNSUPPORTED;
+    const int mode = key_bits == 16 ? MODE_KEY16 : MODE_KEY32;
+    switch (choose_arith(p, OP_PRODUCT)) {
+    case AR_SH32: return launch_polymul_sh32(p, mode, out, t, key, key_stride, count, st);
+    case AR_FQ32: return launch_polymul_fq32(p, mode, out, t, key, key_stride, count, st);
+    case AR_FQ:   return launch_polymul_fq(p, mode, out, t, key, key_stride, count, st);
+    case AR_SQ:   return launch_polymul_sq(p, mode, out, t, key, key_stride, count, st);
+    case AR_MONT: break;
+    default:      return fused_unavailable(p);
     }
-#undef SCGPU_KEY_LAUNCH
-    count_launch();
-    SCGPU_CUDA_CHECK(cudaGetLastError());
-    return SCGPU_OK;
+    const unsigned grid = cta_grid(p.sm_count, p.n, count, 4);
+    return with_int<8, 9, 10>(p.logn, [&](auto L) {
+        return with_int<MODE_KEY16, MODE_KEY32>(mode, [&](auto M) {
+            return launch_kernel(k_polymul<L, M>, grid, kCtaThreads, 0, st, out, t, key, key_stride, count, p.mont->c);
+        });
+    });
 }
 
 int launch_matvec(const NttPlanDev &p, int32_t *out, const int32_t *A, const int32_t *s,
                   int k, int l, size_t count, cudaStream_t st, bool shared)
 {
     if (count == 0) return SCGPU_OK;
-    SCGPU_REQUIRE_FAST(p);
+    if (!p.mont) return fused_unavailable(p);
     if (k < 1 || l < 1 || l > 8) { set_error("matvec supports 1 <= l <= 8 (got k=%d l=%d)", k, l); return SCGPU_ERR_ARG; }
     if (p.logn != 8) { set_error("matvec is instantiated for n = 256 (Kyber / Dilithium); got n=%d", p.n); return SCGPU_ERR_UNSUPPORTED; }
-    if (l > 4) {
-        // only the Shoup-policy kernels take l at run time (Dilithium k = 6, l = 5).  A modulus the float-quotient
-        // mat-vec serves (the small moduli) stays at l <= 4 under every arithmetic, as scgpu.h promises, not only
-        // under the automatic one
-        if (use_sh32(p) && p.sh32_mv_ok && l <= p.sh32_mv_lmax && !(p.fq32_ok && p.fq32_mv_ok))
-            return launch_matvec_sh32(p, out, A, s, k, l, count, st, shared);
-        set_error("matvec l > 4 not instantiated for this modulus");
-        return SCGPU_ERR_UNSUPPORTED;
+    switch (choose_arith(p, OP_MATVEC, l)) {
+    case AR_SH32: return launch_matvec_sh32(p, out, A, s, k, l, count, st, shared);
+    case AR_FQ32: return launch_matvec_fq32(p, out, A, s, k, l, count, st, shared);
+    case AR_FQ:   return launch_matvec_fq(p, out, A, s, k, l, count, st, shared);
+    case AR_SQ:   return launch_matvec_sq(p, out, A, s, k, l, count, st, shared);
+    case AR_MONT: break;
+    default:      set_error("matvec l > 4 not instantiated for this modulus"); return SCGPU_ERR_UNSUPPORTED;
     }
-    if (force_sh32(p) && p.sh32_mv_ok) return launch_matvec_sh32(p, out, A, s, k, l, count, st, shared);
-    if (use_fq32(p) && p.fq32_mv_ok) return launch_matvec_fq32(p, out, A, s, k, l, count, st, shared);
-    if (use_fq(p)) return launch_matvec_fq(p, out, A, s, k, l, count, st, shared);
-    if (use_sq(p)) return launch_matvec_sq(p, out, A, s, k, l, count, st, shared);
-    if (use_sh32(p) && p.sh32_mv_ok) return launch_matvec_sh32(p, out, A, s, k, l, count, st, shared);
-    FastConst c = make_const(p);
-    const size_t G = kCtaThreads / (p.n / 8);
-    // shared-memory stash limits residency to 1-2 CTAs per SM
-    const unsigned grid = grid_for(p, (count + G - 1) / G);
-    if (l <= 4 && shared) k_matvec<8, 4, true><<<grid, kCtaThreads, 0, st>>>(out, A, s, k, l, count, c);
-    else if (l <= 4) k_matvec<8, 4><<<grid, kCtaThreads, 0, st>>>(out, A, s, k, l, count, c);
-    else {
-        set_error("matvec l > 4 not instantiated");
-        return SCGPU_ERR_UNSUPPORTED;
-    }
-    count_launch();
-    SCGPU_CUDA_CHECK(cudaGetLastError());
-    return SCGPU_OK;
+    const unsigned grid = cta_grid(p.sm_count, p.n, count, 4);
+    if (shared) return launch_kernel(k_matvec<8, 4, true>, grid, kCtaThreads, 0, st, out, A, s, k, l, count, p.mont->c);
+    return launch_kernel(k_matvec<8, 4>, grid, kCtaThreads, 0, st, out, A, s, k, l, count, p.mont->c);
 }
 
 }  // namespace scgpu

@@ -21,6 +21,7 @@
 #include "fq_host.h"
 #include "../../include/scgpu.h"
 
+#include <algorithm>
 #include <vector>
 
 namespace scgpu {
@@ -367,53 +368,22 @@ k_matvec_fq(int32_t *__restrict__ out, const int32_t *__restrict__ A, const int3
     }
 }
 
-FqConst fq_const(const NttPlanDev &p, bool matvec)
-{
-    FqConst c;
-    const int n = p.n;
-    c.zf.w = static_cast<const int32_t *>(p.fq_zf);
-    c.zf.wq = reinterpret_cast<const float *>(c.zf.w + n);
-    c.zi.w = static_cast<const int32_t *>(p.fq_zi);
-    c.zi.wq = reinterpret_cast<const float *>(c.zi.w + n);
-    memcpy(c.f0, p.fq_pass0, sizeof(Tw) * 7);
-    memcpy(c.i0, p.fq_pass0 + sizeof(Tw) * 7, sizeof(Tw) * 7);
-    memcpy(&c.ninv, p.fq_ninv, sizeof(Tw));
-    memcpy(&c.one, p.fq_one, sizeof(Tw));
-    c.q = p.rc.q; c.nq = -p.rc.q; c.x0 = p.fq_x0;
-    c.pwk = (int32_t)((uint32_t)kBias * (uint32_t)p.rc.q);
-    c.kf = c.pwk;
-    c.ki = (int32_t)((uint32_t)c.pwk + (uint32_t)kBias);
-    c.invq = (float)(1.0 / (double)p.rc.q);
-    c.M = (uint32_t)((1ull << 32) / (uint64_t)p.rc.q);
-    for (int i = 0; i < 4; i++) c.r_inv[i] = matvec ? p.fq_r_inv_mv[i] : p.fq_r_inv[i];
-    return c;
-}
-
-unsigned fq_grid(const NttPlanDev &p, size_t groups, int per_sm)
-{
-    const int sms = p.sm_count > 0 ? p.sm_count : 148;
-    size_t grid = (size_t)sms * per_sm;
-    if (grid > groups) grid = groups;
-    if (grid == 0) grid = 1;
-    return (unsigned)grid;
-}
-
 }  // namespace
+
+struct FqState {
+    int32_t *zf, *zi;       // w[n] followed by wq[n]
+    FqConst prod, mv;       // mv: range reductions for up to 4 accumulated products
+};
 
 int build_fq_tables(NttPlanDev &p, const int32_t *w_host)
 {
-    p.fq_ok = 0; p.fq_zf = p.fq_zi = nullptr;
     if (p.logn < 8 || p.logn > 10) return SCGPU_OK;
     const fq::Schedule s1 = fq::analyse(p.logn, p.rc.q, 1);
     const fq::Schedule s4 = fq::analyse(p.logn, p.rc.q, 4);
     if (!s1.ok || !s4.ok) return SCGPU_OK;                 // the Barrett / Montgomery kernels serve this (q, n)
     std::vector<Tw> zf, zi;
-    Tw ninv, one;
-    if (!fq::build_tables(p.logn, p.rc.q, w_host, zf, zi, ninv, one)) return SCGPU_OK;
-    memcpy(p.fq_ninv, &ninv, sizeof(Tw));
-    memcpy(p.fq_one, &one, sizeof(Tw));
-    p.fq_x0 = s1.x0;
-    for (int i = 0; i < 4; i++) { p.fq_r_inv[i] = s1.r_inv[i]; p.fq_r_inv_mv[i] = s4.r_inv[i]; }
+    FqConst c;
+    if (!fq::build_tables(p.logn, p.rc.q, w_host, zf, zi, c.ninv, c.one)) return SCGPU_OK;
     // device tables: w[n] followed by wq[n]; the derived k / c of every entry equal the host-built ones
     // (checked here so that a table the derivation cannot reproduce is never used)
     std::vector<int32_t> packf(2 * p.n), packi(2 * p.n);
@@ -427,57 +397,54 @@ int build_fq_tables(NttPlanDev &p, const int32_t *w_host)
         const bool oki = (k < 2 || ki == zi[k].k) && fmaf(zi[k].wq, -fq::kBiasF, fq::kBiasF) == zi[k].c;
         if (!okf || !oki) { set_error("float-quotient table self-check failed at entry %d", k); return SCGPU_ERR_ARG; }
     }
-    memcpy(p.fq_pass0, &zf[1], sizeof(Tw) * 7);
-    memcpy(p.fq_pass0 + sizeof(Tw) * 7, &zi[1], sizeof(Tw) * 7);
-    SCGPU_CUDA_CHECK(cudaMalloc(&p.fq_zf, sizeof(int32_t) * 2 * p.n));
-    SCGPU_CUDA_CHECK(cudaMalloc(&p.fq_zi, sizeof(int32_t) * 2 * p.n));
-    SCGPU_CUDA_CHECK(cudaMemcpy(p.fq_zf, packf.data(), sizeof(int32_t) * 2 * p.n, cudaMemcpyHostToDevice));
-    SCGPU_CUDA_CHECK(cudaMemcpy(p.fq_zi, packi.data(), sizeof(int32_t) * 2 * p.n, cudaMemcpyHostToDevice));
-    p.fq_ok = 1;
+    FqState *s = p.fq = new FqState();
+    SCGPU_CUDA_CHECK(cudaMalloc(&s->zf, sizeof(int32_t) * 2 * p.n));
+    SCGPU_CUDA_CHECK(cudaMalloc(&s->zi, sizeof(int32_t) * 2 * p.n));
+    SCGPU_CUDA_CHECK(cudaMemcpy(s->zf, packf.data(), sizeof(int32_t) * 2 * p.n, cudaMemcpyHostToDevice));
+    SCGPU_CUDA_CHECK(cudaMemcpy(s->zi, packi.data(), sizeof(int32_t) * 2 * p.n, cudaMemcpyHostToDevice));
+    c.zf.w = s->zf;
+    c.zf.wq = reinterpret_cast<const float *>(s->zf + p.n);
+    c.zi.w = s->zi;
+    c.zi.wq = reinterpret_cast<const float *>(s->zi + p.n);
+    std::copy(zf.begin() + 1, zf.begin() + 8, c.f0);         // pass 0: entries 1..7
+    std::copy(zi.begin() + 1, zi.begin() + 8, c.i0);
+    c.q = p.rc.q; c.nq = -p.rc.q; c.x0 = s1.x0;
+    c.pwk = pwk;
+    c.kf = c.pwk;
+    c.ki = (int32_t)((uint32_t)c.pwk + (uint32_t)kBias);
+    c.invq = (float)(1.0 / (double)p.rc.q);
+    c.M = (uint32_t)((1ull << 32) / (uint64_t)p.rc.q);
+    s->prod = s->mv = c;
+    for (int i = 0; i < 4; i++) { s->prod.r_inv[i] = s1.r_inv[i]; s->mv.r_inv[i] = s4.r_inv[i]; }
     return SCGPU_OK;
 }
 
 void free_fq_tables(NttPlanDev &p)
 {
-    if (p.fq_zf) cudaFree(p.fq_zf);
-    if (p.fq_zi) cudaFree(p.fq_zi);
-    p.fq_zf = p.fq_zi = nullptr;
-    p.fq_ok = 0;
+    if (!p.fq) return;
+    cudaFree(p.fq->zf);
+    cudaFree(p.fq->zi);
+    delete p.fq;
+    p.fq = nullptr;
 }
 
 int launch_polymul_fq(const NttPlanDev &p, int mode, int32_t *out, const int32_t *a, const void *b,
                       size_t b_stride, size_t count, cudaStream_t st)
 {
-    const FqConst c = fq_const(p, false);
-    const size_t G = kCtaThreads / (p.n / 8);
-    const unsigned grid = fq_grid(p, (count + G - 1) / G, 3);
-#define FQ_LAUNCH(L)                                                                                             \
-    if (mode == FQ_POLYMUL)    k_polymul_fq<L, FQ_POLYMUL><<<grid, kCtaThreads, 0, st>>>(out, a, b, b_stride, count, c); \
-    else if (mode == FQ_KEY16) k_polymul_fq<L, FQ_KEY16><<<grid, kCtaThreads, 0, st>>>(out, a, b, b_stride, count, c);   \
-    else                       k_polymul_fq<L, FQ_KEY32><<<grid, kCtaThreads, 0, st>>>(out, a, b, b_stride, count, c);
-    switch (p.logn) {
-    case 8:  FQ_LAUNCH(8); break;
-    case 9:  FQ_LAUNCH(9); break;
-    case 10: FQ_LAUNCH(10); break;
-    default: set_error("unsupported n=%d", p.n); return SCGPU_ERR_UNSUPPORTED;
-    }
-#undef FQ_LAUNCH
-    count_launch();
-    SCGPU_CUDA_CHECK(cudaGetLastError());
-    return SCGPU_OK;
+    const unsigned grid = cta_grid(p.sm_count, p.n, count, 3);
+    return with_int<8, 9, 10>(p.logn, [&](auto L) {
+        return with_int<FQ_POLYMUL, FQ_KEY16, FQ_KEY32>(mode, [&](auto M) {
+            return launch_kernel(k_polymul_fq<L, M>, grid, kCtaThreads, 0, st, out, a, b, b_stride, count, p.fq->prod);
+        });
+    });
 }
 
 int launch_matvec_fq(const NttPlanDev &p, int32_t *out, const int32_t *A, const int32_t *s, int k, int l,
                      size_t count, cudaStream_t st, bool shared)
 {
-    const FqConst c = fq_const(p, true);
-    const size_t G = kCtaThreads / (p.n / 8);
-    const unsigned grid = fq_grid(p, (count + G - 1) / G, 2);
-    if (shared) k_matvec_fq<8, 4, true><<<grid, kCtaThreads, 0, st>>>(out, A, s, k, l, count, c);
-    else        k_matvec_fq<8, 4><<<grid, kCtaThreads, 0, st>>>(out, A, s, k, l, count, c);
-    count_launch();
-    SCGPU_CUDA_CHECK(cudaGetLastError());
-    return SCGPU_OK;
+    const unsigned grid = cta_grid(p.sm_count, p.n, count, 2);
+    if (shared) return launch_kernel(k_matvec_fq<8, 4, true>, grid, kCtaThreads, 0, st, out, A, s, k, l, count, p.fq->mv);
+    return launch_kernel(k_matvec_fq<8, 4>, grid, kCtaThreads, 0, st, out, A, s, k, l, count, p.fq->mv);
 }
 
 }  // namespace scgpu

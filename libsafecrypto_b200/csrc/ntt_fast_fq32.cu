@@ -19,6 +19,7 @@
 #include "warp32.cuh"
 #include "fq_host.h"
 
+#include <algorithm>
 #include <cstring>
 #include <vector>
 
@@ -162,31 +163,6 @@ struct ArFq {
 
 typedef w32::W32Const<ArFq> FqConst32;
 
-FqConst32 fq32_const(const NttPlanDev &p, int r0, bool bm = false)
-{
-    FqConst32 c;
-    const int n = p.n;
-    c.pf = static_cast<const int32_t *>(p.fq32_tab);
-    c.pi = c.pf + 4 * n;
-    c.pz = static_cast<const int32_t *>(p.fq32_zeta);
-    memcpy(c.f0, p.fq32_pass0, sizeof(Tw) * 31);
-    memcpy(c.i0, p.fq32_pass0 + sizeof(Tw) * 31, sizeof(Tw) * 31);
-    memcpy(&c.ninv, p.fq_ninv, sizeof(Tw));
-    if (bm) {                                       // two inverse stages fewer: (n/4)^-1 in the last stage
-        memcpy(&c.ninv, p.fq32_ninv_bm, sizeof(Tw));
-        memcpy(&c.i0[0], p.fq32_i01_bm, sizeof(Tw));
-    }
-    memcpy(&c.one, p.fq_one, sizeof(Tw));
-    c.q = p.rc.q; c.nq = -p.rc.q; c.x0 = p.fq32_x0;
-    c.k.q = p.rc.q; c.k.nq = -p.rc.q;
-    c.k.pwk = (int32_t)((uint32_t)kBias * (uint32_t)p.rc.q);
-    c.k.invq = (float)(1.0 / (double)p.rc.q);
-    c.k.pwb = (int32_t)((uint32_t)c.k.pwk + (uint32_t)kBias);
-    c.M = (uint32_t)((1ull << 32) / (uint64_t)p.rc.q);
-    c.r0 = r0;
-    return c;
-}
-
 // ---- key residues for the base-multiplication key product -------------------------------------------------------
 // The key arrives fully transformed (the reference's NTT-domain order).  Two Gentleman-Sande stages and a factor 1/4
 // take the four point values of block b back to the residue modulo X^4 - zeta_b; the table also holds zeta_b times
@@ -226,19 +202,27 @@ __global__ void k_key_residues(int32_t *__restrict__ kres, const KT *__restrict_
 
 }  // namespace
 
+struct Fq32State {
+    int32_t *tab;                        // forward [w | wq | k | c], inverse [w | wq | k | c], n words each
+    // degree-3 base multiplication of the two-operand product (fq_arith.cuh: basemul4); bm_ok == false: (q, n) outside
+    // its bounds
+    int32_t *zeta;                       // (w, wq) of zeta per block of four, [pair][tau][4 words]: n/2 words
+    int32_t *ktab;                       // k_key_residues: [zi stage logn-2 | zi stage logn-1 | zeta], n words
+    int32_t inv4;                        // 4^-1 mod q
+    bool mv_ok, bm_ok;                   // mv_ok: mat-vec with up to 4 accumulated products
+    FqConst32 prod, mv, bm;              // bm: last inverse stage with (n/4)^-1
+};
+
 int build_fq32_tables(NttPlanDev &p, const int32_t *w_host)
 {
-    p.fq32_ok = 0; p.fq32_tab = nullptr;
-    p.fq32_bm_ok = 0; p.fq32_zeta = nullptr; p.fq32_ktab = nullptr;
     if (p.logn < 8 || p.logn > 10) return SCGPU_OK;
     int r0 = 0; int32_t x0 = 0;
     if (!fq::analyse32(p.logn, p.rc.q, 1, &r0, &x0)) return SCGPU_OK;
     int r0_mv = 0; int32_t x0_mv = 0;
-    p.fq32_mv_ok = fq::analyse32(p.logn, p.rc.q, 4, &r0_mv, &x0_mv) ? 1 : 0;     // up to 4 accumulated products
-    p.fq32_r0_mv = r0_mv;
+    const bool mv_ok = fq::analyse32(p.logn, p.rc.q, 4, &r0_mv, &x0_mv);     // up to 4 accumulated products
     std::vector<Tw> zf, zi;
-    Tw ninv, one;
-    if (!fq::build_tables(p.logn, p.rc.q, w_host, zf, zi, ninv, one)) return SCGPU_OK;
+    FqConst32 c;
+    if (!fq::build_tables(p.logn, p.rc.q, w_host, zf, zi, c.ninv, c.one)) return SCGPU_OK;
     const int n = p.n;
     // forward [w | wq | k | c] then inverse [w | wq | k | c], n words each, entries of stages >= 5 thread-major
     std::vector<int32_t> pack(8 * n, 0);
@@ -247,21 +231,17 @@ int build_fq32_tables(NttPlanDev &p, const int32_t *w_host)
         if (k == 0) v = e.w; else if (k == 1) memcpy(&v, &e.wq, 4); else if (k == 2) v = e.k; else memcpy(&v, &e.c, 4);
         return v;
     }, pack.data());
-    SCGPU_CUDA_CHECK(cudaMalloc(&p.fq32_tab, sizeof(int32_t) * 8 * n));
-    SCGPU_CUDA_CHECK(cudaMemcpy(p.fq32_tab, pack.data(), sizeof(int32_t) * 8 * n, cudaMemcpyHostToDevice));
-    memcpy(p.fq32_pass0, &zf[1], sizeof(Tw) * 31);
-    memcpy(p.fq32_pass0 + sizeof(Tw) * 31, &zi[1], sizeof(Tw) * 31);
-    memcpy(p.fq_ninv, &ninv, sizeof(Tw));
-    memcpy(p.fq_one, &one, sizeof(Tw));
-    p.fq32_r0 = r0;
-    p.fq32_x0 = x0;
-    p.fq32_ok = 1;
+    Fq32State *s = p.fq32 = new Fq32State();
+    s->mv_ok = mv_ok;
+    SCGPU_CUDA_CHECK(cudaMalloc(&s->tab, sizeof(int32_t) * 8 * n));
+    SCGPU_CUDA_CHECK(cudaMemcpy(s->tab, pack.data(), sizeof(int32_t) * 8 * n, cudaMemcpyHostToDevice));
     // base multiplication of the two-operand product: zeta pairs thread-major, [pair pr][tau][w, wq, w, wq]
     // (blocks 8 tau + 2 pr and 8 tau + 2 pr + 1 of thread tau)
     int r0_bm = 0;
+    Tw ninv_bm, i01_bm;
     const char *no_bm = getenv("SCGPU_NO_BASEMUL");
     if (!(no_bm && atoi(no_bm) != 0) && fq::analyse32_bm(p.logn, p.rc.q, x0, &r0_bm)) {
-        std::vector<int32_t> zw; std::vector<float> zwq; Tw ninv_bm, i01_bm;
+        std::vector<int32_t> zw; std::vector<float> zwq;
         fq::build_bm_tables(p.logn, p.rc.q, w_host, zw, zwq, ninv_bm, i01_bm);
         const int T = n / 32;
         std::vector<int32_t> zp((size_t)n / 2);
@@ -272,44 +252,63 @@ int build_fq32_tables(NttPlanDev &p, const int32_t *w_host)
                     zp[((size_t)pr * T + tau) * 4 + 2 * u] = zw[blk];
                     memcpy(&zp[((size_t)pr * T + tau) * 4 + 2 * u + 1], &zwq[blk], 4);
                 }
-        SCGPU_CUDA_CHECK(cudaMalloc(&p.fq32_zeta, sizeof(int32_t) * zp.size()));
-        SCGPU_CUDA_CHECK(cudaMemcpy(p.fq32_zeta, zp.data(), sizeof(int32_t) * zp.size(), cudaMemcpyHostToDevice));
-        memcpy(p.fq32_ninv_bm, &ninv_bm, sizeof(Tw));
-        memcpy(p.fq32_i01_bm, &i01_bm, sizeof(Tw));
+        SCGPU_CUDA_CHECK(cudaMalloc(&s->zeta, sizeof(int32_t) * zp.size()));
+        SCGPU_CUDA_CHECK(cudaMemcpy(s->zeta, zp.data(), sizeof(int32_t) * zp.size(), cudaMemcpyHostToDevice));
         // table of k_key_residues: inverse twiddles of the last two stages (natural index) and zeta, in [0, q)
         std::vector<int32_t> kt((size_t)n);
         for (int b = 0; b < n / 4; b++) { kt[b] = zi[n / 4 + b].w; kt[n / 4 + n / 2 + b] = zw[b]; }
         for (int b = 0; b < n / 2; b++) kt[n / 4 + b] = zi[n / 2 + b].w;
-        SCGPU_CUDA_CHECK(cudaMalloc(&p.fq32_ktab, sizeof(int32_t) * kt.size()));
-        SCGPU_CUDA_CHECK(cudaMemcpy(p.fq32_ktab, kt.data(), sizeof(int32_t) * kt.size(), cudaMemcpyHostToDevice));
-        p.fq32_inv4 = (int32_t)fq::powmod(4, p.rc.q - 2, p.rc.q);
-        p.fq32_r0_bm = r0_bm;
-        p.fq32_bm_ok = 1;
+        SCGPU_CUDA_CHECK(cudaMalloc(&s->ktab, sizeof(int32_t) * kt.size()));
+        SCGPU_CUDA_CHECK(cudaMemcpy(s->ktab, kt.data(), sizeof(int32_t) * kt.size(), cudaMemcpyHostToDevice));
+        s->inv4 = (int32_t)fq::powmod(4, p.rc.q - 2, p.rc.q);
+        s->bm_ok = true;
+    }
+    c.pf = s->tab;
+    c.pi = c.pf + 4 * n;
+    c.pz = s->zeta;
+    std::copy(zf.begin() + 1, zf.begin() + 32, c.f0);         // pass 0: entries 1..31
+    std::copy(zi.begin() + 1, zi.begin() + 32, c.i0);
+    c.q = p.rc.q; c.nq = -p.rc.q; c.x0 = x0;
+    c.k.q = p.rc.q; c.k.nq = -p.rc.q;
+    c.k.pwk = (int32_t)((uint32_t)kBias * (uint32_t)p.rc.q);
+    c.k.invq = (float)(1.0 / (double)p.rc.q);
+    c.k.pwb = (int32_t)((uint32_t)c.k.pwk + (uint32_t)kBias);
+    c.M = (uint32_t)((1ull << 32) / (uint64_t)p.rc.q);
+    s->prod = s->mv = s->bm = c;
+    s->prod.r0 = r0;
+    s->mv.r0 = r0_mv;
+    if (s->bm_ok) {                                  // two inverse stages fewer: (n/4)^-1 in the last stage
+        s->bm.r0 = r0_bm;
+        s->bm.ninv = ninv_bm;
+        s->bm.i0[0] = i01_bm;
     }
     return SCGPU_OK;
 }
 
 void free_fq32_tables(NttPlanDev &p)
 {
-    if (p.fq32_tab) cudaFree(p.fq32_tab);
-    if (p.fq32_zeta) cudaFree(p.fq32_zeta);
-    if (p.fq32_ktab) cudaFree(p.fq32_ktab);
-    p.fq32_tab = nullptr; p.fq32_zeta = nullptr; p.fq32_ktab = nullptr;
-    p.fq32_ok = 0; p.fq32_bm_ok = 0;
+    if (!p.fq32) return;
+    cudaFree(p.fq32->tab);
+    cudaFree(p.fq32->zeta);
+    cudaFree(p.fq32->ktab);
+    delete p.fq32;
+    p.fq32 = nullptr;
 }
 
-// n = 256 (Kyber); returns SCGPU_ERR_UNSUPPORTED when this schedule does not apply (the caller falls back)
+int fq32_matvec_lmax(const NttPlanDev &p) { return p.fq32 && p.fq32->mv_ok ? 4 : 0; }
+
+// n = 256 (Kyber), l <= 4 (launch_matvec)
 int launch_matvec_fq32(const NttPlanDev &p, int32_t *out, const int32_t *A, const int32_t *s, int k, int l,
                        size_t count, cudaStream_t st, bool shared)
 {
-    if (!p.fq32_ok || !p.fq32_mv_ok || p.logn != 8 || l > 4) return SCGPU_ERR_UNSUPPORTED;
-    return w32::launch_matvec_w32<ArFq>(fq32_const(p, p.fq32_r0_mv), p.sm_count, out, A, s, k, l, count, st, !p.inputs_in_range, shared);
+    return w32::launch_matvec_w32<ArFq>(p.fq32->mv, p.sm_count, out, A, s, k, l, count, st, !p.inputs_in_range, shared);
 }
 
 int launch_polymul_fq32(const NttPlanDev &p, int mode, int32_t *out, const int32_t *a, const void *b,
                         size_t b_stride, size_t count, cudaStream_t st)
 {
-    if (b_stride == 0 && p.fq32_bm_ok && (mode != w32::FQ_POLYMUL || count >= 64)) {
+    const Fq32State &fs = *p.fq32;
+    if (b_stride == 0 && fs.bm_ok && (mode != w32::FQ_POLYMUL || count >= 64)) {
         // One second operand for the whole batch.  A shared key (the BLISS signing product) arrives transformed: its
         // residues modulo X^4 - zeta are prepared once for the launch in a stream-ordered scratch, then the batch runs
         // the base-multiplication key product.  A shared RAW operand (scgpu_polymul_batch with b_stride = 0) is first
@@ -318,7 +317,7 @@ int launch_polymul_fq32(const NttPlanDev &p, int mode, int32_t *out, const int32
         int32_t *kres = nullptr;
         SCGPU_CUDA_CHECK(cudaMallocAsync(reinterpret_cast<void **>(&kres), sizeof(int32_t) * 5 * (size_t)p.n, st));
         int32_t *hat = kres + 4 * (size_t)p.n;
-        const int nb = p.n / 4, th = 64;
+        const unsigned nb = p.n / 4, th = 64;
         int e = SCGPU_OK;
         if (mode == w32::FQ_POLYMUL) {
             e = launch_ntt_fq32(p, 0, hat, static_cast<const int32_t *>(b), 1, st);
@@ -326,25 +325,24 @@ int launch_polymul_fq32(const NttPlanDev &p, int mode, int32_t *out, const int32
         }
         if (e == SCGPU_OK) {
             if (mode == w32::FQ_KEY16)
-                k_key_residues<int16_t><<<(nb + th - 1) / th, th, 0, st>>>(kres, static_cast<const int16_t *>(b), static_cast<const int32_t *>(p.fq32_ktab), p.logn, p.rc.q, p.fq32_inv4);
+                e = launch_kernel(k_key_residues<int16_t>, (nb + th - 1) / th, th, 0, st, kres, static_cast<const int16_t *>(b), fs.ktab, p.logn, p.rc.q, fs.inv4);
             else
-                k_key_residues<int32_t><<<(nb + th - 1) / th, th, 0, st>>>(kres, static_cast<const int32_t *>(b), static_cast<const int32_t *>(p.fq32_ktab), p.logn, p.rc.q, p.fq32_inv4);
-            count_launch();
-            e = w32::launch_polymul_w32<ArFq>(fq32_const(p, p.fq32_r0_bm, true), p.logn, p.sm_count, w32::FQ_KEYBM, out, a, kres, 0,
-                                              count, st, true, !p.inputs_in_range);
+                e = launch_kernel(k_key_residues<int32_t>, (nb + th - 1) / th, th, 0, st, kres, static_cast<const int32_t *>(b), fs.ktab, p.logn, p.rc.q, fs.inv4);
         }
+        if (e == SCGPU_OK)
+            e = w32::launch_polymul_w32<ArFq>(fs.bm, p.logn, p.sm_count, w32::FQ_KEYBM, out, a, kres, 0, count, st, true, !p.inputs_in_range);
         const cudaError_t fe = cudaFreeAsync(kres, st);
         if (e == SCGPU_OK && fe != cudaSuccess) { set_error("cudaFreeAsync failed: %s", cudaGetErrorString(fe)); e = SCGPU_ERR_CUDA; }
         return e;
     }
-    const bool bm = mode == w32::FQ_POLYMUL && p.fq32_bm_ok;
-    return w32::launch_polymul_w32<ArFq>(fq32_const(p, bm ? p.fq32_r0_bm : p.fq32_r0, bm), p.logn, p.sm_count, mode, out, a, b,
-                                         b_stride, count, st, bm, !p.inputs_in_range);
+    const bool bm = mode == w32::FQ_POLYMUL && fs.bm_ok;
+    return w32::launch_polymul_w32<ArFq>(bm ? fs.bm : fs.prod, p.logn, p.sm_count, mode, out, a, b, b_stride, count, st, bm,
+                                         !p.inputs_in_range);
 }
 
 int launch_ntt_fq32(const NttPlanDev &p, int inverse, int32_t *out, const int32_t *a, size_t count, cudaStream_t st)
 {
-    return w32::launch_ntt_w32<ArFq>(fq32_const(p, p.fq32_r0), p.logn, p.sm_count, inverse, out, a, count, st, !p.inputs_in_range);
+    return w32::launch_ntt_w32<ArFq>(p.fq32->prod, p.logn, p.sm_count, inverse, out, a, count, st, !p.inputs_in_range);
 }
 
 }  // namespace scgpu

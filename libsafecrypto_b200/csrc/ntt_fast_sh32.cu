@@ -11,7 +11,7 @@
 // Coefficients are plain signed integers, lazily reduced; the host bounds every intermediate (analyse_sh).
 #include "warp32.cuh"
 
-#include <cstring>
+#include <algorithm>
 #include <vector>
 
 namespace scgpu {
@@ -157,42 +157,29 @@ bool analyse_sh(int logn, int64_t qi, int accumulate, int *r0_out, int32_t *x0_o
     return false;
 }
 
-ShConst32 sh32_const(const NttPlanDev &p, int r0)
-{
-    ShConst32 c;
-    const int n = p.n;
-    c.pf = static_cast<const int32_t *>(p.sh32_tab);
-    c.pi = c.pf + 2 * n;
-    c.pz = nullptr;
-    memcpy(c.f0, p.sh32_pass0, sizeof(ArSh::E) * 31);
-    memcpy(c.i0, p.sh32_pass0 + sizeof(ArSh::E) * 31, sizeof(ArSh::E) * 31);
-    memcpy(&c.ninv, p.sh32_ninv, sizeof(ArSh::E));
-    memcpy(&c.one, p.sh32_one, sizeof(ArSh::E));
-    c.q = p.rc.q; c.nq = -p.rc.q; c.x0 = p.sh32_x0;
-    c.k.q = p.rc.q; c.k.nq = -p.rc.q; c.k.qinv = p.qinv;
-    c.M = (uint32_t)((1ull << 32) / (uint64_t)p.rc.q);
-    c.r0 = r0;
-    return c;
-}
-
 }  // namespace
+
+struct Sh32State {
+    int32_t *tab;                        // forward [w | wp], inverse [w | wp], n words each
+    int mv_lmax;                         // largest l whose exact 64-bit sums stay inside the Montgomery range (analyse_sh)
+    ShConst32 prod, mv;
+    ShConst32 inv;                       // stand-alone inverse transform: last-stage multipliers without the factor R
+};
 
 int build_sh32_tables(NttPlanDev &p, const int32_t *w_host)
 {
-    p.sh32_ok = 0; p.sh32_mv_ok = 0; p.sh32_mv_lmax = 0; p.sh32_tab = nullptr;
     if (p.logn < 8 || p.logn > 10) return SCGPU_OK;
     const int64_t q = p.rc.q;
     int r0 = 0; int32_t x0 = 0;
     if (!analyse_sh(p.logn, q, 1, &r0, &x0)) return SCGPU_OK;
     int r0_mv = 0; int32_t x0_mv = 0;
-    p.sh32_mv_ok = analyse_sh(p.logn, q, 4, &r0_mv, &x0_mv) ? 1 : 0;
-    p.sh32_r0_mv = r0_mv;
+    const bool mv_ok = analyse_sh(p.logn, q, 4, &r0_mv, &x0_mv);
     // Dilithium's largest set is k = 6, l = 5 (240 q < 2^31 for q = 8380417): accept every l the sum bound admits
-    p.sh32_mv_lmax = p.sh32_mv_ok ? 4 : 0;
-    for (int L = 5; L <= 8 && p.sh32_mv_ok; L++) {
+    int mv_lmax = mv_ok ? 4 : 0;
+    for (int L = 5; L <= 8 && mv_ok; L++) {
         int r0x = 0; int32_t x0x = 0;
         if (!analyse_sh(p.logn, q, L, &r0x, &x0x) || r0x != r0_mv) break;
-        p.sh32_mv_lmax = L;
+        mv_lmax = L;
     }
     const int n = p.n;
     const int64_t psi = (((int64_t)w_host[1] % q) + q) % q;
@@ -209,58 +196,64 @@ int build_sh32_tables(NttPlanDev &p, const int32_t *w_host)
         zf[k] = make_entry(z, q);
         zi[k] = make_entry(zinv, q);
     }
-    const ArSh::E ninv = make_entry(ninvR, q), one = make_entry(1, q);
-    {
-        // a stand-alone inverse transform has no Montgomery product to compensate: plain n^-1 and n^-1 psi^-(n/2)
-        const int64_t nin = powmod(n, q - 2, q);
-        const int e1 = 1 << (p.logn - 1);                                    // brv(1)
-        const int64_t zinv1 = (q - (((int64_t)w_host[n - e1] % q) + q) % q) % q;
-        const ArSh::E np = make_entry(nin, q), zp = make_entry((int64_t)(((__int128)zinv1 * nin) % q), q);
-        memcpy(p.sh32_ninv_plain, &np, sizeof(np));
-        memcpy(p.sh32_zi1_plain, &zp, sizeof(zp));
-    }
     std::vector<int32_t> pack(4 * n, 0);
     w32::pack_pass1<ArSh>(p.logn, zf, zi, [](const ArSh::E &e, int k) { return k == 0 ? e.w : e.wp; }, pack.data());
-    SCGPU_CUDA_CHECK(cudaMalloc(&p.sh32_tab, sizeof(int32_t) * 4 * n));
-    SCGPU_CUDA_CHECK(cudaMemcpy(p.sh32_tab, pack.data(), sizeof(int32_t) * 4 * n, cudaMemcpyHostToDevice));
-    memcpy(p.sh32_pass0, &zf[1], sizeof(ArSh::E) * 31);
-    memcpy(p.sh32_pass0 + sizeof(ArSh::E) * 31, &zi[1], sizeof(ArSh::E) * 31);
-    memcpy(p.sh32_ninv, &ninv, sizeof(ArSh::E));
-    memcpy(p.sh32_one, &one, sizeof(ArSh::E));
-    p.sh32_r0 = r0;
-    p.sh32_x0 = x0;
-    p.sh32_ok = 1;
+    Sh32State *s = p.sh32 = new Sh32State();
+    s->mv_lmax = mv_lmax;
+    SCGPU_CUDA_CHECK(cudaMalloc(&s->tab, sizeof(int32_t) * 4 * n));
+    SCGPU_CUDA_CHECK(cudaMemcpy(s->tab, pack.data(), sizeof(int32_t) * 4 * n, cudaMemcpyHostToDevice));
+    uint32_t qinv = 1;
+    for (int i = 0; i < 5; i++) qinv *= 2u - (uint32_t)q * qinv;         // Newton: q^-1 mod 2^32
+    ShConst32 c;
+    c.pf = s->tab;
+    c.pi = c.pf + 2 * n;
+    c.pz = nullptr;
+    std::copy(zf.begin() + 1, zf.begin() + 32, c.f0);         // pass 0: entries 1..31
+    std::copy(zi.begin() + 1, zi.begin() + 32, c.i0);
+    c.ninv = make_entry(ninvR, q);
+    c.one = make_entry(1, q);
+    c.q = (int32_t)q; c.nq = (int32_t)-q; c.x0 = x0;
+    c.k.q = (int32_t)q; c.k.nq = (int32_t)-q; c.k.qinv = (int32_t)qinv;
+    c.M = (uint32_t)((1ull << 32) / (uint64_t)q);
+    s->prod = s->mv = s->inv = c;
+    s->prod.r0 = s->inv.r0 = r0;
+    s->mv.r0 = r0_mv;
+    // a stand-alone inverse transform has no Montgomery product to compensate: plain n^-1 and n^-1 psi^-(n/2)
+    const int64_t nin = powmod(n, q - 2, q);
+    const int e1 = 1 << (p.logn - 1);                                        // brv(1)
+    const int64_t zinv1 = (q - (((int64_t)w_host[n - e1] % q) + q) % q) % q;
+    s->inv.ninv = make_entry(nin, q);
+    s->inv.i0[0] = make_entry((int64_t)(((__int128)zinv1 * nin) % q), q);
     return SCGPU_OK;
 }
 
 void free_sh32_tables(NttPlanDev &p)
 {
-    if (p.sh32_tab) cudaFree(p.sh32_tab);
-    p.sh32_tab = nullptr;
-    p.sh32_ok = 0;
+    if (!p.sh32) return;
+    cudaFree(p.sh32->tab);
+    delete p.sh32;
+    p.sh32 = nullptr;
 }
 
+int sh32_matvec_lmax(const NttPlanDev &p) { return p.sh32 ? p.sh32->mv_lmax : 0; }
+
+// n = 256, l <= mv_lmax (launch_matvec)
 int launch_matvec_sh32(const NttPlanDev &p, int32_t *out, const int32_t *A, const int32_t *s, int k, int l,
                        size_t count, cudaStream_t st, bool shared)
 {
-    if (!p.sh32_ok || !p.sh32_mv_ok || p.logn != 8 || l > p.sh32_mv_lmax) return SCGPU_ERR_UNSUPPORTED;
-    return w32::launch_matvec_w32<ArSh>(sh32_const(p, p.sh32_r0_mv), p.sm_count, out, A, s, k, l, count, st, !p.inputs_in_range, shared);
+    return w32::launch_matvec_w32<ArSh>(p.sh32->mv, p.sm_count, out, A, s, k, l, count, st, !p.inputs_in_range, shared);
 }
 
 int launch_polymul_sh32(const NttPlanDev &p, int mode, int32_t *out, const int32_t *a, const void *b,
                         size_t b_stride, size_t count, cudaStream_t st)
 {
-    return w32::launch_polymul_w32<ArSh>(sh32_const(p, p.sh32_r0), p.logn, p.sm_count, mode, out, a, b, b_stride, count, st, false, !p.inputs_in_range);
+    return w32::launch_polymul_w32<ArSh>(p.sh32->prod, p.logn, p.sm_count, mode, out, a, b, b_stride, count, st, false, !p.inputs_in_range);
 }
 
 int launch_ntt_sh32(const NttPlanDev &p, int inverse, int32_t *out, const int32_t *a, size_t count, cudaStream_t st)
 {
-    ShConst32 c = sh32_const(p, p.sh32_r0);
-    if (inverse) {
-        memcpy(&c.ninv, p.sh32_ninv_plain, sizeof(ArSh::E));
-        memcpy(&c.i0[0], p.sh32_zi1_plain, sizeof(ArSh::E));
-    }
-    return w32::launch_ntt_w32<ArSh>(c, p.logn, p.sm_count, inverse, out, a, count, st, !p.inputs_in_range);
+    return w32::launch_ntt_w32<ArSh>(inverse ? p.sh32->inv : p.sh32->prod, p.logn, p.sm_count, inverse, out, a, count, st,
+                                     !p.inputs_in_range);
 }
 
 }  // namespace scgpu

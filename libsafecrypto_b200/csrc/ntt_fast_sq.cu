@@ -295,38 +295,20 @@ int64_t powmod64(int64_t b, int64_t e, int64_t q)
 
 int32_t centre(int64_t v, int64_t q) { return (int32_t)(v > q / 2 ? v - q : v); }
 
-SqConst sq_const(const NttPlanDev &p)
-{
-    SqConst c;
-    c.zf = p.sq_zf; c.zi = p.sq_zi; c.q = p.rc.q; c.nq = -p.rc.q; c.M = (int32_t)p.sq_M; c.ninv = p.sq_ninv; c.x0 = p.sq_x0;
-    c.qbits = p.sq_qbits; c.r_pw = p.sq_r_pw;
-    for (int i = 0; i < 4; i++) c.r_inv[i] = p.sq_r_inv[i];
-    return c;
-}
-
-unsigned sq_grid(const NttPlanDev &p, size_t groups, int per_sm)
-{
-    const int sms = p.sm_count > 0 ? p.sm_count : 148;
-    size_t grid = (size_t)sms * per_sm;
-    if (grid > groups) grid = groups;
-    if (grid == 0) grid = 1;
-    return (unsigned)grid;
-}
-
 }  // namespace
 
 // Interval propagation over the kernel's dataflow.  All magnitudes are upper bounds on |value|.
-// Returns true and fills the compress schedule when every 32-bit product is provably below 2^31.
-static bool sq_analyse(NttPlanDev &p, int max_accumulate, int *r_inv_out)
+// Returns true and fills sc's compress schedule when every 32-bit product is provably below 2^31.
+static bool sq_analyse(const NttPlanDev &p, SqConst &sc, int max_accumulate)
 {
     const double q = p.rc.q, lim = 2147483647.0;
     const double wmax = (double)(p.rc.q / 2);           // centred twiddles
-    const int L = p.sq_qbits;
+    const int L = sc.qbits;
     const double f = 1.0 - q / (double)(1ll << L);      // compress: |x'| <= f |x| + q
     auto comp = [&](double b, int rounds) { for (int r = 0; r < rounds; r++) b = f * b + q; return b; };
     const double t = q;                                 // |bred(.)| < q for any 32-bit argument
     // forward: additive growth from the proven input magnitude
-    double bf = p.sq_x0;
+    double bf = sc.x0;
     for (int s = 0; s < p.logn; s++) {
         if (bf * wmax >= lim) return false;
         bf += t;
@@ -338,7 +320,7 @@ static bool sq_analyse(NttPlanDev &p, int max_accumulate, int *r_inv_out)
         if (c * c < lim && c * (q > 32768.0 ? q : 32768.0) < lim) { r_pw = r; break; }
     }
     if (r_pw < 0) return false;
-    p.sq_r_pw = r_pw;
+    sc.r_pw = r_pw;
     // inverse passes, last pass of the schedule first; matvec accumulates up to max_accumulate products
     const int npass = (p.logn + 2) / 3;
     double bin = t * max_accumulate;
@@ -367,27 +349,32 @@ static bool sq_analyse(NttPlanDev &p, int max_accumulate, int *r_inv_out)
             }
         }
         if (chosen < 0) return false;
-        r_inv_out[pass] = chosen;
+        sc.r_inv[pass] = chosen;
         bin = bout;
     }
     return true;
 }
 
+struct SqState {
+    int32_t *zf, *zi;
+    SqConst prod, mv;       // mv: compress schedule for up to 4 accumulated products
+};
+
 int build_sq_tables(NttPlanDev &p, const int32_t *w_host)
 {
-    p.sq_ok = 0; p.sq_zf = p.sq_zi = nullptr;
     const int n = p.n;
     const int64_t q = p.rc.q;
     if ((q & 1) == 0 || q < 257 || q >= (1 << 20) || p.logn < 8 || p.logn > 10) return SCGPU_OK;
     const int64_t psi = (((int64_t)w_host[1] % q) + q) % q;
     if (powmod64(psi, n, q) != q - 1) return SCGPU_OK;
-    p.sq_qbits = 0;
-    while ((1ll << p.sq_qbits) < q) p.sq_qbits++;
-    p.sq_M = (uint32_t)((1ull << 32) / (uint64_t)q);
-    p.sq_x0 = (int32_t)(4 * q);
-    for (int i = 0; i < 4; i++) p.sq_r_inv[i] = p.sq_r_inv_mv[i] = 0;
+    SqConst c{};
+    c.q = (int32_t)q; c.nq = (int32_t)-q;
+    while ((1ll << c.qbits) < q) c.qbits++;
+    c.M = (int32_t)(uint32_t)((1ull << 32) / (uint64_t)q);
+    c.x0 = (int32_t)(4 * q);
+    SqConst mv = c;
     // products can exceed 32 bits for this (q, n): the Montgomery kernels serve it
-    if (!sq_analyse(p, 1, p.sq_r_inv) || !sq_analyse(p, 4, p.sq_r_inv_mv)) return SCGPU_OK;
+    if (!sq_analyse(p, c, 1) || !sq_analyse(p, mv, 4)) return SCGPU_OK;
     const int64_t ninv = powmod64(n, q - 2, q);
     std::vector<int32_t> zf(n), zi(n);
     zf[0] = zi[0] = 1;
@@ -400,57 +387,45 @@ int build_sq_tables(NttPlanDev &p, const int32_t *w_host)
         zf[k] = centre(z, q);
         zi[k] = centre(zinv, q);
     }
-    p.sq_ninv = centre(ninv, q);
-    SCGPU_CUDA_CHECK(cudaMalloc(&p.sq_zf, sizeof(int32_t) * n));
-    SCGPU_CUDA_CHECK(cudaMalloc(&p.sq_zi, sizeof(int32_t) * n));
-    SCGPU_CUDA_CHECK(cudaMemcpy(p.sq_zf, zf.data(), sizeof(int32_t) * n, cudaMemcpyHostToDevice));
-    SCGPU_CUDA_CHECK(cudaMemcpy(p.sq_zi, zi.data(), sizeof(int32_t) * n, cudaMemcpyHostToDevice));
-    p.sq_ok = 1;
+    SqState *s = p.sq = new SqState();
+    SCGPU_CUDA_CHECK(cudaMalloc(&s->zf, sizeof(int32_t) * n));
+    SCGPU_CUDA_CHECK(cudaMalloc(&s->zi, sizeof(int32_t) * n));
+    SCGPU_CUDA_CHECK(cudaMemcpy(s->zf, zf.data(), sizeof(int32_t) * n, cudaMemcpyHostToDevice));
+    SCGPU_CUDA_CHECK(cudaMemcpy(s->zi, zi.data(), sizeof(int32_t) * n, cudaMemcpyHostToDevice));
+    c.zf = mv.zf = s->zf;
+    c.zi = mv.zi = s->zi;
+    c.ninv = mv.ninv = centre(ninv, q);
+    s->prod = c;
+    s->mv = mv;
     return SCGPU_OK;
 }
 
 void free_sq_tables(NttPlanDev &p)
 {
-    if (p.sq_zf) cudaFree(p.sq_zf);
-    if (p.sq_zi) cudaFree(p.sq_zi);
-    p.sq_zf = p.sq_zi = nullptr;
-    p.sq_ok = 0;
+    if (!p.sq) return;
+    cudaFree(p.sq->zf);
+    cudaFree(p.sq->zi);
+    delete p.sq;
+    p.sq = nullptr;
 }
 
 int launch_polymul_sq(const NttPlanDev &p, int mode, int32_t *out, const int32_t *a, const void *b,
                       size_t b_stride, size_t count, cudaStream_t st)
 {
-    SqConst c = sq_const(p);
-    const size_t G = kCtaThreads / (p.n / 8);
-    const unsigned grid = sq_grid(p, (count + G - 1) / G, 4);
-#define SQ_LAUNCH(L)                                                                                             \
-    if (mode == SQ_POLYMUL)    k_polymul_sq<L, SQ_POLYMUL><<<grid, kCtaThreads, 0, st>>>(out, a, b, b_stride, count, c); \
-    else if (mode == SQ_KEY16) k_polymul_sq<L, SQ_KEY16><<<grid, kCtaThreads, 0, st>>>(out, a, b, b_stride, count, c);   \
-    else                       k_polymul_sq<L, SQ_KEY32><<<grid, kCtaThreads, 0, st>>>(out, a, b, b_stride, count, c);
-    switch (p.logn) {
-    case 8:  SQ_LAUNCH(8); break;
-    case 9:  SQ_LAUNCH(9); break;
-    case 10: SQ_LAUNCH(10); break;
-    default: set_error("unsupported n=%d", p.n); return SCGPU_ERR_UNSUPPORTED;
-    }
-#undef SQ_LAUNCH
-    count_launch();
-    SCGPU_CUDA_CHECK(cudaGetLastError());
-    return SCGPU_OK;
+    const unsigned grid = cta_grid(p.sm_count, p.n, count, 4);
+    return with_int<8, 9, 10>(p.logn, [&](auto L) {
+        return with_int<SQ_POLYMUL, SQ_KEY16, SQ_KEY32>(mode, [&](auto M) {
+            return launch_kernel(k_polymul_sq<L, M>, grid, kCtaThreads, 0, st, out, a, b, b_stride, count, p.sq->prod);
+        });
+    });
 }
 
 int launch_matvec_sq(const NttPlanDev &p, int32_t *out, const int32_t *A, const int32_t *s, int k, int l,
                      size_t count, cudaStream_t st, bool shared)
 {
-    SqConst c = sq_const(p);
-    for (int i = 0; i < 4; i++) c.r_inv[i] = p.sq_r_inv_mv[i];
-    const size_t G = kCtaThreads / (p.n / 8);
-    const unsigned grid = sq_grid(p, (count + G - 1) / G, 2);
-    if (shared) k_matvec_sq<8, 4, true><<<grid, kCtaThreads, 0, st>>>(out, A, s, k, l, count, c);
-    else        k_matvec_sq<8, 4><<<grid, kCtaThreads, 0, st>>>(out, A, s, k, l, count, c);
-    count_launch();
-    SCGPU_CUDA_CHECK(cudaGetLastError());
-    return SCGPU_OK;
+    const unsigned grid = cta_grid(p.sm_count, p.n, count, 2);
+    if (shared) return launch_kernel(k_matvec_sq<8, 4, true>, grid, kCtaThreads, 0, st, out, A, s, k, l, count, p.sq->mv);
+    return launch_kernel(k_matvec_sq<8, 4>, grid, kCtaThreads, 0, st, out, A, s, k, l, count, p.sq->mv);
 }
 
 }  // namespace scgpu

@@ -4,8 +4,11 @@
 #include <cuda_runtime.h>
 #include <cstdint>
 #include <cstddef>
+#include <type_traits>
+#include <utility>
 
 #include "reduce.cuh"
+#include "../../include/scgpu.h"
 
 namespace scgpu {
 
@@ -23,55 +26,61 @@ int init_work_counters();      // per-device ring of counters, allocated at plan
         }                                                                                   \
     } while (0)
 
-// Device-resident state of one (q, n, variant) parameter set.
+// One kernel launch: the 200 KiB opt-in for a kernel with dynamic shared memory (per launch, not once: the attribute
+// belongs to the current device's context and plans exist per device), the launch, the launch count, the error check.
+template <class... P, class... A>
+int launch_kernel(void (*kernel)(P...), unsigned grid, unsigned block, size_t smem, cudaStream_t st, A &&...args)
+{
+    if (smem > 0) SCGPU_CUDA_CHECK(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
+    kernel<<<grid, block, smem, st>>>(std::forward<A>(args)...);
+    count_launch();
+    SCGPU_CUDA_CHECK(cudaGetLastError());
+    return SCGPU_OK;
+}
+
+// Run-time choices to template arguments.  with_int<Vs...>(v, f): f(std::integral_constant<int, v>{}) for the listed
+// value v (SCGPU_ERR_UNSUPPORTED for any other); with_flags(f, b0, b1, ...): f(std::bool_constant<b0>{}, ...).
+template <int... Vs, class F>
+int with_int(int v, F &&f)
+{
+    int r = SCGPU_ERR_UNSUPPORTED;
+    (void)((v == Vs ? (r = f(std::integral_constant<int, Vs>{}), true) : false) || ...);
+    return r;
+}
+template <class F>
+int with_flags(F &&f) { return f(); }
+template <class F, class... B>
+int with_flags(F &&f, bool b, B... rest)
+{
+    if (b) return with_flags([&](auto... t) { return f(std::true_type{}, t...); }, rest...);
+    return with_flags([&](auto... t) { return f(std::false_type{}, t...); }, rest...);
+}
+
+// Plan state of each arithmetic of the fused and warp-local kernels, defined in its own .cu: device tables, the
+// kernel-constant structs its launches pass (built once at plan creation, read-only afterwards: plans are shared by
+// host threads) and what the arithmetic can serve.
+struct MontState;      // ntt_fast.cu: Montgomery, any odd q < 2^30
+struct SqState;        // ntt_fast_sq.cu: 32-bit Barrett, small moduli
+struct FqState;        // ntt_fast_fq.cu: float-quotient products on the 8-coefficient schedule
+struct Fq32State;      // ntt_fast_fq32.cu: float-quotient products on the warp-local schedule
+struct Sh32State;      // ntt_fast_sh32.cu: Shoup products on the warp-local schedule, moduli up to 2^26
+struct Xw32State;      // ntt_exact_w32.cu: variant-exact transforms on the warp-local schedule
+
+// Device-resident state of one (q, n, variant) parameter set.  Zero-initialised by scgpu_ntt_plan_create; a state
+// pointer is nullptr when its arithmetic does not apply to (q, n).
 struct NttPlanDev {
     int n, logn, variant, tw_bits, device;
     RedConst rc;
     int32_t *w;          // caller's w[n], sign-extended to 32 bits
     int32_t *r;          // caller's r[n]
-    // fused-kernel constants (Montgomery domain, R = 2^32)
-    MontTw *zeta_fwd;    // [n]: index 2^s + b  -> psi^brv(.) * R
-    MontTw *zeta_inv;    // [n]: inverses, last-stage entries pre-multiplied by n^-1
-    MontTw ninv;         // n^-1 * R   (sum branch of the last inverse stage)
-    MontTw rsq;          // R^2 mod q  (brings one pointwise operand into Montgomery form)
-    int32_t qinv;        // q^-1 mod 2^32
-    int32_t fold;        // reserved
     int sm_count;
-    // small-modulus fused kernels (32-bit Barrett, ntt_fast_sq.cu); sq_ok == 0: not applicable to (q, n)
-    int sq_ok, sq_qbits, sq_r_pw, sq_r_inv[4], sq_r_inv_mv[4];
-    int32_t *sq_zf, *sq_zi;
-    int32_t sq_ninv, sq_x0;
-    uint32_t sq_M;
-    // small-modulus fused kernels, float-quotient arithmetic (ntt_fast_fq.cu); fq_ok == 0: not applicable
-    int fq_ok, fq_r_inv[4], fq_r_inv_mv[4];
-    int32_t fq_x0;
-    void *fq_zf, *fq_zi;                 // int32 w[n] followed by float wq[n]
-    alignas(16) unsigned char fq_ninv[16], fq_one[16];
-    alignas(16) unsigned char fq_pass0[2 * 7 * 16];   // fq::Tw entries 1..7 of the forward / inverse table
-    // warp-local 32-coefficient schedule of the same arithmetic (ntt_fast_fq32.cu)
-    int fq32_ok, fq32_r0, fq32_mv_ok, fq32_r0_mv;
-    int32_t fq32_x0;
-    void *fq32_tab;                      // forward [w | wq | k | c], inverse [w | wq | k | c], n words each
-    alignas(16) unsigned char fq32_pass0[2 * 31 * 16];
-    // degree-3 base multiplication of the two-operand product (fq_arith.cuh: basemul4); 0: (q, n) outside its bounds
-    int fq32_bm_ok, fq32_r0_bm;
-    void *fq32_zeta;                     // (w, wq) of zeta per block of four, [pair][tau][4 words]: n/2 words
-    void *fq32_ktab;                     // k_key_residues: [zi stage logn-2 | zi stage logn-1 | zeta], n words
-    int32_t fq32_inv4;                   // 4^-1 mod q
-    alignas(16) unsigned char fq32_ninv_bm[16], fq32_i01_bm[16];      // last inverse stage with (n/4)^-1
     int inputs_in_range;                 // SCGPU_PLAN_INPUTS_IN_RANGE: the fused products skip the range vote
-    // Shoup / Montgomery arithmetic on the same schedule, for moduli up to 2^25 (ntt_fast_sh32.cu)
-    int sh32_ok, sh32_r0, sh32_mv_ok, sh32_r0_mv;
-    int sh32_mv_lmax;          // largest l whose exact 64-bit sums stay inside the Montgomery range (analyse_sh)
-    int32_t sh32_x0;
-    void *sh32_tab;                      // forward [w | wp], inverse [w | wp], n words each
-    alignas(16) unsigned char sh32_pass0[2 * 31 * 8], sh32_ninv[8], sh32_one[8];
-    alignas(16) unsigned char sh32_ninv_plain[8], sh32_zi1_plain[8];   // last-stage multipliers without the factor R
-    // variant-exact transforms on the warp-local schedule (ntt_exact_w32.cu): 0 not applicable, 1 forward only (no r), 2 both
-    int xw32_ok;
-    int xw32_fpint;                      // fp / avx: the double quotient is evaluated in integers (ntt_exact_w32.cu header)
-    void *xw32_tab;                      // [pass-1 w | aux | fwd twist w | aux | inv twist w | aux], n words each
-    int32_t xw32_f0[62];                 // stages 0..4: 31 x w, 31 x aux
+    MontState *mont;
+    SqState *sq;
+    FqState *fq;
+    Fq32State *fq32;
+    Sh32State *sh32;
+    Xw32State *xw32;
 };
 
 struct ExactArgs {
@@ -127,6 +136,9 @@ int launch_ntt_sh32(const NttPlanDev &plan, int inverse, int32_t *out, const int
 int launch_ntt_canonical(const NttPlanDev &plan, int inverse, int32_t *out, const int32_t *a, size_t count, cudaStream_t stream);
 int launch_matvec_fq32(const NttPlanDev &plan, int32_t *out, const int32_t *A, const int32_t *s, int k, int l,
                        size_t count, cudaStream_t stream, bool shared = false);
+// largest l of the mat-vec of a warp-local arithmetic the plan has (0: none)
+int fq32_matvec_lmax(const NttPlanDev &plan);
+int sh32_matvec_lmax(const NttPlanDev &plan);
 int launch_matvec_fq(const NttPlanDev &plan, int32_t *out, const int32_t *A, const int32_t *s, int k, int l,
                      size_t count, cudaStream_t stream, bool shared = false);
 int build_sq_tables(NttPlanDev &plan, const int32_t *w_host);

@@ -214,7 +214,7 @@ extern "C" int scgpu_ntt_plan_create(scgpu_ntt_plan_t **out, const void *params,
         if (rcode == SCGPU_OK) rcode = build_fq32_tables(d, wh.data());
         // needed where the float-quotient arithmetic does not apply; built for every modulus it can serve so that
         // scgpu_set_fast_arith(4) can cross-check it against the other arithmetics
-        if (rcode == SCGPU_OK && d.zeta_fwd) rcode = build_sh32_tables(d, wh.data());
+        if (rcode == SCGPU_OK) rcode = build_sh32_tables(d, wh.data());
         if (rcode == SCGPU_OK) rcode = build_xw32_tables(d, wh.data(), r ? rh.data() : nullptr);
         if (rcode != SCGPU_OK) return rcode;
     }

@@ -1482,108 +1482,66 @@ inline bool tma_allowed()
     return !(no_tma && atoi(no_tma) != 0);
 }
 
+// Persistent grid over `count` rows in groups of per_group: min(SMs x per_sm, groups) CTAs; the groups after the first
+// grid-full are claimed from a work counter, chunk groups per claim (*ctr stays nullptr when one grid-full holds them).
+inline int persistent_grid(int sm_count, int per_sm, size_t count, int per_group, int chunk, cudaStream_t st,
+                           unsigned *grid, unsigned long long **ctr)
+{
+    const size_t groups = (count + per_group - 1) / per_group;
+    size_t g = (size_t)(sm_count > 0 ? sm_count : 148) * per_sm;
+    if (g > groups) g = groups;
+    if (!groups_fit(groups, g)) { set_error("batch of %zu rows is too large", count); return SCGPU_ERR_ARG; }
+    *grid = (unsigned)g;
+    *ctr = nullptr;
+    return groups > g ? next_work_counter(st, ctr, chunk) : SCGPU_OK;
+}
+
 // bm: base-multiplication kernel (FQ_POLYMUL, policies with AR::BASEMUL; c must carry the (n/4)^-1 entries);
 // chk = false: no range vote on the operands
 template <class AR>
 int launch_polymul_w32(const W32Const<AR> &c, int logn, int sm_count, int mode, int32_t *out, const int32_t *a,
                        const void *b, size_t b_stride, size_t count, cudaStream_t st, bool bm = false, bool chk = true)
 {
-    const int sms = sm_count > 0 ? sm_count : 148;
     // bulk copies need 16-byte aligned rows; the second operand is only staged in FQ_POLYMUL mode
     bool tma = ((uintptr_t)a % 16) == 0 && tma_allowed();
     if (mode == FQ_POLYMUL) tma = tma && ((uintptr_t)b % 16) == 0 && (b_stride % 4) == 0;
-    unsigned long long *ctr = nullptr;               // work counter, only when the batch exceeds one grid-full
     if (mode == FQ_KEYBM && !(AR::BASEMUL && bm)) { set_error("key residue product: not available for this arithmetic"); return SCGPU_ERR_UNSUPPORTED; }
     if (mode != FQ_POLYMUL && mode != FQ_KEYBM) bm = false;
     if (!AR::BASEMUL) bm = false;
-#define W32_GO(L, MODE, TMA_, BM_, CHK_) \
-    k_polymul_w32<AR, L, MODE, TMA_, BM_, CHK_><<<(unsigned)grid, kThreads32, 0, st>>>(out, a, b, b_stride, count, ctr, c)
-#define W32_PM(L, TMA_)                                                                                    \
-    {                                                                                                      \
-        if constexpr (AR::BASEMUL) {                                                                       \
-            if (bm && chk) W32_GO(L, FQ_POLYMUL, TMA_, true, true);                                        \
-            else if (bm)   W32_GO(L, FQ_POLYMUL, TMA_, true, false);                                       \
-        }                                                                                                  \
-        if (!bm && chk) W32_GO(L, FQ_POLYMUL, TMA_, false, true);                                          \
-        else if (!bm)   W32_GO(L, FQ_POLYMUL, TMA_, false, false);                                         \
-    }
-#define W32_KB(L, TMA_)                                                                                    \
-    {                                                                                                      \
-        if constexpr (AR::BASEMUL) {                                                                       \
-            if (chk) W32_GO(L, FQ_KEYBM, TMA_, true, true); else W32_GO(L, FQ_KEYBM, TMA_, true, false);   \
-        }                                                                                                  \
-    }
-#define W32_LAUNCH(L)                                                                                      \
-    {                                                                                                      \
-        const size_t groups = (count + Cfg32<L>::POLYS - 1) / Cfg32<L>::POLYS;                             \
-        size_t grid = (size_t)sms * FQ32_MINB;                                                             \
-        if (grid > groups) grid = groups;                                                                  \
-        if (!groups_fit(groups, grid)) { set_error("batch of %zu rows is too large", count); return SCGPU_ERR_ARG; } \
-        if (groups > grid) { const int e = next_work_counter(st, &ctr, 2); if (e != SCGPU_OK) return e; }     \
-        if (mode == FQ_KEYBM) { if (tma) W32_KB(L, true) else W32_KB(L, false) }                           \
-        else if (tma) {                                                                                    \
-            if (mode == FQ_POLYMUL)    W32_PM(L, true)                                                     \
-            else if (mode == FQ_KEY16) { if (chk) W32_GO(L, FQ_KEY16, true, false, true); else W32_GO(L, FQ_KEY16, true, false, false); } \
-            else                       { if (chk) W32_GO(L, FQ_KEY32, true, false, true); else W32_GO(L, FQ_KEY32, true, false, false); } \
-        } else {                                                                                           \
-            if (mode == FQ_POLYMUL)    W32_PM(L, false)                                                    \
-            else if (mode == FQ_KEY16) { if (chk) W32_GO(L, FQ_KEY16, false, false, true); else W32_GO(L, FQ_KEY16, false, false, false); } \
-            else                       { if (chk) W32_GO(L, FQ_KEY32, false, false, true); else W32_GO(L, FQ_KEY32, false, false, false); } \
-        }                                                                                                  \
-    }
-    switch (logn) {
-    case 8:  W32_LAUNCH(8); break;
-    case 9:  W32_LAUNCH(9); break;
-    case 10: W32_LAUNCH(10); break;
-    default: set_error("unsupported n=%d", 1 << logn); return SCGPU_ERR_UNSUPPORTED;
-    }
-#undef W32_LAUNCH
-#undef W32_KB
-#undef W32_PM
-#undef W32_GO
-    count_launch();
-    SCGPU_CUDA_CHECK(cudaGetLastError());
-    return SCGPU_OK;
+    if (logn < 8 || logn > 10) { set_error("unsupported n=%d", 1 << logn); return SCGPU_ERR_UNSUPPORTED; }
+    return with_int<8, 9, 10>(logn, [&](auto L) {
+        unsigned grid;
+        unsigned long long *ctr;
+        const int e = persistent_grid(sm_count, FQ32_MINB, count, Cfg32<L>::POLYS, 2, st, &grid, &ctr);
+        if (e != SCGPU_OK) return e;
+        return with_int<FQ_POLYMUL, FQ_KEY16, FQ_KEY32, FQ_KEYBM>(mode, [&](auto M) {
+            return with_flags([&](auto TMA, auto BM, auto CHK) {
+                // the base multiplication serves the two-operand product and is the only form of the residue product
+                if constexpr (BM ? AR::BASEMUL && (M == FQ_POLYMUL || M == FQ_KEYBM) : M != FQ_KEYBM)
+                    return launch_kernel(k_polymul_w32<AR, L, M, TMA, BM, CHK>, grid, kThreads32, 0, st, out, a, b, b_stride,
+                                         count, ctr, c);
+                else
+                    return SCGPU_ERR_UNSUPPORTED;
+            }, tma, bm, chk);
+        });
+    });
 }
 
 template <class AR>
 int launch_ntt_w32(const W32Const<AR> &c, int logn, int sm_count, int inverse, int32_t *out, const int32_t *a, size_t count,
                    cudaStream_t st, bool chk = true)
 {
-    const int sms = sm_count > 0 ? sm_count : 148;
     const bool tma = ((uintptr_t)a % 16) == 0 && tma_allowed();
-    unsigned long long *ctr = nullptr;
-#define W32_NTT(L)                                                                                         \
-    {                                                                                                      \
-        const size_t groups = (count + Cfg32<L>::POLYS - 1) / Cfg32<L>::POLYS;                             \
-        size_t grid = (size_t)sms * FQ32_MINB;                                                             \
-        if (grid > groups) grid = groups;                                                                  \
-        if (!groups_fit(groups, grid)) { set_error("batch of %zu rows is too large", count); return SCGPU_ERR_ARG; } \
-        if (groups > grid) { const int e = next_work_counter(st, &ctr, 2); if (e != SCGPU_OK) return e; }  \
-        if (tma && chk) {                                                                                  \
-            if (inverse) k_ntt_w32<AR, L, true, true, true><<<(unsigned)grid, kThreads32, 0, st>>>(out, a, count, ctr, c);   \
-            else         k_ntt_w32<AR, L, false, true, true><<<(unsigned)grid, kThreads32, 0, st>>>(out, a, count, ctr, c);  \
-        } else if (tma) {                                                                                  \
-            if (inverse) k_ntt_w32<AR, L, true, true, false><<<(unsigned)grid, kThreads32, 0, st>>>(out, a, count, ctr, c);  \
-            else         k_ntt_w32<AR, L, false, true, false><<<(unsigned)grid, kThreads32, 0, st>>>(out, a, count, ctr, c); \
-        } else if (chk) {                                                                                  \
-            if (inverse) k_ntt_w32<AR, L, true, false, true><<<(unsigned)grid, kThreads32, 0, st>>>(out, a, count, ctr, c);  \
-            else         k_ntt_w32<AR, L, false, false, true><<<(unsigned)grid, kThreads32, 0, st>>>(out, a, count, ctr, c); \
-        } else {                                                                                           \
-            if (inverse) k_ntt_w32<AR, L, true, false, false><<<(unsigned)grid, kThreads32, 0, st>>>(out, a, count, ctr, c); \
-            else         k_ntt_w32<AR, L, false, false, false><<<(unsigned)grid, kThreads32, 0, st>>>(out, a, count, ctr, c);\
-        }                                                                                                  \
-    }
-    switch (logn) {
-    case 8:  W32_NTT(8); break;
-    case 9:  W32_NTT(9); break;
-    case 10: W32_NTT(10); break;
-    default: set_error("unsupported n=%d", 1 << logn); return SCGPU_ERR_UNSUPPORTED;
-    }
-#undef W32_NTT
-    count_launch();
-    SCGPU_CUDA_CHECK(cudaGetLastError());
-    return SCGPU_OK;
+    if (logn < 8 || logn > 10) { set_error("unsupported n=%d", 1 << logn); return SCGPU_ERR_UNSUPPORTED; }
+    return with_int<8, 9, 10>(logn, [&](auto L) {
+        unsigned grid;
+        unsigned long long *ctr;
+        const int e = persistent_grid(sm_count, FQ32_MINB, count, Cfg32<L>::POLYS, 2, st, &grid, &ctr);
+        if (e != SCGPU_OK) return e;
+        return with_flags([&](auto INV, auto TMA, auto CHK) {
+            return launch_kernel(k_ntt_w32<AR, L, INV, TMA, CHK>, grid, kThreads32, 0, st, out, a, count, ctr, c);
+        }, inverse != 0, tma, chk);
+    });
 }
 
 // One shared matrix: its k_matrix_table table in a stream-ordered scratch of the call (not of the plan: two streams may
@@ -1593,25 +1551,18 @@ int matrix_table(const W32Const<AR> &c, const int32_t *A, int rows, cudaStream_t
 {
     const size_t words = (size_t)rows * Cfg32<8>::N * sizeof(TE) / 16;          // one thread per 128-bit word
     SCGPU_CUDA_CHECK(cudaMallocAsync(reinterpret_cast<void **>(tab), words * 16, st));
-    k_matrix_table<AR, TE><<<(unsigned)((words + 127) / 128), 128, 0, st>>>(reinterpret_cast<TE *>(*tab), A, rows, c.q);
-    count_launch();
-    const cudaError_t e = cudaGetLastError();
-    if (e != cudaSuccess) {
-        cudaFreeAsync(*tab, st);
-        set_error("k_matrix_table launch failed: %s", cudaGetErrorString(e));
-        return SCGPU_ERR_CUDA;
-    }
-    return SCGPU_OK;
+    const int e = launch_kernel(k_matrix_table<AR, TE>, (unsigned)((words + 127) / 128), 128, 0, st,
+                                reinterpret_cast<TE *>(*tab), A, rows, c.q);
+    if (e != SCGPU_OK) cudaFreeAsync(*tab, st);
+    return e;
 }
 
-// the batch kernel has been launched (or refused): check it, release the table in stream order
-inline int launched_with_table(int32_t *tab, cudaStream_t st)
+// the batch kernel has been launched (or refused, e != SCGPU_OK): release the table in stream order
+inline int release_table(int32_t *tab, cudaStream_t st, int e)
 {
-    const cudaError_t e = cudaGetLastError();
-    const cudaError_t fe = tab ? cudaFreeAsync(tab, st) : cudaSuccess;
-    if (e != cudaSuccess) { set_error("matvec launch failed: %s", cudaGetErrorString(e)); return SCGPU_ERR_CUDA; }
-    if (fe != cudaSuccess) { set_error("cudaFreeAsync failed: %s", cudaGetErrorString(fe)); return SCGPU_ERR_CUDA; }
-    return SCGPU_OK;
+    const cudaError_t fe = cudaFreeAsync(tab, st);
+    if (e == SCGPU_OK && fe != cudaSuccess) { set_error("cudaFreeAsync failed: %s", cudaGetErrorString(fe)); return SCGPU_ERR_CUDA; }
+    return e;
 }
 
 // n = 256 (Kyber, Dilithium).  shared: A is ONE matrix [k][l][n] for every instance (scgpu_matvec_shared_batch)
@@ -1623,9 +1574,9 @@ int launch_matvec_w32(const W32Const<AR> &c, int sm_count, int32_t *out, const i
     const bool tma = ((uintptr_t)A % 16) == 0 && ((uintptr_t)s % 16) == 0 && tma_allowed();
     // the kernels below that read a shared matrix from its table stage only the s rows
     const bool tma_rows = shared ? ((uintptr_t)s % 16) == 0 && tma_allowed() : tma;
-    const int sms = sm_count > 0 ? sm_count : 148;
-    const size_t groups = (count + C::POLYS - 1) / C::POLYS;
-    unsigned long long *ctr = nullptr;
+    unsigned grid;
+    unsigned long long *ctr;
+    int32_t *tab = nullptr;                          // the shared matrix's table
     // 16-bit stash: the reduced transform values must fit an int16 (|x| <= 0.55 q + 2)
     const char *no16 = getenv("SCGPU_MATVEC_STASH32");
     // measured (Kyber, q = 7681, tools/matvec_stash_ab.py): with the spill-free kernel the 16-bit stash wins for every l
@@ -1639,135 +1590,54 @@ int launch_matvec_w32(const W32Const<AR> &c, int sm_count, int32_t *out, const i
         // |s| <= 0.55 q + 2 (the reduced stash)
         const char *facc = getenv("SCGPU_MATVEC_FLOAT_ACC");
         const bool iacc = (double)l * (double)c.x0 * (0.55 * (double)c.q + 2.0) < 2147483648.0 && !(facc && atoi(facc) != 0);
-        if (shared) {
-            if constexpr (AR::STASH16) {
-                SCGPU_CUDA_CHECK(cudaFuncSetAttribute(k_matvec16_w32<AR, 8, true, true, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
-                SCGPU_CUDA_CHECK(cudaFuncSetAttribute(k_matvec16_w32<AR, 8, true, false, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
-                SCGPU_CUDA_CHECK(cudaFuncSetAttribute(k_matvec16_w32<AR, 8, true, true, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
-                SCGPU_CUDA_CHECK(cudaFuncSetAttribute(k_matvec16_w32<AR, 8, true, false, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
-            }
-        } else {
-            SCGPU_CUDA_CHECK(cudaFuncSetAttribute(k_matvec16_w32<AR, 8, true, true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
-            SCGPU_CUDA_CHECK(cudaFuncSetAttribute(k_matvec16_w32<AR, 8, true, false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
-            if constexpr (AR::STASH16) {
-                SCGPU_CUDA_CHECK(cudaFuncSetAttribute(k_matvec16_w32<AR, 8, true, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
-                SCGPU_CUDA_CHECK(cudaFuncSetAttribute(k_matvec16_w32<AR, 8, true, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
-            }
-        }
         int per_sm = (int)((227 * 1024) / (smem + 1024 + 64));
         if (per_sm > 16) per_sm = 16;
         if (per_sm < 1) per_sm = 1;
-        size_t grid = (size_t)sms * per_sm;
-        if (grid > groups) grid = groups;
-        if (!groups_fit(groups, grid)) { set_error("batch of %zu rows is too large", count); return SCGPU_ERR_ARG; }
-        if (groups > grid) { const int e = next_work_counter(st, &ctr, 2); if (e != SCGPU_OK) return e; }
-        if (shared) {
-            if constexpr (AR::STASH16) {
-                int32_t *tab = nullptr;
-                const int e = matrix_table<AR, int16_t>(c, A, k * l, st, &tab);
-                if (e != SCGPU_OK) return e;
-                if (iacc && chk) k_matvec16_w32<AR, 8, true, true, true, true><<<(unsigned)grid, kThreads32, smem, st>>>(out, tab, s, k, l, count, ctr, c);
-                else if (iacc)   k_matvec16_w32<AR, 8, true, false, true, true><<<(unsigned)grid, kThreads32, smem, st>>>(out, tab, s, k, l, count, ctr, c);
-                else if (chk)    k_matvec16_w32<AR, 8, true, true, false, true><<<(unsigned)grid, kThreads32, smem, st>>>(out, tab, s, k, l, count, ctr, c);
-                else             k_matvec16_w32<AR, 8, true, false, false, true><<<(unsigned)grid, kThreads32, smem, st>>>(out, tab, s, k, l, count, ctr, c);
-                count_launch();
-                return launched_with_table(tab, st);
-            }
-        }
-        bool launched = false;
+        int e = persistent_grid(sm_count, per_sm, count, C::POLYS, 2, st, &grid, &ctr);
+        // integer accumulators and shared matrices are instantiated for the policies with a 16-bit stash only
         if constexpr (AR::STASH16) {
-            if (iacc) {
-                if (chk) k_matvec16_w32<AR, 8, true, true, true><<<(unsigned)grid, kThreads32, smem, st>>>(out, A, s, k, l, count, ctr, c);
-                else     k_matvec16_w32<AR, 8, true, false, true><<<(unsigned)grid, kThreads32, smem, st>>>(out, A, s, k, l, count, ctr, c);
-                launched = true;
-            }
+            if (e == SCGPU_OK && shared) e = matrix_table<AR, int16_t>(c, A, k * l, st, &tab);
         }
-        if (!launched) {
-            if (chk) k_matvec16_w32<AR, 8, true, true, false><<<(unsigned)grid, kThreads32, smem, st>>>(out, A, s, k, l, count, ctr, c);
-            else     k_matvec16_w32<AR, 8, true, false, false><<<(unsigned)grid, kThreads32, smem, st>>>(out, A, s, k, l, count, ctr, c);
-        }
-        count_launch();
-        SCGPU_CUDA_CHECK(cudaGetLastError());
-        return SCGPU_OK;
+        if (e != SCGPU_OK) return e;
+        e = with_flags([&](auto CHK, auto IACC, auto SHARED) {
+            if constexpr (AR::STASH16 || !(IACC || SHARED))
+                return launch_kernel(k_matvec16_w32<AR, 8, true, CHK, IACC, SHARED>, grid, kThreads32, smem, st, out,
+                                     shared ? tab : A, s, k, l, count, ctr, c);
+            else
+                return SCGPU_ERR_UNSUPPORTED;
+        }, chk, iacc, shared);
+        return shared ? release_table(tab, st, e) : e;
     }
-    {
-        // one warp per output row (k_matvec_rows_w32): aligned rows, 2 <= k <= 8; SCGPU_MATVEC_ONE_WARP=1 keeps k_matvec_w32.
-        // A shared matrix needs no staging rows: each warp keeps only its exchange tile
-        const char *ow = getenv("SCGPU_MATVEC_ONE_WARP");
-        const size_t warp_words = shared ? (size_t)C::PW * C::TS : (size_t)C::PW * C::TS + C::PW * (C::N + C::T);
-        const size_t smem_rows = ((size_t)l * C::PW * C::TS + (size_t)k * warp_words) * sizeof(int32_t);
-        if (tma_rows && k >= 2 && k <= 8 && smem_rows <= 110 * 1024 && !(ow && atoi(ow) != 0)) {
-            if (shared) {
-                SCGPU_CUDA_CHECK(cudaFuncSetAttribute(k_matvec_rows_w32<AR, 8, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
-                SCGPU_CUDA_CHECK(cudaFuncSetAttribute(k_matvec_rows_w32<AR, 8, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
-            } else {
-                SCGPU_CUDA_CHECK(cudaFuncSetAttribute(k_matvec_rows_w32<AR, 8, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
-                SCGPU_CUDA_CHECK(cudaFuncSetAttribute(k_matvec_rows_w32<AR, 8, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
-            }
-            const size_t rgroups = (count + C::PW - 1) / C::PW;
-            int per_sm = (int)((227 * 1024) / (smem_rows + 1024 + 256));
-            const int by_regs = 65536 / (k * 32 * 128);
-            if (per_sm > by_regs) per_sm = by_regs;
-            if (per_sm < 1) per_sm = 1;
-            size_t grid = (size_t)sms * per_sm;
-            if (grid > rgroups) grid = rgroups;
-            if (!groups_fit(rgroups, grid)) { set_error("batch of %zu rows is too large", count); return SCGPU_ERR_ARG; }
-            if (rgroups > grid) { const int e = next_work_counter(st, &ctr, 1); if (e != SCGPU_OK) return e; }
-            if (shared) {
-                int32_t *tab = nullptr;
-                const int e = matrix_table<AR, int32_t>(c, A, k * l, st, &tab);
-                if (e != SCGPU_OK) return e;
-                if (chk) k_matvec_rows_w32<AR, 8, true, true><<<(unsigned)grid, 32 * k, smem_rows, st>>>(out, tab, s, k, l, count, ctr, c);
-                else     k_matvec_rows_w32<AR, 8, false, true><<<(unsigned)grid, 32 * k, smem_rows, st>>>(out, tab, s, k, l, count, ctr, c);
-                count_launch();
-                return launched_with_table(tab, st);
-            }
-            if (chk) k_matvec_rows_w32<AR, 8, true><<<(unsigned)grid, 32 * k, smem_rows, st>>>(out, A, s, k, l, count, ctr, c);
-            else     k_matvec_rows_w32<AR, 8, false><<<(unsigned)grid, 32 * k, smem_rows, st>>>(out, A, s, k, l, count, ctr, c);
-            count_launch();
-            SCGPU_CUDA_CHECK(cudaGetLastError());
-            return SCGPU_OK;
-        }
+    // one warp per output row (k_matvec_rows_w32): aligned rows, 2 <= k <= 8; SCGPU_MATVEC_ONE_WARP=1 keeps k_matvec_w32.
+    // A shared matrix needs no staging rows: each warp keeps only its exchange tile
+    const char *ow = getenv("SCGPU_MATVEC_ONE_WARP");
+    const size_t warp_words = shared ? (size_t)C::PW * C::TS : (size_t)C::PW * C::TS + C::PW * (C::N + C::T);
+    const size_t smem_rows = ((size_t)l * C::PW * C::TS + (size_t)k * warp_words) * sizeof(int32_t);
+    if (tma_rows && k >= 2 && k <= 8 && smem_rows <= 110 * 1024 && !(ow && atoi(ow) != 0)) {
+        int per_sm = (int)((227 * 1024) / (smem_rows + 1024 + 256));
+        const int by_regs = 65536 / (k * 32 * 128);
+        if (per_sm > by_regs) per_sm = by_regs;
+        if (per_sm < 1) per_sm = 1;
+        int e = persistent_grid(sm_count, per_sm, count, C::PW, 1, st, &grid, &ctr);
+        if (e == SCGPU_OK && shared) e = matrix_table<AR, int32_t>(c, A, k * l, st, &tab);
+        if (e != SCGPU_OK) return e;
+        e = with_flags([&](auto CHK, auto SHARED) {
+            return launch_kernel(k_matvec_rows_w32<AR, 8, CHK, SHARED>, grid, 32 * k, smem_rows, st, out, shared ? tab : A, s,
+                                 k, l, count, ctr, c);
+        }, chk, shared);
+        return shared ? release_table(tab, st, e) : e;
     }
+    // k = 1, unaligned rows, SCGPU_MATVEC_ONE_WARP: a shared matrix is addressed with an instance stride of 0
     const size_t smem = ((size_t)(l + 1) * C::POLYS * C::TS + (tma ? (size_t)C::POLYS * (C::N + C::T) : 0)) * sizeof(int32_t);
-    // per launch, not once: the attribute belongs to the current device's context and plans exist per device
-    if (shared) {
-        if (tma) {
-            SCGPU_CUDA_CHECK(cudaFuncSetAttribute(k_matvec_w32<AR, 8, true, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
-            SCGPU_CUDA_CHECK(cudaFuncSetAttribute(k_matvec_w32<AR, 8, true, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
-        } else {
-            SCGPU_CUDA_CHECK(cudaFuncSetAttribute(k_matvec_w32<AR, 8, false, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
-            SCGPU_CUDA_CHECK(cudaFuncSetAttribute(k_matvec_w32<AR, 8, false, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
-        }
-    } else if (tma) {
-        SCGPU_CUDA_CHECK(cudaFuncSetAttribute(k_matvec_w32<AR, 8, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
-        SCGPU_CUDA_CHECK(cudaFuncSetAttribute(k_matvec_w32<AR, 8, true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
-    } else {
-        SCGPU_CUDA_CHECK(cudaFuncSetAttribute(k_matvec_w32<AR, 8, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
-        SCGPU_CUDA_CHECK(cudaFuncSetAttribute(k_matvec_w32<AR, 8, false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
-    }
     if (smem > 200 * 1024) { set_error("matvec: l=%d needs %zu bytes of shared memory", l, smem); return SCGPU_ERR_UNSUPPORTED; }
     int per_sm = (int)((227 * 1024) / (smem + 1024 + 64));
     if (per_sm > 16) per_sm = 16;
     if (per_sm < 1) per_sm = 1;
-    size_t grid = (size_t)sms * per_sm;
-    if (grid > groups) grid = groups;
-    if (!groups_fit(groups, grid)) { set_error("batch of %zu rows is too large", count); return SCGPU_ERR_ARG; }
-    if (groups > grid) { const int e = next_work_counter(st, &ctr, 2); if (e != SCGPU_OK) return e; }
-    // k = 1, unaligned rows, SCGPU_MATVEC_ONE_WARP: a shared matrix is addressed with an instance stride of 0
-    if (shared) {
-        if (tma && chk)  k_matvec_w32<AR, 8, true, true, true><<<(unsigned)grid, kThreads32, smem, st>>>(out, A, s, k, l, count, ctr, c);
-        else if (tma)    k_matvec_w32<AR, 8, true, false, true><<<(unsigned)grid, kThreads32, smem, st>>>(out, A, s, k, l, count, ctr, c);
-        else if (chk)    k_matvec_w32<AR, 8, false, true, true><<<(unsigned)grid, kThreads32, smem, st>>>(out, A, s, k, l, count, ctr, c);
-        else             k_matvec_w32<AR, 8, false, false, true><<<(unsigned)grid, kThreads32, smem, st>>>(out, A, s, k, l, count, ctr, c);
-    }
-    else if (tma && chk)  k_matvec_w32<AR, 8, true, true><<<(unsigned)grid, kThreads32, smem, st>>>(out, A, s, k, l, count, ctr, c);
-    else if (tma)    k_matvec_w32<AR, 8, true, false><<<(unsigned)grid, kThreads32, smem, st>>>(out, A, s, k, l, count, ctr, c);
-    else if (chk)    k_matvec_w32<AR, 8, false, true><<<(unsigned)grid, kThreads32, smem, st>>>(out, A, s, k, l, count, ctr, c);
-    else             k_matvec_w32<AR, 8, false, false><<<(unsigned)grid, kThreads32, smem, st>>>(out, A, s, k, l, count, ctr, c);
-    count_launch();
-    SCGPU_CUDA_CHECK(cudaGetLastError());
-    return SCGPU_OK;
+    const int e = persistent_grid(sm_count, per_sm, count, C::POLYS, 2, st, &grid, &ctr);
+    if (e != SCGPU_OK) return e;
+    return with_flags([&](auto TMA, auto CHK, auto SHARED) {
+        return launch_kernel(k_matvec_w32<AR, 8, TMA, CHK, SHARED>, grid, kThreads32, smem, st, out, A, s, k, l, count, ctr, c);
+    }, tma, chk, shared);
 }
 
 }  // namespace w32
