@@ -120,6 +120,59 @@ FQ_HD int32_t mul_unb(int32_t x, float xf, int32_t w, float wq, int32_t pwk, int
     return mad(as_i(f), nq, p);
 }
 
+// ---- products by a twiddle known at compile time: every per-twiddle word is an instruction immediate -----------
+// An FFMA and an IMAD take one immediate each, so the two addends c and k of Tw cannot both stay per twiddle.
+// The twiddle is centred, w = sigma a with 0 < a < q/2, and the float side multiplies by a:  k22 = round(a 2^22 / q),
+// wq = k22 2^-22 <= 1/2.  With ONE addend 2^23 for every twiddle
+//     fmaf(as_float(xb), wq, 2^23)  =  RN( 2^23 + 3 k22 + x wq )
+// stays inside the binade [2^23, 2^24) for |x| < 2^22 (0 <= wq (3 2^22 -+ |x|) < 2^23), so it is again one rounding
+// to an integer and its bits are 0x4B000000 + 3 k22 + qe, qe = rint(x wq), |qe - x a / q| <= 1/2 + |x| 2^-23: the
+// bound of mul.  The integer side takes the per-twiddle constant in its FIRST multiply-add:
+//     p2 = bits (-sigma q) + K,   r = xb w + p2  =  x w - sigma qe q + extra,   K = extra - K0,
+//     K0 = kBias w - sigma q (0x4B000000 + 3 k22)   (mod 2^32)
+// so a product is FFMA (wq immediate) + IMAD (K immediate) + IMAD (w immediate) and the butterfly's two adds carry no
+// per-twiddle constant.  2^23 and -+q come from registers (ImmK).
+struct ImmTw {
+    int32_t w;      // centred multiplier sigma a
+    float wq;       // k22 2^-22, for a
+    bool neg;       // sigma = -1
+    uint32_t k0;    // K0
+};
+
+constexpr ImmTw make_imm(int64_t w, int64_t q)
+{
+    w = ((w % q) + q) % q;
+    if (w > q / 2) w -= q;
+    const int64_t a = w < 0 ? -w : w;
+    const int64_t k22 = (a * (1ll << 23) + q) / (2 * q);             // round(a * 2^22 / q) <= 2^21
+    const uint32_t sq = w < 0 ? (uint32_t)(-q) : (uint32_t)q;
+    return ImmTw{(int32_t)w, (float)k22 / 4194304.0f, w < 0,
+                 (uint32_t)kBias * (uint32_t)w - sq * (0x4B000000u + 3u * (uint32_t)k22)};
+}
+
+struct ImmK { float two23; int32_t q, nq; };        // 2^23, q, -q
+
+// xb biased, |x| < 2^22: x w - sigma qe q + extra.
+// On the device every operation is opaque to the compiler: with 2^23 or -+q as literals it would give the FFMA's or the
+// IMAD's one immediate to them and move wq / K into a register per twiddle, and seen through, the product of a value
+// that an add with a constant produced, (a + C) w, becomes a w + C w, with w in a register.
+FQ_HD uint32_t mul_imm(uint32_t xb, const ImmTw &t, uint32_t extra, const ImmK &kk)
+{
+    const uint32_t K = extra - t.k0;
+    const int32_t sq = t.neg ? kk.q : kk.nq;
+#ifdef __CUDA_ARCH__
+    float f;
+    uint32_t p2, r;
+    asm("fma.rn.f32 %0, %1, %2, %3;" : "=f"(f) : "f"(__uint_as_float(xb)), "f"(t.wq), "f"(kk.two23));
+    asm("mad.lo.u32 %0, %1, %2, %3;" : "=r"(p2) : "r"(__float_as_uint(f)), "r"(sq), "r"(K));
+    asm("mad.lo.u32 %0, %1, %2, %3;" : "=r"(r) : "r"(xb), "r"(t.w), "r"(p2));
+    return r;
+#else
+    const float f = fma_rn(as_f((int32_t)xb), t.wq, kk.two23);
+    return (uint32_t)mad((int32_t)xb, t.w, mad(as_i(f), sq, (int32_t)K));
+#endif
+}
+
 // ---- degree-3 base multiplication: the transform stops two stages early -------------------------------------
 // After stage logn - 3 the polynomial is split into n/4 residues modulo X^4 - zeta_b (four consecutive elements,
 // natural order).  Their products

@@ -185,6 +185,21 @@ inline bool analyse32_bm(int logn, int64_t qi, int32_t x0, int *r0_out, BmBounds
     return false;
 }
 
+// The same schedule with the pass-0 entries as instruction immediates (fq_arith.cuh: make_imm, mul_imm).  A product by an immediate entry has the error bound of mul (|qe - x a / q| <= 1/2 + |x| 2^-23), so the
+// bounds of analyse32_bm hold unchanged; what is new is that its FFMA must stay inside the binade [2^23, 2^24) for
+// every entry w[0 .. count) and every value analyse32_bm admits (|x| < lim):  0 <= wq (3 2^22 - lim)  and
+// 2^23 + wq (3 2^22 + lim) <= 2^24 - 1.
+inline bool analyse32_bm_imm(int logn, int64_t qi, int32_t x0, const int64_t *w, int count, int *r0_out)
+{
+    if (!analyse32_bm(logn, qi, x0, r0_out)) return false;
+    const double lim = (double)kLimit - 2.0;
+    for (int i = 0; i < count; i++) {
+        const double wq = (double)make_imm(w[i], qi).wq;
+        if (wq * (12582912.0 - lim) < 0.0 || 8388608.0 + wq * (12582912.0 + lim) > 16777215.0) return false;
+    }
+    return true;
+}
+
 // zeta_b = zf[n/4 + b]^2 (the modulus X^4 - zeta_b of block b after stage logn - 3) as (w, wq) pairs, and the two
 // entries of the last inverse stage with (n/4)^-1 instead of n^-1 (two Gentleman-Sande stages fewer double the
 // result twice less)

@@ -4,7 +4,8 @@
 // 1024), so a whole product needs one shared-memory exchange per transform and only __syncwarp():
 //
 //   pass 0   stages 0..4   thread tau holds elements tau + (n/32) m, m = 0..31.  The 31 twiddles of these
-//                          stages are the same for every thread: they live in the kernel's constant bank.
+//                          stages are the same for every thread: they live in the kernel's constant bank, or, for
+//                          the reference's (12289, 512) table, in the instructions themselves (ArFqImm).
 //   pass 1   stages 5..    thread tau holds the 32 contiguous elements 32 tau .. 32 tau + 31, i.e. 32 / SUB
 //                          independent sub-chunks of SUB = n/32 elements; both operands of a sub-chunk are
 //                          transformed together (shared twiddles), multiplied pointwise and taken back through
@@ -21,6 +22,8 @@
 
 #include <algorithm>
 #include <cstring>
+#include <type_traits>
+#include <utility>
 #include <vector>
 
 namespace scgpu {
@@ -34,10 +37,12 @@ using w32::u32;
 // Arithmetic policy: float-quotient products (fq_arith.cuh); coefficients travel biased by kBias.
 struct ArFq {
     typedef Tw E;
-    struct K { int32_t nq, q, pwk; float invq; int32_t pwb; };
+    struct K { int32_t nq, q, pwk; float invq; int32_t pwb; float two23; };   // two23 = 2^23: ArFqImm's FFMA addend
     static constexpr bool STASH16 = true;          // mat-vec may keep the transformed vectors as int16
     static constexpr bool BASEMUL = true;          // two-operand products stop two stages early (fq::basemul4)
     static constexpr int WORDS = 4;
+    static constexpr bool PASS0_IMM = false;
+    template <int L, int M, bool BM> static constexpr bool serves() { return true; }
     static __device__ __forceinline__ u32 enc(int32_t x) { return (u32)x + (u32)kBias; }
     static __device__ __forceinline__ int32_t dec(u32 x) { return (int32_t)(x - (u32)kBias); }
     static __device__ __forceinline__ u32 zero() { return (u32)kBias; }
@@ -163,6 +168,104 @@ struct ArFq {
 
 typedef w32::W32Const<ArFq> FqConst32;
 
+// ---- pass 0 of the reference's (q, n) = (12289, 512) table, compiled in ------------------------------------------
+// The reference's ntt_table_gen table is w[e] = psi^e, psi the smallest m >= 2 with m^n = -1 (mod q).  From it
+// build_tables / build_bm_tables derive the pass-0 entries zf[k] = psi^brv(k) and zi[k] = -psi^(n - brv(k)), and for the
+// last stage of the base-multiplication schedule (n/4)^-1 and zi[1] (n/4)^-1.  The same formulas, evaluated by the
+// compiler, make every pass-0 entry of the fused product an instruction immediate (fq_arith.cuh: make_imm): no constant
+// loads, no registers.  build_fq32_tables selects this kernel only when the plan's own entries equal these.
+namespace p0 {
+constexpr int64_t kQ = 12289;
+constexpr int kLogN = 9, kN = 1 << kLogN;
+constexpr int64_t pow_c(int64_t b, int64_t e)
+{
+    int64_t r = 1;
+    for (b %= kQ; e > 0; e >>= 1, b = b * b % kQ)
+        if (e & 1) r = r * b % kQ;
+    return r;
+}
+constexpr int64_t first_root()
+{
+    for (int64_t m = 2; m < kQ - 1; m++)
+        if (pow_c(m, kN) == kQ - 1) return m;
+    return 0;
+}
+constexpr int64_t kPsi = first_root();
+constexpr int brv(int k)
+{
+    int e = 0;
+    for (int b = 0; b < kLogN; b++) e |= ((k >> b) & 1) << (kLogN - 1 - b);
+    return e;
+}
+constexpr int64_t fwd(int k) { return pow_c(kPsi, brv(k)); }                       // zf[k].w
+constexpr int64_t inv(int k) { return (kQ - pow_c(kPsi, kN - brv(k))) % kQ; }     // zi[k].w, k >= 2
+constexpr int64_t ninv() { return pow_c(kN / 4, kQ - 2); }                         // (n/4)^-1
+constexpr int64_t inv1() { return inv(1) * ninv() % kQ; }                          // zi[1] (n/4)^-1
+static_assert(kPsi != 0 && pow_c(kPsi, 2 * kN) == 1, "no 2n-th root of unity");
+
+template <int... I, class F>
+__device__ __forceinline__ void static_for_(std::integer_sequence<int, I...>, F &&f) { (f(std::integral_constant<int, I>{}), ...); }
+template <int N, class F>
+__device__ __forceinline__ void static_for(F &&f) { static_for_(std::make_integer_sequence<int, N>{}, f); }
+}  // namespace p0
+
+// ArFq with pass 0 compiled for the reference's (12289, 512) table: the two-operand product with the base
+// multiplication only (serves).  Same stages, same bounds (fq_host.h: analyse32_bm_imm), 5 instructions per butterfly
+// (fq_arith.cuh: mul_imm) and no constant loads.
+struct ArFqImm : ArFq {
+    static constexpr bool PASS0_IMM = true;
+    template <int L, int M, bool BM> static constexpr bool serves() { return L == p0::kLogN && M == w32::FQ_POLYMUL && BM; }
+    // stages 0..4 on x[m] = element tau + T m; x[0..15] arrive raw (load_operand)
+    static __device__ __forceinline__ void fwd_pass0(u32 (&x)[32], const K &k)
+    {
+        const fq::ImmK kk{k.two23, k.q, k.nq};
+        p0::static_for<5>([&](auto S) {
+            constexpr int s = S, half = 16 >> s;
+            p0::static_for<16>([&](auto J) {
+                constexpr int m = (J / half) * 2 * half + J % half;
+                constexpr fq::ImmTw t = fq::make_imm(p0::fwd((1 << s) + (m >> (5 - s))), p0::kQ);
+                const u32 r = fq::mul_imm(x[m + half], t, 0u, kk);
+                if constexpr (s == 0) {
+                    // two opaque copies of kBias, as in ArFq::ct0: each result is one 3-input add
+                    u32 kb1, kb2;
+                    asm("mov.u32 %0, 0x4B400000;" : "=r"(kb1));
+                    asm("mov.u32 %0, 1262485504;" : "=r"(kb2));
+                    x[m + half] = x[m] - r + kb1;
+                    x[m] = x[m] + r + kb2;
+                } else {
+                    x[m + half] = x[m] - r;
+                    x[m] = x[m] + r;
+                }
+            });
+        });
+    }
+    // stages 4..1 (biased products), then stage 0 with (n/4)^-1 folded into both branches; canonical residues out
+    static __device__ __forceinline__ void inv_pass0(u32 (&x)[32], const K &k)
+    {
+        const fq::ImmK kk{k.two23, k.q, k.nq};
+        p0::static_for<4>([&](auto I) {
+            constexpr int s = 4 - I, half = 16 >> s;
+            p0::static_for<16>([&](auto J) {
+                constexpr int m = (J / half) * 2 * half + J % half;
+                constexpr fq::ImmTw t = fq::make_imm(p0::inv((1 << s) + (m >> (5 - s))), p0::kQ);
+                const u32 d = x[m] - x[m + half] + (u32)kBias;
+                x[m] = x[m] + x[m + half] - (u32)kBias;
+                x[m + half] = fq::mul_imm(d, t, (u32)kBias, kk);
+            });
+        });
+        constexpr fq::ImmTw ni = fq::make_imm(p0::ninv(), p0::kQ), z = fq::make_imm(p0::inv1(), p0::kQ);
+        p0::static_for<16>([&](auto M) {
+            constexpr int m = M;
+            const u32 s = x[m] + x[m + 16] - (u32)kBias;
+            const u32 d = x[m] - x[m + 16] + (u32)kBias;
+            const u32 ys = fq::mul_imm(s, ni, 0u, kk), yd = fq::mul_imm(d, z, 0u, kk);
+            x[m] = min(ys, ys + (u32)k.q);
+            x[m + 16] = min(yd, yd + (u32)k.q);
+        });
+    }
+};
+typedef w32::W32Const<ArFqImm> FqImmConst32;
+
 // ---- key residues for the base-multiplication key product -------------------------------------------------------
 // The key arrives fully transformed (the reference's NTT-domain order).  Two Gentleman-Sande stages and a factor 1/4
 // take the four point values of block b back to the residue modulo X^4 - zeta_b; the table also holds zeta_b times
@@ -210,8 +313,28 @@ struct Fq32State {
     int32_t *ktab;                       // k_key_residues: [zi stage logn-2 | zi stage logn-1 | zeta], n words
     int32_t inv4;                        // 4^-1 mod q
     bool mv_ok, bm_ok;                   // mv_ok: mat-vec with up to 4 accumulated products
+    bool imm;                            // the plan's pass-0 entries are ArFqImm's: its two-operand product runs that kernel
     FqConst32 prod, mv, bm;              // bm: last inverse stage with (n/4)^-1
+    FqImmConst32 bm_imm;                 // bm for the ArFqImm kernel (the same words)
 };
+
+// true when the pass-0 entries of the base-multiplication constants are the ones compiled into ArFqImm and the
+// interval analysis admits them as immediates
+static bool imm_pass0_matches(const NttPlanDev &p, const FqConst32 &bm)
+{
+    if (p.rc.q != p0::kQ || p.logn != p0::kLogN) return false;
+    int64_t w[64];
+    for (int k = 1; k < 32; k++) {
+        if (bm.f0[k - 1].w != p0::fwd(k) || (k > 1 && bm.i0[k - 1].w != p0::inv(k))) return false;
+        w[2 * k - 2] = bm.f0[k - 1].w;
+        w[2 * k - 1] = bm.i0[k - 1].w;
+    }
+    if (bm.i0[0].w != p0::inv1() || bm.ninv.w != p0::ninv()) return false;
+    w[62] = bm.ninv.w;
+    w[63] = bm.i0[0].w;
+    int r0 = 0;
+    return fq::analyse32_bm_imm(p.logn, p.rc.q, bm.x0, w, 64, &r0) && r0 == bm.r0;
+}
 
 int build_fq32_tables(NttPlanDev &p, const int32_t *w_host)
 {
@@ -273,6 +396,7 @@ int build_fq32_tables(NttPlanDev &p, const int32_t *w_host)
     c.k.pwk = (int32_t)((uint32_t)kBias * (uint32_t)p.rc.q);
     c.k.invq = (float)(1.0 / (double)p.rc.q);
     c.k.pwb = (int32_t)((uint32_t)c.k.pwk + (uint32_t)kBias);
+    c.k.two23 = 8388608.0f;
     c.M = (uint32_t)((1ull << 32) / (uint64_t)p.rc.q);
     s->prod = s->mv = s->bm = c;
     s->prod.r0 = r0;
@@ -281,6 +405,9 @@ int build_fq32_tables(NttPlanDev &p, const int32_t *w_host)
         s->bm.r0 = r0_bm;
         s->bm.ninv = ninv_bm;
         s->bm.i0[0] = i01_bm;
+        s->imm = imm_pass0_matches(p, s->bm);
+        static_assert(sizeof(FqImmConst32) == sizeof(FqConst32) && std::is_trivially_copyable<FqConst32>::value, "same words");
+        memcpy(&s->bm_imm, &s->bm, sizeof(FqConst32));
     }
     return SCGPU_OK;
 }
@@ -336,6 +463,9 @@ int launch_polymul_fq32(const NttPlanDev &p, int mode, int32_t *out, const int32
         return e;
     }
     const bool bm = mode == w32::FQ_POLYMUL && fs.bm_ok;
+    if (bm && fs.imm)
+        return w32::launch_polymul_w32<ArFqImm>(fs.bm_imm, p.logn, p.sm_count, mode, out, a, b, b_stride, count, st, true,
+                                                !p.inputs_in_range);
     return w32::launch_polymul_w32<ArFq>(bm ? fs.bm : fs.prod, p.logn, p.sm_count, mode, out, a, b, b_stride, count, st, bm,
                                          !p.inputs_in_range);
 }

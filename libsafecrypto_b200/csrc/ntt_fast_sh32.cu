@@ -26,6 +26,8 @@ struct ArSh {
     static constexpr bool BASEMUL = false;         // Montgomery pointwise products: no shared-quotient sums
     static constexpr bool STASH16 = false;          // mat-vec may keep the transformed vectors as int16
     static constexpr int WORDS = 2;
+    static constexpr bool PASS0_IMM = false;
+    template <int L, int M, bool BM> static constexpr bool serves() { return true; }
     static __device__ __forceinline__ u32 enc(int32_t x) { return (u32)x; }
     static __device__ __forceinline__ int32_t dec(u32 x) { return (int32_t)x; }
     static __device__ __forceinline__ u32 zero() { return 0u; }

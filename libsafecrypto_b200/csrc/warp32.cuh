@@ -7,6 +7,8 @@
 // Policy interface:  E (twiddle entry), K (scalar constants), WORDS (32-bit words of E in the tables),
 //   enc / dec / zero            raw <-> internal representation of a coefficient, internal zero
 //   cb(e)                       entry read from the kernel's constant bank
+//   PASS0_IMM                   true: AR::fwd_pass0(x, k) / AR::inv_pass0(x, k) replace the table-driven pass 0 (entries
+//                               compiled into the policy); serves<LOGN, MODE, BM>() limits the kernels it is built for
 //   mk(words)                   entry from WORDS table words
 //   ct / gs                     forward / inverse butterfly on internal values
 //   ct0                         ct whose lo operand is still RAW (stage 0 encodes it for free in its 3-input adds)
@@ -248,6 +250,7 @@ static __device__ __forceinline__ bool out_of_range(int32_t v, const Const &c)
 // ---- pass 0: stages 0..4 on x[m] = element tau + T m ---------------------------------------------------
 static __device__ __forceinline__ void fwd_pass0(u32 (&x)[32], const Const &c)
 {
+    if constexpr (AR::PASS0_IMM) { AR::fwd_pass0(x, c.k); return; }
 #pragma unroll
     for (int s = 0; s < 5; s++) {
         const int half = 16 >> s;
@@ -263,6 +266,7 @@ static __device__ __forceinline__ void fwd_pass0(u32 (&x)[32], const Const &c)
 // stages 4..1, then stage 0 with n^-1 folded into both branches; returns canonical residues
 static __device__ __forceinline__ void inv_pass0(u32 (&x)[32], const Const &c)
 {
+    if constexpr (AR::PASS0_IMM) { AR::inv_pass0(x, c.k); return; }
 #pragma unroll
     for (int s = 4; s >= 1; s--) {
         const int half = 16 >> s;
@@ -1517,7 +1521,8 @@ int launch_polymul_w32(const W32Const<AR> &c, int logn, int sm_count, int mode, 
         return with_int<FQ_POLYMUL, FQ_KEY16, FQ_KEY32, FQ_KEYBM>(mode, [&](auto M) {
             return with_flags([&](auto TMA, auto BM, auto CHK) {
                 // the base multiplication serves the two-operand product and is the only form of the residue product
-                if constexpr (BM ? AR::BASEMUL && (M == FQ_POLYMUL || M == FQ_KEYBM) : M != FQ_KEYBM)
+                if constexpr ((BM ? AR::BASEMUL && (M == FQ_POLYMUL || M == FQ_KEYBM) : M != FQ_KEYBM) &&
+                              AR::template serves<L, M, BM>())
                     return launch_kernel(k_polymul_w32<AR, L, M, TMA, BM, CHK>, grid, kThreads32, 0, st, out, a, b, b_stride,
                                          count, ctr, c);
                 else

@@ -59,9 +59,12 @@ static void polymul(int logn, int64_t q, const std::vector<Tw> &zf, const std::v
 
 // warp-local schedule with the degree-3 base multiplication (fq_arith.cuh: basemul4)
 static double g_max_sum;
+// imm: stages 0..4 of both directions with the entries as instruction immediates (fq_arith.cuh: mul_imm), as the
+// kernel compiled for the reference's (12289, 512) table runs them
 static void polymul_bm(int logn, int64_t q, const std::vector<Tw> &zf, const std::vector<Tw> &zi, const Tw &one, int r0,
-                       const int32_t *a, const int32_t *b, int32_t *out, const int32_t *w_host)
+                       const int32_t *a, const int32_t *b, int32_t *out, const int32_t *w_host, bool imm = false)
 {
+    const ImmK kk{8388608.0f, (int32_t)q, (int32_t)-q};
     const int n = 1 << logn; const int32_t nq = (int32_t)-q;
     std::vector<int32_t> zw; std::vector<float> zwq; Tw ninv_bm, i01_bm;
     build_bm_tables(logn, q, w_host, zw, zwq, ninv_bm, i01_bm);
@@ -73,7 +76,8 @@ static void polymul_bm(int logn, int64_t q, const std::vector<Tw> &zf, const std
             for (int blk = 0; blk < (1 << s); blk++)
                 for (int j = 0; j < len; j++) {
                     int32_t &lo = x[op][2 * blk * len + j], &hi = x[op][2 * blk * len + j + len];
-                    int32_t t = mul(rd(hi, g_max_fwd), zf[(1 << s) + blk], nq);
+                    int32_t t = imm && s < 5 ? (int32_t)mul_imm((uint32_t)rd(hi, g_max_fwd), make_imm(zf[(1 << s) + blk].w, q), 0u, kk)
+                                             : mul(rd(hi, g_max_fwd), zf[(1 << s) + blk], nq);
                     hi = lo - t; lo = lo + t;
                     if (s == logn - 3) { hi -= kBias; lo -= kBias; }         // the last stage emits unbiased values
                 }
@@ -100,12 +104,19 @@ static void polymul_bm(int logn, int64_t q, const std::vector<Tw> &zf, const std
                 int32_t &lo = y[2 * blk * len + j], &hi = y[2 * blk * len + j + len];
                 int32_t sb = lo + hi - kBias, db = lo - hi + kBias;
                 if (s == 0) {
-                    lo = mul(rd(sb, g_max_inv), ninv_bm, nq); hi = mul(rd(db, g_max_inv), i01_bm, nq);
+                    if (imm) {
+                        lo = (int32_t)mul_imm((uint32_t)rd(sb, g_max_inv), make_imm(ninv_bm.w, q), 0u, kk);
+                        hi = (int32_t)mul_imm((uint32_t)rd(db, g_max_inv), make_imm(i01_bm.w, q), 0u, kk);
+                    } else {
+                        lo = mul(rd(sb, g_max_inv), ninv_bm, nq); hi = mul(rd(db, g_max_inv), i01_bm, nq);
+                    }
                     if (fabs((double)lo) > g_max_fin) g_max_fin = fabs((double)lo);
                     if (fabs((double)hi) > g_max_fin) g_max_fin = fabs((double)hi);
                     lo += (lo >> 31) & (int32_t)q; hi += (hi >> 31) & (int32_t)q;
                 } else {
-                    hi = mul(rd(db, g_max_inv), zi[(1 << s) + blk], nq); lo = sb;
+                    hi = imm && s < 5 ? (int32_t)mul_imm((uint32_t)rd(db, g_max_inv), make_imm(zi[(1 << s) + blk].w, q), (uint32_t)kBias, kk)
+                                      : mul(rd(db, g_max_inv), zi[(1 << s) + blk], nq);
+                    lo = sb;
                 }
             }
     }
@@ -141,10 +152,21 @@ int main()
         if (!build_tables(logn, q, w.data(), zf, zi, ninv, one)) { printf("  tables failed\n"); bad++; continue; }
         std::vector<int32_t> a(n), b(n), o(n), e(n);
         const int x0 = sc.x0;
-        for (int sched = 0; sched < 3; sched++) {
+        for (int sched = 0; sched < 4; sched++) {
         g_max_fwd = g_max_inv = g_max_fin = g_max_sum = 0;
         g_r0 = -1;
         BmBounds bmb; int r0bm = 0;
+        if (sched == 3) {
+            // the pass-0 entries as immediates: the 62 entries of stages 0..4 and the two of the last stage
+            std::vector<int32_t> zw; std::vector<float> zwq; Tw nb, ib;
+            build_bm_tables(logn, q, w.data(), zw, zwq, nb, ib);
+            std::vector<int64_t> ent;
+            for (int k = 1; k < 32; k++) { ent.push_back(zf[k].w); if (k > 1) ent.push_back(zi[k].w); }
+            ent.push_back(nb.w); ent.push_back(ib.w);
+            if (!analyse32_bm_imm(logn, q, x0, ent.data(), (int)ent.size(), &r0bm)) { printf("  pass 0 with immediate entries: refused\n"); continue; }
+            analyse32_bm(logn, q, x0, &r0bm, &bmb);
+            printf("  pass 0 with immediate entries: accepted r0=%d\n", r0bm);
+        }
         if (sched == 2) {
             if (!analyse32_bm(logn, q, x0, &r0bm, &bmb)) { printf("  base multiplication: not applicable\n"); continue; }
             printf("  warp-local schedule with base multiplication: r0=%d fwd_max=%.0f pw_max=%.0f\n", r0bm, bmb.fwd_max, bmb.pw_max);
@@ -166,13 +188,13 @@ int main()
                 default: a[i] = (int32_t)(q - 1); b[i] = (int32_t)(q - 1); break;
                 }
             }
-            if (sched == 2) polymul_bm(logn, q, zf, zi, one, r0bm, a.data(), b.data(), o.data(), w.data());
+            if (sched >= 2) polymul_bm(logn, q, zf, zi, one, r0bm, a.data(), b.data(), o.data(), w.data(), sched == 3);
             else polymul(logn, q, zf, zi, ninv, one, sc, a.data(), b.data(), o.data());
             school(n, q, a.data(), b.data(), e.data());
             for (int i = 0; i < n; i++) if (o[i] != e[i]) { if (bad < 5) printf("  MISMATCH trial %d i=%d got %d want %d\n", trial, i, o[i], e[i]); bad++; break; }
         }
         printf("  observed: fwd %.0f inv %.0f final %.0f  (limit %d)\n", g_max_fwd, g_max_inv, g_max_fin, kLimit);
-        if (sched == 2 && (g_max_fwd > bmb.fwd_max || g_max_sum > bmb.pw_max)) { printf("  BOUND VIOLATED (base multiplication: fwd %.0f pw %.0f)\n", g_max_fwd, g_max_sum); bad++; }
+        if (sched >= 2 && (g_max_fwd > bmb.fwd_max || g_max_sum > bmb.pw_max)) { printf("  BOUND VIOLATED (base multiplication: fwd %.0f pw %.0f)\n", g_max_fwd, g_max_sum); bad++; }
         if (g_max_fwd > sc.fwd_max || g_max_inv >= (double)kLimit || g_max_fin >= (double)q) { printf("  BOUND VIOLATED\n"); bad++; }
         if (sched == 0 && (g_max_inv > sc.inv_max || g_max_fin > sc.final_max)) { printf("  BOUND VIOLATED (8-coefficient schedule)\n"); bad++; }
         }
