@@ -56,6 +56,10 @@ def lib():
         L.scgpu_rand_product_csprng_batch.argtypes = [vp, vp, vp, vp, sz, ctypes.c_int, u32, ctypes.c_int, ctypes.c_int, ctypes.c_int, sz, vp]
         L.scgpu_rand_product_csprng_batch_host.argtypes = [vp, vp, vp, vp, sz, ctypes.c_int, u32, ctypes.c_int, ctypes.c_int, ctypes.c_int, sz]
         L.scgpu_matvec_shared_batch.argtypes = [vp, vp, vp, vp, ctypes.c_int, ctypes.c_int, sz, vp]
+        L.scgpu_polymul_add_batch.argtypes = [vp, vp, vp, vp, sz, vp, sz, vp]
+        L.scgpu_ntt_mul_key_add_batch.argtypes = [vp, vp, vp, vp, ctypes.c_int, sz, vp, sz, vp]
+        L.scgpu_matvec_add_batch.argtypes = [vp, vp, vp, vp, vp, ctypes.c_int, ctypes.c_int, sz, vp]
+        L.scgpu_matvec_shared_add_batch.argtypes = [vp, vp, vp, vp, vp, ctypes.c_int, ctypes.c_int, sz, vp]
         L.scgpu_rand_product_csprng_shared_batch.argtypes = [vp, vp, vp, vp, sz, ctypes.c_int, u32, ctypes.c_int, ctypes.c_int, ctypes.c_int, sz, vp]
         L.scgpu_rand_product_csprng_shared_batch_host.argtypes = [vp, vp, vp, vp, sz, ctypes.c_int, u32, ctypes.c_int, ctypes.c_int, ctypes.c_int, sz]
         L.scgpu_rand_matrix_csprng_batch.argtypes = [vp, vp, sz, ctypes.c_int, i32, u32, ctypes.c_int, ctypes.c_int, ctypes.c_int, ctypes.c_int, sz, vp]
@@ -205,6 +209,35 @@ class NttPlan:
             count = s.shape[0]
         return _check(lib().scgpu_matvec_shared_batch(self.handle, _ptr(out), _ptr(A), _ptr(s), k, l, count,
                                                       _stream_handle(stream)), "scgpu_matvec_shared_batch")
+
+    # ---- the products above with an addend e laid out like out: out = (product + e) mod q; out may be e ----------
+    def polymul_add(self, out, a, b, e, count=None, stream=None):
+        if count is None:
+            count = a.shape[0]
+        b_stride = 0 if b.dim() == 1 else b.shape[-1]
+        return _check(lib().scgpu_polymul_add_batch(self.handle, _ptr(out), _ptr(a), _ptr(b), b_stride, _ptr(e), count,
+                                                    _stream_handle(stream)), "scgpu_polymul_add_batch")
+
+    def mul_key_add(self, out, t, key, e, count=None, stream=None):
+        if count is None:
+            count = t.shape[0]
+        key_bits = key.element_size() * 8
+        key_stride = 0 if key.dim() == 1 else key.shape[-1]
+        return _check(lib().scgpu_ntt_mul_key_add_batch(self.handle, _ptr(out), _ptr(t), _ptr(key), key_bits, key_stride,
+                                                        _ptr(e), count, _stream_handle(stream)), "scgpu_ntt_mul_key_add_batch")
+
+    def matvec_add(self, out, A, s, e, k, l, count=None, stream=None):
+        if count is None:
+            count = s.shape[0]
+        return _check(lib().scgpu_matvec_add_batch(self.handle, _ptr(out), _ptr(A), _ptr(s), _ptr(e), k, l, count,
+                                                   _stream_handle(stream)), "scgpu_matvec_add_batch")
+
+    def matvec_shared_add(self, out, A, s, e, k, l, count=None, stream=None):
+        """matvec_add with ONE matrix A [k, l, n] for every instance of s [count, l, n]."""
+        if count is None:
+            count = s.shape[0]
+        return _check(lib().scgpu_matvec_shared_add_batch(self.handle, _ptr(out), _ptr(A), _ptr(s), _ptr(e), k, l, count,
+                                                          _stream_handle(stream)), "scgpu_matvec_shared_add_batch")
 
     def rand_product(self, out, y, seeds, prng_type, q_bits, k, l, transpose=False, count=None, stream=None):
         """create_rand_product_{16,32}_csprng with the matrix sampled on the device from seeds [count, seed_len]."""

@@ -3,6 +3,7 @@
 //   polymul:  out = INTT(NTT(a) o NTT(b))          two operands in, one result out: 12 n bytes of HBM
 //   mul_key:  out = INTT(NTT(t) o key)             key already in the reference's NTT domain
 //   matvec:   t_i = INTT(sum_j A_ij o NTT(s_j))    module-LWE product (module_lwe.c:588-748)
+//   each with an optional addend e (the *_add entry points): out = (product + e) mod q
 //
 // The result of these compositions is the canonical residue in [0, q) in the reference
 // (inv_ntt_* ends with ntt32_flip_generic's conditional +q / -q, ntt.c:571-604), so the
@@ -456,15 +457,49 @@ int fused_unavailable(const NttPlanDev &p)
     return SCGPU_ERR_UNSUPPORTED;
 }
 
+// out = (prod + e) mod q for a canonical prod and any SINT32 e (64-bit sum: q + e may leave 32 bits).  out may be prod.
+__global__ void k_add_canonical(int32_t *out, const int32_t *prod, const int32_t *e, size_t words, int32_t q)
+{
+    for (size_t i = blockIdx.x * (size_t)blockDim.x + threadIdx.x; i < words; i += (size_t)gridDim.x * blockDim.x) {
+        const int64_t v = ((int64_t)prod[i] + (int64_t)e[i]) % q;
+        out[i] = (int32_t)(v < 0 ? v + q : v);
+    }
+}
+
+// The addend on the arithmetics whose kernels have no epilogue for it (Montgomery, 32-bit Barrett, the 8-coefficient
+// float-quotient schedule: cross-checks of the warp-local kernels, which add it in the product's own kernel):
+// product(P) writes the sibling call's result, then one elementwise kernel adds e.  P is out, or a stream-ordered
+// scratch of the call when out is e itself.
+template <class F>
+int add_after(const NttPlanDev &p, int32_t *out, const int32_t *e, size_t words, cudaStream_t st, F &&product)
+{
+    int32_t *P = out;
+    if (out == e) SCGPU_CUDA_CHECK(cudaMallocAsync(reinterpret_cast<void **>(&P), words * sizeof(int32_t), st));
+    int r = product(P);
+    if (r == SCGPU_OK) {
+        const size_t cap = (size_t)(p.sm_count > 0 ? p.sm_count : 148) * 8;
+        const size_t blocks = (words + 255) / 256;
+        r = launch_kernel(k_add_canonical, (unsigned)(blocks < cap ? blocks : cap), 256, 0, st, out, P, e, words, p.rc.q);
+    }
+    if (P != out) {
+        const cudaError_t fe = cudaFreeAsync(P, st);
+        if (r == SCGPU_OK && fe != cudaSuccess) { set_error("cudaFreeAsync failed: %s", cudaGetErrorString(fe)); r = SCGPU_ERR_CUDA; }
+    }
+    return r;
+}
+
 }  // namespace
 
 int launch_polymul(const NttPlanDev &p, int32_t *out, const int32_t *a, const int32_t *b,
-                   size_t b_stride, size_t count, cudaStream_t st)
+                   size_t b_stride, size_t count, cudaStream_t st, const int32_t *e)
 {
     if (count == 0) return SCGPU_OK;
-    switch (choose_arith(p, OP_PRODUCT)) {
-    case AR_SH32: return launch_polymul_sh32(p, 0, out, a, b, b_stride, count, st);
-    case AR_FQ32: return launch_polymul_fq32(p, 0, out, a, b, b_stride, count, st);
+    const Arith ar = choose_arith(p, OP_PRODUCT);
+    if (e && ar != AR_SH32 && ar != AR_FQ32)
+        return add_after(p, out, e, count * p.n, st, [&](int32_t *P) { return launch_polymul(p, P, a, b, b_stride, count, st); });
+    switch (ar) {
+    case AR_SH32: return launch_polymul_sh32(p, 0, out, a, b, b_stride, count, st, e);
+    case AR_FQ32: return launch_polymul_fq32(p, 0, out, a, b, b_stride, count, st, e);
     case AR_FQ:   return launch_polymul_fq(p, 0, out, a, b, b_stride, count, st);
     case AR_SQ:   return launch_polymul_sq(p, 0, out, a, b, b_stride, count, st);
     case AR_MONT: break;
@@ -489,14 +524,18 @@ int launch_ntt_canonical(const NttPlanDev &p, int inverse, int32_t *out, const i
 }
 
 int launch_mul_key(const NttPlanDev &p, int32_t *out, const int32_t *t, const void *key,
-                   int key_bits, size_t key_stride, size_t count, cudaStream_t st)
+                   int key_bits, size_t key_stride, size_t count, cudaStream_t st, const int32_t *e)
 {
     if (count == 0) return SCGPU_OK;
     if (key_bits != 16 && key_bits != 32) { set_error("key_bits must be 16 or 32"); return SCGPU_ERR_ARG; }
     const int mode = key_bits == 16 ? MODE_KEY16 : MODE_KEY32;
-    switch (choose_arith(p, OP_PRODUCT)) {
-    case AR_SH32: return launch_polymul_sh32(p, mode, out, t, key, key_stride, count, st);
-    case AR_FQ32: return launch_polymul_fq32(p, mode, out, t, key, key_stride, count, st);
+    const Arith ar = choose_arith(p, OP_PRODUCT);
+    if (e && ar != AR_SH32 && ar != AR_FQ32)
+        return add_after(p, out, e, count * p.n, st,
+                         [&](int32_t *P) { return launch_mul_key(p, P, t, key, key_bits, key_stride, count, st); });
+    switch (ar) {
+    case AR_SH32: return launch_polymul_sh32(p, mode, out, t, key, key_stride, count, st, e);
+    case AR_FQ32: return launch_polymul_fq32(p, mode, out, t, key, key_stride, count, st, e);
     case AR_FQ:   return launch_polymul_fq(p, mode, out, t, key, key_stride, count, st);
     case AR_SQ:   return launch_polymul_sq(p, mode, out, t, key, key_stride, count, st);
     case AR_MONT: break;
@@ -511,15 +550,19 @@ int launch_mul_key(const NttPlanDev &p, int32_t *out, const int32_t *t, const vo
 }
 
 int launch_matvec(const NttPlanDev &p, int32_t *out, const int32_t *A, const int32_t *s,
-                  int k, int l, size_t count, cudaStream_t st, bool shared)
+                  int k, int l, size_t count, cudaStream_t st, bool shared, const int32_t *e)
 {
     if (count == 0) return SCGPU_OK;
     if (!p.mont) return fused_unavailable(p);
     if (k < 1 || l < 1 || l > 8) { set_error("matvec supports 1 <= l <= 8 (got k=%d l=%d)", k, l); return SCGPU_ERR_ARG; }
     if (p.logn != 8) { set_error("matvec is instantiated for n = 256 (Kyber / Dilithium); got n=%d", p.n); return SCGPU_ERR_UNSUPPORTED; }
-    switch (choose_arith(p, OP_MATVEC, l)) {
-    case AR_SH32: return launch_matvec_sh32(p, out, A, s, k, l, count, st, shared);
-    case AR_FQ32: return launch_matvec_fq32(p, out, A, s, k, l, count, st, shared);
+    const Arith ar = choose_arith(p, OP_MATVEC, l);
+    if (e && ar != AR_SH32 && ar != AR_FQ32)
+        return add_after(p, out, e, count * (size_t)k * p.n, st,
+                         [&](int32_t *P) { return launch_matvec(p, P, A, s, k, l, count, st, shared); });
+    switch (ar) {
+    case AR_SH32: return launch_matvec_sh32(p, out, A, s, k, l, count, st, shared, e);
+    case AR_FQ32: return launch_matvec_fq32(p, out, A, s, k, l, count, st, shared, e);
     case AR_FQ:   return launch_matvec_fq(p, out, A, s, k, l, count, st, shared);
     case AR_SQ:   return launch_matvec_sq(p, out, A, s, k, l, count, st, shared);
     case AR_MONT: break;

@@ -426,13 +426,13 @@ int fq32_matvec_lmax(const NttPlanDev &p) { return p.fq32 && p.fq32->mv_ok ? 4 :
 
 // n = 256 (Kyber), l <= 4 (launch_matvec)
 int launch_matvec_fq32(const NttPlanDev &p, int32_t *out, const int32_t *A, const int32_t *s, int k, int l,
-                       size_t count, cudaStream_t st, bool shared)
+                       size_t count, cudaStream_t st, bool shared, const int32_t *e)
 {
-    return w32::launch_matvec_w32<ArFq>(p.fq32->mv, p.sm_count, out, A, s, k, l, count, st, !p.inputs_in_range, shared);
+    return w32::launch_matvec_w32<ArFq>(p.fq32->mv, p.sm_count, out, A, s, k, l, count, st, !p.inputs_in_range, shared, e);
 }
 
 int launch_polymul_fq32(const NttPlanDev &p, int mode, int32_t *out, const int32_t *a, const void *b,
-                        size_t b_stride, size_t count, cudaStream_t st)
+                        size_t b_stride, size_t count, cudaStream_t st, const int32_t *e)
 {
     const Fq32State &fs = *p.fq32;
     if (b_stride == 0 && fs.bm_ok && (mode != w32::FQ_POLYMUL || count >= 64)) {
@@ -445,29 +445,30 @@ int launch_polymul_fq32(const NttPlanDev &p, int mode, int32_t *out, const int32
         SCGPU_CUDA_CHECK(cudaMallocAsync(reinterpret_cast<void **>(&kres), sizeof(int32_t) * 5 * (size_t)p.n, st));
         int32_t *hat = kres + 4 * (size_t)p.n;
         const unsigned nb = p.n / 4, th = 64;
-        int e = SCGPU_OK;
+        int r = SCGPU_OK;
         if (mode == w32::FQ_POLYMUL) {
-            e = launch_ntt_fq32(p, 0, hat, static_cast<const int32_t *>(b), 1, st);
+            r = launch_ntt_fq32(p, 0, hat, static_cast<const int32_t *>(b), 1, st);
             b = hat;
         }
-        if (e == SCGPU_OK) {
+        if (r == SCGPU_OK) {
             if (mode == w32::FQ_KEY16)
-                e = launch_kernel(k_key_residues<int16_t>, (nb + th - 1) / th, th, 0, st, kres, static_cast<const int16_t *>(b), fs.ktab, p.logn, p.rc.q, fs.inv4);
+                r = launch_kernel(k_key_residues<int16_t>, (nb + th - 1) / th, th, 0, st, kres, static_cast<const int16_t *>(b), fs.ktab, p.logn, p.rc.q, fs.inv4);
             else
-                e = launch_kernel(k_key_residues<int32_t>, (nb + th - 1) / th, th, 0, st, kres, static_cast<const int32_t *>(b), fs.ktab, p.logn, p.rc.q, fs.inv4);
+                r = launch_kernel(k_key_residues<int32_t>, (nb + th - 1) / th, th, 0, st, kres, static_cast<const int32_t *>(b), fs.ktab, p.logn, p.rc.q, fs.inv4);
         }
-        if (e == SCGPU_OK)
-            e = w32::launch_polymul_w32<ArFq>(fs.bm, p.logn, p.sm_count, w32::FQ_KEYBM, out, a, kres, 0, count, st, true, !p.inputs_in_range);
+        if (r == SCGPU_OK)
+            r = w32::launch_polymul_w32<ArFq>(fs.bm, p.logn, p.sm_count, w32::FQ_KEYBM, out, a, kres, 0, count, st, true,
+                                              !p.inputs_in_range, e);
         const cudaError_t fe = cudaFreeAsync(kres, st);
-        if (e == SCGPU_OK && fe != cudaSuccess) { set_error("cudaFreeAsync failed: %s", cudaGetErrorString(fe)); e = SCGPU_ERR_CUDA; }
-        return e;
+        if (r == SCGPU_OK && fe != cudaSuccess) { set_error("cudaFreeAsync failed: %s", cudaGetErrorString(fe)); r = SCGPU_ERR_CUDA; }
+        return r;
     }
     const bool bm = mode == w32::FQ_POLYMUL && fs.bm_ok;
     if (bm && fs.imm)
         return w32::launch_polymul_w32<ArFqImm>(fs.bm_imm, p.logn, p.sm_count, mode, out, a, b, b_stride, count, st, true,
-                                                !p.inputs_in_range);
+                                                !p.inputs_in_range, e);
     return w32::launch_polymul_w32<ArFq>(bm ? fs.bm : fs.prod, p.logn, p.sm_count, mode, out, a, b, b_stride, count, st, bm,
-                                         !p.inputs_in_range);
+                                         !p.inputs_in_range, e);
 }
 
 int launch_ntt_fq32(const NttPlanDev &p, int inverse, int32_t *out, const int32_t *a, size_t count, cudaStream_t st)

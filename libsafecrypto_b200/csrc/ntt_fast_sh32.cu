@@ -241,15 +241,16 @@ int sh32_matvec_lmax(const NttPlanDev &p) { return p.sh32 ? p.sh32->mv_lmax : 0;
 
 // n = 256, l <= mv_lmax (launch_matvec)
 int launch_matvec_sh32(const NttPlanDev &p, int32_t *out, const int32_t *A, const int32_t *s, int k, int l,
-                       size_t count, cudaStream_t st, bool shared)
+                       size_t count, cudaStream_t st, bool shared, const int32_t *e)
 {
-    return w32::launch_matvec_w32<ArSh>(p.sh32->mv, p.sm_count, out, A, s, k, l, count, st, !p.inputs_in_range, shared);
+    return w32::launch_matvec_w32<ArSh>(p.sh32->mv, p.sm_count, out, A, s, k, l, count, st, !p.inputs_in_range, shared, e);
 }
 
 int launch_polymul_sh32(const NttPlanDev &p, int mode, int32_t *out, const int32_t *a, const void *b,
-                        size_t b_stride, size_t count, cudaStream_t st)
+                        size_t b_stride, size_t count, cudaStream_t st, const int32_t *e)
 {
-    return w32::launch_polymul_w32<ArSh>(p.sh32->prod, p.logn, p.sm_count, mode, out, a, b, b_stride, count, st, false, !p.inputs_in_range);
+    return w32::launch_polymul_w32<ArSh>(p.sh32->prod, p.logn, p.sm_count, mode, out, a, b, b_stride, count, st, false,
+                                         !p.inputs_in_range, e);
 }
 
 int launch_ntt_sh32(const NttPlanDev &p, int inverse, int32_t *out, const int32_t *a, size_t count, cudaStream_t st)

@@ -106,13 +106,14 @@ int launch_gen_rings(int prng_type, const uint8_t *seeds, size_t seed_len, size_
 int build_xw32_tables(NttPlanDev &plan, const int32_t *w_host, const int32_t *r_host);
 void free_xw32_tables(NttPlanDev &plan);
 int launch_exact_w32(const NttPlanDev &plan, int op, int32_t *out, const int32_t *a, size_t count, cudaStream_t stream);
+// e != nullptr (the *_add entry points): out = (product + e) mod q, e laid out like out and possibly out itself
 int launch_polymul(const NttPlanDev &plan, int32_t *out, const int32_t *a, const int32_t *b,
-                   size_t b_stride, size_t count, cudaStream_t stream);
+                   size_t b_stride, size_t count, cudaStream_t stream, const int32_t *e = nullptr);
 int launch_mul_key(const NttPlanDev &plan, int32_t *out, const int32_t *t, const void *key,
-                   int key_bits, size_t key_stride, size_t count, cudaStream_t stream);
+                   int key_bits, size_t key_stride, size_t count, cudaStream_t stream, const int32_t *e = nullptr);
 // shared: A is ONE matrix [k][l][n] for all `count` instances (scgpu_matvec_shared_batch)
 int launch_matvec(const NttPlanDev &plan, int32_t *out, const int32_t *A, const int32_t *s,
-                  int k, int l, size_t count, cudaStream_t stream, bool shared = false);
+                  int k, int l, size_t count, cudaStream_t stream, bool shared = false, const int32_t *e = nullptr);
 int build_fast_tables(NttPlanDev &plan, const int32_t *w_host);
 void free_fast_tables(NttPlanDev &plan);
 int set_force_montgomery(int on);
@@ -124,18 +125,18 @@ int launch_polymul_fq(const NttPlanDev &plan, int mode, int32_t *out, const int3
 int build_fq32_tables(NttPlanDev &plan, const int32_t *w_host);
 void free_fq32_tables(NttPlanDev &plan);
 int launch_polymul_fq32(const NttPlanDev &plan, int mode, int32_t *out, const int32_t *a, const void *b,
-                        size_t b_stride, size_t count, cudaStream_t stream);
+                        size_t b_stride, size_t count, cudaStream_t stream, const int32_t *e = nullptr);
 int build_sh32_tables(NttPlanDev &plan, const int32_t *w_host);
 void free_sh32_tables(NttPlanDev &plan);
 int launch_polymul_sh32(const NttPlanDev &plan, int mode, int32_t *out, const int32_t *a, const void *b,
-                        size_t b_stride, size_t count, cudaStream_t stream);
+                        size_t b_stride, size_t count, cudaStream_t stream, const int32_t *e = nullptr);
 int launch_matvec_sh32(const NttPlanDev &plan, int32_t *out, const int32_t *A, const int32_t *s, int k, int l,
-                       size_t count, cudaStream_t stream, bool shared = false);
+                       size_t count, cudaStream_t stream, bool shared = false, const int32_t *e = nullptr);
 int launch_ntt_fq32(const NttPlanDev &plan, int inverse, int32_t *out, const int32_t *a, size_t count, cudaStream_t stream);
 int launch_ntt_sh32(const NttPlanDev &plan, int inverse, int32_t *out, const int32_t *a, size_t count, cudaStream_t stream);
 int launch_ntt_canonical(const NttPlanDev &plan, int inverse, int32_t *out, const int32_t *a, size_t count, cudaStream_t stream);
 int launch_matvec_fq32(const NttPlanDev &plan, int32_t *out, const int32_t *A, const int32_t *s, int k, int l,
-                       size_t count, cudaStream_t stream, bool shared = false);
+                       size_t count, cudaStream_t stream, bool shared = false, const int32_t *e = nullptr);
 // largest l of the mat-vec of a warp-local arithmetic the plan has (0: none)
 int fq32_matvec_lmax(const NttPlanDev &plan);
 int sh32_matvec_lmax(const NttPlanDev &plan);

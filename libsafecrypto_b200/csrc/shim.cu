@@ -342,6 +342,40 @@ extern "C" int scgpu_matvec_shared_batch(const scgpu_ntt_plan_t *plan, int32_t *
     return launch_matvec(plan->dev, out, A, s, k, l, count, static_cast<cudaStream_t>(stream), true);
 }
 
+// ---- the products above with an addend: out = (product + e) mod q ---------------------------------------------------
+
+extern "C" int scgpu_polymul_add_batch(const scgpu_ntt_plan_t *plan, int32_t *out, const int32_t *a, const int32_t *b,
+                                       size_t b_stride, const int32_t *e, size_t count, void *stream)
+{
+    if (!plan || !out || !a || !b || !e) { set_error("polymul_add_batch: null argument"); return SCGPU_ERR_ARG; }
+    SCGPU_CUDA_CHECK(cudaSetDevice(plan->dev.device));
+    return launch_polymul(plan->dev, out, a, b, b_stride, count, static_cast<cudaStream_t>(stream), e);
+}
+
+extern "C" int scgpu_ntt_mul_key_add_batch(const scgpu_ntt_plan_t *plan, int32_t *out, const int32_t *t, const void *key,
+                                           int key_bits, size_t key_stride, const int32_t *e, size_t count, void *stream)
+{
+    if (!plan || !out || !t || !key || !e) { set_error("ntt_mul_key_add_batch: null argument"); return SCGPU_ERR_ARG; }
+    SCGPU_CUDA_CHECK(cudaSetDevice(plan->dev.device));
+    return launch_mul_key(plan->dev, out, t, key, key_bits, key_stride, count, static_cast<cudaStream_t>(stream), e);
+}
+
+extern "C" int scgpu_matvec_add_batch(const scgpu_ntt_plan_t *plan, int32_t *out, const int32_t *A, const int32_t *s,
+                                      const int32_t *e, int k, int l, size_t count, void *stream)
+{
+    if (!plan || !out || !A || !s || !e) { set_error("matvec_add_batch: null argument"); return SCGPU_ERR_ARG; }
+    SCGPU_CUDA_CHECK(cudaSetDevice(plan->dev.device));
+    return launch_matvec(plan->dev, out, A, s, k, l, count, static_cast<cudaStream_t>(stream), false, e);
+}
+
+extern "C" int scgpu_matvec_shared_add_batch(const scgpu_ntt_plan_t *plan, int32_t *out, const int32_t *A, const int32_t *s,
+                                             const int32_t *e, int k, int l, size_t count, void *stream)
+{
+    if (!plan || !out || !A || !s || !e) { set_error("matvec_shared_add_batch: null argument"); return SCGPU_ERR_ARG; }
+    SCGPU_CUDA_CHECK(cudaSetDevice(plan->dev.device));
+    return launch_matvec(plan->dev, out, A, s, k, l, count, static_cast<cudaStream_t>(stream), true, e);
+}
+
 // ---- module product with the matrix sampled on the device (rand_product.cu) ----------------------------------------
 
 static int check_rand_args(const char *what, int prng_type, size_t seed_len, int n, int k, int l)

@@ -460,15 +460,60 @@ static __device__ __forceinline__ void load_operand_staged(u32 (&x)[32], const i
     for (int m = 0; m < 32; m++) x[m] = m < 16 ? (u32)v[m] : AR::enc(v[m]);
 }
 
+// ---- the addend of the *_add entry points:  out = (product + e) mod q ----------------------------------------------
+// x in [0, q), |v| <= 4 q:  t = x + v + 4 q lies in [0, 9 q) (< 2^31 for q < 2^27); with M = floor(2^32 / q) the
+// quotient floor(t M / 2^32) is floor(t / q) or one less (t (2^32 / q - M) < 2^32), so t minus it times q lies in
+// [0, 2 q) and one conditional -q is canonical.  IADD3, IMAD.HI, IMAD, IADD, VIMNMX per coefficient.
+static __device__ __forceinline__ u32 add_canon(u32 x, int32_t v, u32 q4, const Const &c)
+{
+    const u32 t = x + (u32)v + q4;
+    const u32 r = __umulhi(t, c.M) * (u32)c.nq + t;
+    return min(r, r - (u32)c.q);
+}
+// x[m] = canonical residue of element tau + T m of a row  ->  (x[m] + erow[tau + T m]) mod q.  The lane reads the
+// addresses it stores to (for each m the T lanes of a polynomial read T consecutive words: whole sectors, any
+// alignment).  CHK: a warp vote on |e| > 4 q, then the Barrett reduction of the out-of-range path (|bred(e)| <= q);
+// without it the caller vouches |e| <= 4 q.  (32 addend words next to the 32 results spill nothing, k_matvec16_w32
+// included: its accumulators are dead once the inverse transform has run.)
+template <int LOGN, bool CHK>
+static __device__ __forceinline__ void add_addend(u32 (&x)[32], const int32_t *erow, int tau, const Const &c)
+{
+    constexpr int T = Cfg32<LOGN>::T;
+    const u32 q4 = 4u * (u32)c.q;
+    int32_t v[32];
+    bool wide = false;
+#pragma unroll
+    for (int m = 0; m < 32; m++) {
+        v[m] = erow[tau + m * T];
+        if (CHK) wide |= (u32)v[m] + q4 > 2u * q4;
+    }
+    if (CHK && __any_sync(0xFFFFFFFFu, wide)) {
+#pragma unroll
+        for (int m = 0; m < 32; m++) v[m] = bred(v[m], c);
+    }
+#pragma unroll
+    for (int m = 0; m < 32; m++) x[m] = add_canon(x[m], v[m], q4, c);
+}
+
 };  // struct W32
+
+// The addend rows of an iteration are requested into L2 when it starts (one 128-byte line per lane: the n/32 lanes of a
+// row cover its 4 n bytes), so that the loads of the epilogue find them there.  Every address lies inside an addend
+// row (rows beyond the batch are clamped to row 0, as the operands are).
+__device__ __forceinline__ void prefetch_l2(const int32_t *p)
+{
+    asm volatile("prefetch.global.L2 [%0];" ::"l"(p));
+}
 
 // TMA = true: operand rows arrive by bulk copy (16-byte aligned rows); false: plain LDG (any alignment)
 // BM = true (FQ_POLYMUL, policies with AR::BASEMUL): the transforms stop two stages early and the residues modulo
 // X^4 - zeta are multiplied directly (c carries the last-stage entries for (n/4)^-1).  CHK = false: no range vote.
-template <class AR, int LOGN, int MODE, bool TMA, bool BM = false, bool CHK = true>
+// ADD: out = (product + e) mod q, e [count][n] (may be out itself); without it e is not read.
+template <class AR, int LOGN, int MODE, bool TMA, bool BM = false, bool CHK = true, bool ADD = false>
 __global__ void __launch_bounds__(kThreads32, FQ32_MINB)
 k_polymul_w32(int32_t *__restrict__ out, const int32_t *__restrict__ a, const void *__restrict__ bsrc,
-               size_t b_stride, size_t count, unsigned long long *ctr, const __grid_constant__ W32Const<AR> c)
+               size_t b_stride, size_t count, unsigned long long *ctr, const __grid_constant__ W32Const<AR> c,
+               const int32_t *e)
 {
     using C = Cfg32<LOGN>;
     using W = W32<AR>;
@@ -518,6 +563,7 @@ k_polymul_w32(int32_t *__restrict__ out, const int32_t *__restrict__ a, const vo
         const size_t prow = live ? poly : 0;
         cl.issue(ctr, lane);
         const size_t nbase = (size_t)cl.gn * C::POLYS;
+        if (ADD) prefetch_l2(e + prow * N + 32 * tau);
         // rolled loops (operand, sub-chunk): the fully unrolled body was 60 KB of SASS and spent 2 of every
         // 7 stall cycles waiting for instructions (profiles/polymul_r02c_*); the L1.5 I-cache holds 32 KB
 #pragma unroll 1
@@ -617,6 +663,7 @@ k_polymul_w32(int32_t *__restrict__ out, const int32_t *__restrict__ a, const vo
                 for (int m = 0; m < 32; m++) x[m] = AR::red(x[m], c.one, c.k);
             }
             W::inv_pass0(x, c);
+            if (ADD) W::template add_addend<LOGN, CHK>(x, e + prow * N, tau, c);
             if (live) {
                 int32_t *orow = out + poly * N;
 #pragma unroll
@@ -792,10 +839,12 @@ k_ntt_w32(int32_t *__restrict__ out, const int32_t *__restrict__ a, size_t count
 // consecutive words: conflict-free from the staging row (instances 8 banks apart), one full sector from HBM
 // in the LDG variant.
 // SHARED_A: one matrix [k][l][n] for every instance (scgpu_matvec_shared_batch), addressed with an instance stride of 0
-template <class AR, int LOGN, bool TMA, bool CHK = true, bool SHARED_A = false>
+// ADD: t_i = (t_i + e_i) mod q, e [count][k][n] (may be out itself); without it e is not read.
+template <class AR, int LOGN, bool TMA, bool CHK = true, bool SHARED_A = false, bool ADD = false>
 __global__ void __launch_bounds__(kThreads32)
 k_matvec_w32(int32_t *__restrict__ out, const int32_t *__restrict__ A, const int32_t *__restrict__ s,
-              int k, int l, size_t count, unsigned long long *ctr, const __grid_constant__ W32Const<AR> c)
+              int k, int l, size_t count, unsigned long long *ctr, const __grid_constant__ W32Const<AR> c,
+              const int32_t *e)
 {
     using C = Cfg32<LOGN>;
     using W = W32<AR>;
@@ -858,6 +907,9 @@ k_matvec_w32(int32_t *__restrict__ out, const int32_t *__restrict__ A, const int
         const size_t irow = live ? inst : 0;
         cl.issue(ctr, lane);
         const size_t nbase = (size_t)cl.gn * C::POLYS;
+        if (ADD) {
+            for (int i = 0; i < k; i++) prefetch_l2(e + (irow * k + i) * N + 32 * tau);
+        }
         if (TMA) { mbar_wait(&bars[warp][0], par_s); par_s ^= 1u; }
 #pragma unroll 1
         for (int j = 0; j < l; j++) {
@@ -963,6 +1015,7 @@ k_matvec_w32(int32_t *__restrict__ out, const int32_t *__restrict__ A, const int
                     for (int m = 0; m < 32; m++) x[m] = AR::red(x[m], c.one, c.k);
                 }
                 W::inv_pass0(x, c);
+                if (ADD) W::template add_addend<LOGN, CHK>(x, e + (irow * k + i) * N, tau, c);
                 if (live) {
                     int32_t *orow = out + (inst * k + i) * N;
 #pragma unroll
@@ -1046,10 +1099,12 @@ __device__ __forceinline__ void load_table_row(int32_t (&av)[32], const int32_t 
 // l + 2 to l / k + 2 tiles: 15 warps per SM at k = 5, l = 4.  The s rows of the next group can only be requested after
 // every warp has left the stash (second barrier); the matrix rows of the next group are requested before it.
 // SHARED_A: the matrix is a k_matrix_table table (int32) read by 128-bit loads; no staging rows, no mbarrier per row.
-template <class AR, int LOGN, bool CHK = true, bool SHARED_A = false>
+// ADD: as in k_matvec_w32.
+template <class AR, int LOGN, bool CHK = true, bool SHARED_A = false, bool ADD = false>
 __global__ void __launch_bounds__(256, 2)
 k_matvec_rows_w32(int32_t *__restrict__ out, const int32_t *__restrict__ A, const int32_t *__restrict__ s,
-                  int k, int l, size_t count, unsigned long long *ctr, const __grid_constant__ W32Const<AR> c)
+                  int k, int l, size_t count, unsigned long long *ctr, const __grid_constant__ W32Const<AR> c,
+                  const int32_t *e)
 {
     using C = Cfg32<LOGN>;
     using W = W32<AR>;
@@ -1110,6 +1165,8 @@ k_matvec_rows_w32(int32_t *__restrict__ out, const int32_t *__restrict__ A, cons
         const size_t nbase = (size_t)gn * PW;
         const size_t inst = base + slot;
         const bool live = inst < count;
+        const int32_t *erow = e + ((live ? inst : 0) * k + warp) * N;     // this warp's output row i = warp
+        if (ADD) prefetch_l2(erow + 32 * tau);
         // the group after the next one (read behind the second barrier of this iteration)
         if (threadIdx.x == 0)
             s_next[it & 1u] = ctr != nullptr ? atomicAdd(reinterpret_cast<unsigned *>(ctr), 1u) + 2u * gridDim.x : gn + gridDim.x;
@@ -1201,6 +1258,7 @@ k_matvec_rows_w32(int32_t *__restrict__ out, const int32_t *__restrict__ A, cons
                     for (int m = 0; m < 32; m++) x[m] = AR::red(x[m], c.one, c.k);
                 }
                 W::inv_pass0(x, c);
+                if (ADD) W::template add_addend<LOGN, CHK>(x, erow, tau, c);
                 if (live) {
                     int32_t *orow = out + (inst * k + i) * N;
 #pragma unroll
@@ -1233,10 +1291,12 @@ k_matvec_rows_w32(int32_t *__restrict__ out, const int32_t *__restrict__ A, cons
 // instead of an IMAD, an FFMA and two conversions per term (AR::Acc), and in 32 instead of 64 accumulator registers.
 // SHARED_A (with TMA): the matrix is a k_matrix_table table (int16) read by 128-bit loads; only the s rows travel
 // through the staging row, and s_0 of the warp's next instances is put in flight as soon as s_{l-1} is in registers.
-template <class AR, int LOGN, bool TMA, bool CHK = true, bool IACC = false, bool SHARED_A = false>
+// ADD: as in k_matvec_w32.
+template <class AR, int LOGN, bool TMA, bool CHK = true, bool IACC = false, bool SHARED_A = false, bool ADD = false>
 __global__ void __launch_bounds__(kThreads32, 16)        // 128 registers: 4 warps per scheduler fit (140 allowed 3)
 k_matvec16_w32(int32_t *__restrict__ out, const int32_t *__restrict__ A, const int32_t *__restrict__ s,
-               int k, int l, size_t count, unsigned long long *ctr, const __grid_constant__ W32Const<AR> c)
+               int k, int l, size_t count, unsigned long long *ctr, const __grid_constant__ W32Const<AR> c,
+               const int32_t *e)
 {
     using C = Cfg32<LOGN>;
     using W = W32<AR>;
@@ -1293,6 +1353,9 @@ k_matvec16_w32(int32_t *__restrict__ out, const int32_t *__restrict__ A, const i
         const size_t inst = base + slot;
         const bool live = inst < count;
         const size_t irow = live ? inst : 0;
+        if (ADD) {
+            for (int i = 0; i < k; i++) prefetch_l2(e + (irow * k + i) * N + 32 * tau);
+        }
         // after a row of S has been read into registers: the next row of the S sequence (s rows, then the even columns
         // output row by output row), or row 0 of the warp's next instances; nxt = that row's number in the instance's
         // sequence (s rows 0 .. l-1, matrix rows l + i l + j), -1 = the instance has no further row for S
@@ -1429,6 +1492,7 @@ k_matvec16_w32(int32_t *__restrict__ out, const int32_t *__restrict__ A, const i
                     for (int m = 0; m < 32; m++) x[m] = AR::red(x[m], c.one, c.k);
                 }
                 W::inv_pass0(x, c);
+                if (ADD) W::template add_addend<LOGN, CHK>(x, e + (irow * k + i) * N, tau, c);
                 if (live) {
                     int32_t *orow = out + (inst * k + i) * N;
 #pragma unroll
@@ -1501,10 +1565,11 @@ inline int persistent_grid(int sm_count, int per_sm, size_t count, int per_group
 }
 
 // bm: base-multiplication kernel (FQ_POLYMUL, policies with AR::BASEMUL; c must carry the (n/4)^-1 entries);
-// chk = false: no range vote on the operands
+// chk = false: no range vote on the operands (nor on the addend); e != nullptr: out = (product + e) mod q
 template <class AR>
 int launch_polymul_w32(const W32Const<AR> &c, int logn, int sm_count, int mode, int32_t *out, const int32_t *a,
-                       const void *b, size_t b_stride, size_t count, cudaStream_t st, bool bm = false, bool chk = true)
+                       const void *b, size_t b_stride, size_t count, cudaStream_t st, bool bm = false, bool chk = true,
+                       const int32_t *e = nullptr)
 {
     // bulk copies need 16-byte aligned rows; the second operand is only staged in FQ_POLYMUL mode
     bool tma = ((uintptr_t)a % 16) == 0 && tma_allowed();
@@ -1516,18 +1581,18 @@ int launch_polymul_w32(const W32Const<AR> &c, int logn, int sm_count, int mode, 
     return with_int<8, 9, 10>(logn, [&](auto L) {
         unsigned grid;
         unsigned long long *ctr;
-        const int e = persistent_grid(sm_count, FQ32_MINB, count, Cfg32<L>::POLYS, 2, st, &grid, &ctr);
-        if (e != SCGPU_OK) return e;
+        const int r = persistent_grid(sm_count, FQ32_MINB, count, Cfg32<L>::POLYS, 2, st, &grid, &ctr);
+        if (r != SCGPU_OK) return r;
         return with_int<FQ_POLYMUL, FQ_KEY16, FQ_KEY32, FQ_KEYBM>(mode, [&](auto M) {
-            return with_flags([&](auto TMA, auto BM, auto CHK) {
+            return with_flags([&](auto TMA, auto BM, auto CHK, auto ADD) {
                 // the base multiplication serves the two-operand product and is the only form of the residue product
                 if constexpr ((BM ? AR::BASEMUL && (M == FQ_POLYMUL || M == FQ_KEYBM) : M != FQ_KEYBM) &&
                               AR::template serves<L, M, BM>())
-                    return launch_kernel(k_polymul_w32<AR, L, M, TMA, BM, CHK>, grid, kThreads32, 0, st, out, a, b, b_stride,
-                                         count, ctr, c);
+                    return launch_kernel(k_polymul_w32<AR, L, M, TMA, BM, CHK, ADD>, grid, kThreads32, 0, st, out, a, b,
+                                         b_stride, count, ctr, c, e);
                 else
                     return SCGPU_ERR_UNSUPPORTED;
-            }, tma, bm, chk);
+            }, tma, bm, chk, e != nullptr);
         });
     });
 }
@@ -1570,10 +1635,11 @@ inline int release_table(int32_t *tab, cudaStream_t st, int e)
     return e;
 }
 
-// n = 256 (Kyber, Dilithium).  shared: A is ONE matrix [k][l][n] for every instance (scgpu_matvec_shared_batch)
+// n = 256 (Kyber, Dilithium).  shared: A is ONE matrix [k][l][n] for every instance (scgpu_matvec_shared_batch);
+// e != nullptr: t = (product + e) mod q
 template <class AR>
 int launch_matvec_w32(const W32Const<AR> &c, int sm_count, int32_t *out, const int32_t *A, const int32_t *s, int k, int l,
-                      size_t count, cudaStream_t st, bool chk = true, bool shared = false)
+                      size_t count, cudaStream_t st, bool chk = true, bool shared = false, const int32_t *e = nullptr)
 {
     using C = Cfg32<8>;
     const bool tma = ((uintptr_t)A % 16) == 0 && ((uintptr_t)s % 16) == 0 && tma_allowed();
@@ -1598,20 +1664,20 @@ int launch_matvec_w32(const W32Const<AR> &c, int sm_count, int32_t *out, const i
         int per_sm = (int)((227 * 1024) / (smem + 1024 + 64));
         if (per_sm > 16) per_sm = 16;
         if (per_sm < 1) per_sm = 1;
-        int e = persistent_grid(sm_count, per_sm, count, C::POLYS, 2, st, &grid, &ctr);
+        int r = persistent_grid(sm_count, per_sm, count, C::POLYS, 2, st, &grid, &ctr);
         // integer accumulators and shared matrices are instantiated for the policies with a 16-bit stash only
         if constexpr (AR::STASH16) {
-            if (e == SCGPU_OK && shared) e = matrix_table<AR, int16_t>(c, A, k * l, st, &tab);
+            if (r == SCGPU_OK && shared) r = matrix_table<AR, int16_t>(c, A, k * l, st, &tab);
         }
-        if (e != SCGPU_OK) return e;
-        e = with_flags([&](auto CHK, auto IACC, auto SHARED) {
+        if (r != SCGPU_OK) return r;
+        r = with_flags([&](auto CHK, auto IACC, auto SHARED, auto ADD) {
             if constexpr (AR::STASH16 || !(IACC || SHARED))
-                return launch_kernel(k_matvec16_w32<AR, 8, true, CHK, IACC, SHARED>, grid, kThreads32, smem, st, out,
-                                     shared ? tab : A, s, k, l, count, ctr, c);
+                return launch_kernel(k_matvec16_w32<AR, 8, true, CHK, IACC, SHARED, ADD>, grid, kThreads32, smem, st, out,
+                                     shared ? tab : A, s, k, l, count, ctr, c, e);
             else
                 return SCGPU_ERR_UNSUPPORTED;
-        }, chk, iacc, shared);
-        return shared ? release_table(tab, st, e) : e;
+        }, chk, iacc, shared, e != nullptr);
+        return shared ? release_table(tab, st, r) : r;
     }
     // one warp per output row (k_matvec_rows_w32): aligned rows, 2 <= k <= 8; SCGPU_MATVEC_ONE_WARP=1 keeps k_matvec_w32.
     // A shared matrix needs no staging rows: each warp keeps only its exchange tile
@@ -1623,14 +1689,14 @@ int launch_matvec_w32(const W32Const<AR> &c, int sm_count, int32_t *out, const i
         const int by_regs = 65536 / (k * 32 * 128);
         if (per_sm > by_regs) per_sm = by_regs;
         if (per_sm < 1) per_sm = 1;
-        int e = persistent_grid(sm_count, per_sm, count, C::PW, 1, st, &grid, &ctr);
-        if (e == SCGPU_OK && shared) e = matrix_table<AR, int32_t>(c, A, k * l, st, &tab);
-        if (e != SCGPU_OK) return e;
-        e = with_flags([&](auto CHK, auto SHARED) {
-            return launch_kernel(k_matvec_rows_w32<AR, 8, CHK, SHARED>, grid, 32 * k, smem_rows, st, out, shared ? tab : A, s,
-                                 k, l, count, ctr, c);
-        }, chk, shared);
-        return shared ? release_table(tab, st, e) : e;
+        int r = persistent_grid(sm_count, per_sm, count, C::PW, 1, st, &grid, &ctr);
+        if (r == SCGPU_OK && shared) r = matrix_table<AR, int32_t>(c, A, k * l, st, &tab);
+        if (r != SCGPU_OK) return r;
+        r = with_flags([&](auto CHK, auto SHARED, auto ADD) {
+            return launch_kernel(k_matvec_rows_w32<AR, 8, CHK, SHARED, ADD>, grid, 32 * k, smem_rows, st, out,
+                                 shared ? tab : A, s, k, l, count, ctr, c, e);
+        }, chk, shared, e != nullptr);
+        return shared ? release_table(tab, st, r) : r;
     }
     // k = 1, unaligned rows, SCGPU_MATVEC_ONE_WARP: a shared matrix is addressed with an instance stride of 0
     const size_t smem = ((size_t)(l + 1) * C::POLYS * C::TS + (tma ? (size_t)C::POLYS * (C::N + C::T) : 0)) * sizeof(int32_t);
@@ -1638,11 +1704,12 @@ int launch_matvec_w32(const W32Const<AR> &c, int sm_count, int32_t *out, const i
     int per_sm = (int)((227 * 1024) / (smem + 1024 + 64));
     if (per_sm > 16) per_sm = 16;
     if (per_sm < 1) per_sm = 1;
-    const int e = persistent_grid(sm_count, per_sm, count, C::POLYS, 2, st, &grid, &ctr);
-    if (e != SCGPU_OK) return e;
-    return with_flags([&](auto TMA, auto CHK, auto SHARED) {
-        return launch_kernel(k_matvec_w32<AR, 8, TMA, CHK, SHARED>, grid, kThreads32, smem, st, out, A, s, k, l, count, ctr, c);
-    }, tma, chk, shared);
+    const int r = persistent_grid(sm_count, per_sm, count, C::POLYS, 2, st, &grid, &ctr);
+    if (r != SCGPU_OK) return r;
+    return with_flags([&](auto TMA, auto CHK, auto SHARED, auto ADD) {
+        return launch_kernel(k_matvec_w32<AR, 8, TMA, CHK, SHARED, ADD>, grid, kThreads32, smem, st, out, A, s, k, l, count,
+                             ctr, c, e);
+    }, tma, chk, shared, e != nullptr);
 }
 
 }  // namespace w32
